@@ -10,6 +10,7 @@ H2D copy of the bags and D2H read of the pooled vectors inside the timed region.
 
   python bench.py --gpus N --steps K --warmup W            (N>1: launched by torch.distributed.run)
   python bench.py --impl reference ...                      (CPU arm: the oracle's torch fp32 restatement)
+  python bench.py ... --dump-outputs DIR                    (also write the last timed step's outputs as DIR/*.npy)
 """
 from __future__ import annotations
 
@@ -29,6 +30,7 @@ sys.path.insert(0, ROOT)
 L_FEAT, D_GATE = 1024, 192
 LEN_LO, LEN_HI = 100, 20000
 FALLBACK_PEAKS = {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0}
+DUMP_BUDGET_BYTES = 64 << 20
 
 
 def load_peaks():
@@ -40,6 +42,27 @@ def load_peaks():
         except Exception:
             pass
     return dict(FALLBACK_PEAKS), "fallback"
+
+
+def dump_outputs(dirname, arrays):
+    """--dump-outputs: the {name: tensor} the timed path produced in its last step, one DIR/<name>.npy each, so that two
+    builds can be compared output for output on the same seeded inputs.  Integer and float64 tensors are written as
+    float64 (exact), every other tensor as float32.  A tensor larger than its equal share of the 64 MB budget is written
+    as a fixed sample of its elements: flat indices drawn without replacement from numpy's default_rng(0), in increasing
+    order, so the same shape always gives the same sample."""
+    import numpy as np
+    import torch
+    os.makedirs(dirname, exist_ok=True)
+    share = DUMP_BUDGET_BYTES // len(arrays)
+    for name, t in arrays.items():
+        t = t.detach()
+        wide = t.dtype == torch.float64 or not t.dtype.is_floating_point
+        a = t.to(torch.float64 if wide else torch.float32).cpu().numpy()
+        if a.nbytes > share:
+            keep = share // a.itemsize
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(dirname, name + ".npy"), a)
+    print(f"[bench] last timed step's outputs: {', '.join(sorted(arrays))} -> {dirname}", file=sys.stderr)
 
 
 def bag_lengths(n_bags, seed):
@@ -582,10 +605,12 @@ def fusion_main(args, out):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        tr.step_bags(ct, xp, lens, xt, labels)
+        loss, prob = tr.step_bags(ct, xp, lens, xt, labels)
     e1.record()
     barrier()
     launches = mil_b200.launch_count() - l0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"loss": loss, "prob": prob, "params": tr.params, "grads": tr.grads})
     t = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -711,7 +736,12 @@ def main():
                     help="abmil, world > 1: deal ONE draw of bags x world lengths to the ranks longest-first (dp.shard_bags) "
                          "instead of giving every rank the lengths of the single-GPU workload")
     ap.add_argument("--patients", type=int, default=8, help="fusion: patients per rank per step (<= 8)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32 or "
+                         "float64, at most 64 MB in all; rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.steps < 1):
+        ap.error("--dump-outputs needs --impl ours and --steps >= 1")
     if args.workload == "fusion" and args.impl == "ours":
         return fusion_main(args, out)
     warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
@@ -819,11 +849,16 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        run_step(X, offsets)
+        M = run_step(X, offsets)
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
     launches = mil_b200.launch_count() - l0
+    if args.dump_outputs and rank == 0:
+        # the pooled vectors the step returns, the per-instance attention scores and per-bag argmax, and the trainer's
+        # parameters (after the Adam update) and gradients
+        dump_outputs(args.dump_outputs, {"M": M, "scores": tr.last_scores, "argmax": tr.last_argmax, "params": tr.params,
+                                         "grads": tr.grads})
     t = torch.tensor([ms], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -1,35 +1,30 @@
-"""oracle/_ref (the reference's own ABMIL.py, copied unmodified by oracle/make_ref.py at build time) against the oracle's
-restatements — a live pin in addition to the committed fixtures.  Skipped where the recipe has not run."""
+"""The reference's own ABMIL (model/dim1/ABMIL.py, run unmodified in float64 by tests/golden/make_golden.py, outputs stored
+in tests/golden/abmil_L96_N37.npz) against the oracle's restatements, forward and backward."""
 import numpy as np
-import pytest
 import torch
 
 from oracle import fusion_oracle as fo
-from oracle import make_ref
 from oracle import mil_oracle as mo
+from tests.helpers import load_golden, rnd
 
 
 def test_reference_abmil_module_equals_both_oracles():
-    Ref = make_ref.load_reference_abmil()
-    if Ref is None:
-        pytest.skip("oracle/_ref/ABMIL.py absent (python oracle/make_ref.py needs /root/reference)")
-    L = 96
-    p = mo.procedural_state(mo.abmil_shapes(L), 3)
-    ref = Ref(None, L=L).eval()
-    ref.load_state_dict({k: torch.from_numpy(v) for k, v in p.items()}, strict=True)
-    x = torch.from_numpy(np.random.RandomState(4).standard_normal((1, 57, L)).astype(np.float32)).requires_grad_(True)
-    M = ref(x)
-    M.sum().backward()
-    f = mo.abmil_forward(p, x.detach().numpy()[0])
-    assert np.abs(M.detach().numpy() - f["M"]).max() <= 1e-5 * np.abs(f["M"]).max()
+    fx = load_golden("abmil_L96_N37")
+    L, N, seed = int(fx["L"]), int(fx["N"]), int(fx["seed"])
+    p = mo.procedural_state(mo.abmil_shapes(L), seed)
+    x = rnd(seed + 100, 1, N, L)
+    dM = torch.from_numpy(rnd(seed + 200, 1, L)).double()
+    f = mo.abmil_forward(p, x[0])
+    assert np.abs(fx["M"] - f["M"]).max() <= 1e-5 * np.abs(f["M"]).max()
     sd = {"a." + k: torch.from_numpy(v).double().requires_grad_(True) for k, v in p.items()}
-    xd = x.detach().double().requires_grad_(True)
+    xd = torch.from_numpy(x).double().requires_grad_(True)
     Mo = fo.abmil(sd, "a", xd)
-    Mo.sum().backward()
-    assert float((M.detach().double() - Mo.detach()).abs().max()) <= 1e-5 * float(Mo.abs().max())
-    assert float((x.grad.double() - xd.grad).abs().max()) <= 1e-5 * float(xd.grad.abs().max())
-    for k, v in ref.named_parameters():
+    (Mo * dM).sum().backward()
+    Mo = Mo.detach()
+    assert float((torch.from_numpy(fx["M"]) - Mo).abs().max()) <= 1e-5 * float(Mo.abs().max())
+    assert float((torch.from_numpy(fx["dx"]) - xd.grad[0]).abs().max()) <= 1e-5 * float(xd.grad.abs().max())
+    for k in p:
         if k == "attention_weights.bias":
             continue
         g = sd["a." + k].grad
-        assert float((v.grad.double() - g).abs().max()) <= 2e-5 * float(g.abs().max()), k
+        assert float((torch.from_numpy(fx["g:" + k]) - g).abs().max()) <= 2e-5 * float(g.abs().max()), k

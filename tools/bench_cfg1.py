@@ -1,5 +1,5 @@
 import os, sys, torch, numpy as np
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import mil_b200
 from mil_b200.dp import AbmilTrainer
 B1, N1 = 32, 512
