@@ -307,18 +307,6 @@ int milb200_tape_backward(const milb200_tape_op* ops, int n_ops, const milb200_t
                           const float* p_f32, float* g_f32, const void* arena, size_t arena_bytes, void* workspace,
                           size_t ws_bytes, int dtype, const milb200_segments* segs, void* stream);
 
-/* ---- single-pass forward of the gated pool (ABMIL.py:52-59 in one pass over X) ---------------------------------
- * = milb200_gated_score_fwd (gate_act required) + milb200_segment_softmax_pool_fwd with the same outputs, reading X
- * from HBM once: extra warps of the score GEMM reduce every finished 128-row tile to softmax-pooling records while it is
- * L2-resident and the pooling kernel runs over the records.  milb200_gated_score_pool_supported() == 0 (other dtypes,
- * L > 1024, the single-SM kernel selected): the entry returns MILB200_EUNSUPPORTED and the caller makes the two calls. */
-int milb200_gated_score_pool_supported(int L, int D, int dtype);
-size_t milb200_gated_score_pool_workspace_bytes(int64_t total_n, int B, int L);
-int milb200_gated_score_pool_fwd(const void* X, const void* Wcat, const float* bcat, const float* ww, const float* bw,
-                                 const int32_t* offsets, int B, float* scores, void* gate_act, float* M, int32_t* argmax,
-                                 float* lse, int64_t total_n, int L, int D, int dtype, void* workspace, size_t ws_bytes,
-                                 void* stream);
-
 /* ---- mirrored single-pass backward of the gated pool (autograd of ABMIL.py:52-59 in one pass over X) -----------
  * = milb200_segment_softmax_pool_bwd (attn == NULL) + milb200_gated_score_bwd (gate_act given, dX == NULL) with the same
  * outputs: dscores_i = a_i (dM_b . x_i - dM_b . M_b) is computed by extra warps INSIDE the dWcat tensor-core kernel, a few

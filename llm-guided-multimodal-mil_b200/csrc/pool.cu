@@ -11,7 +11,6 @@
 #include <cfloat>
 
 #include "common.cuh"
-#include "tc_gemm.cuh"
 
 namespace milb200 {
 
@@ -550,91 +549,6 @@ static int pool_check(const void* X, const float* scores, const int32_t* offsets
   return MILB200_OK;
 }
 
-// ---- single-pass forward: the second stage over the pooling records of the score kernel (tc_gemm.cu, EpiScoreT POOL) ----
-// Record k + b holds the normalised partial of (32-row block k, bag b).  Bag b owns records [o_b / 32 + b, (o_{b+1} - 1) / 32 + b];
-// when o_{b+1} is a multiple of 32 the index o_{b+1} / 32 + b is never written (the next block starts the next bag): it
-// becomes an explicit zero-weight record so that the record offsets stay a contiguous CSR.
-constexpr int REC_ROWS = 32;
-__global__ void __launch_bounds__(128)
-k_record_prepare(const int32_t* __restrict__ offsets, int B, int L, int32_t* __restrict__ rec_off, float* __restrict__ rec_x,
-                 float* __restrict__ rec_s, float* __restrict__ rec_key, int32_t* __restrict__ rec_val) {
-  const int b = blockIdx.x;   // 0 .. B
-  const int32_t ob = __ldg(offsets + b);
-  if (threadIdx.x == 0) rec_off[b] = ob / REC_ROWS + b;
-  if (b == B) return;
-  const int32_t oe = __ldg(offsets + b + 1);
-  if (oe % REC_ROWS != 0) return;
-  const int64_t gap = oe / REC_ROWS + b;
-  for (int c = threadIdx.x; c < L; c += blockDim.x) rec_x[gap * L + c] = 0.f;
-  if (threadIdx.x == 0) {
-    rec_s[gap] = -FLT_MAX;
-    rec_key[gap] = -FLT_MAX;
-    rec_val[gap] = 0;
-  }
-}
-
-// argmax[b] = instance (index within the bag) of the largest score: first maximum in row order
-__global__ void __launch_bounds__(128)
-k_record_argmax(const int32_t* __restrict__ rec_off, const float* __restrict__ rec_key, const int32_t* __restrict__ rec_val,
-                int32_t* __restrict__ argmax) {
-  __shared__ float sv[4];
-  __shared__ int si[4];
-  const int b = blockIdx.x, t = threadIdx.x, lane = t & 31, warp = t >> 5;
-  const int r0 = rec_off[b], r1 = rec_off[b + 1];
-  float mv = -FLT_MAX;
-  int mi = 0x7fffffff;
-  for (int r = r0 + t; r < r1; r += 128) {
-    const float v = rec_key[r];
-    if (v > mv) { mv = v; mi = r; }
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    const float ov = __shfl_xor_sync(0xffffffffu, mv, o);
-    const int oi = __shfl_xor_sync(0xffffffffu, mi, o);
-    if (ov > mv || (ov == mv && oi < mi)) { mv = ov; mi = oi; }
-  }
-  if (lane == 0) { sv[warp] = mv; si[warp] = mi; }
-  __syncthreads();
-  if (t == 0) {
-    for (int w = 1; w < 4; ++w)
-      if (sv[w] > mv || (sv[w] == mv && si[w] < mi)) { mv = sv[w]; mi = si[w]; }
-    argmax[b] = mi == 0x7fffffff ? 0 : rec_val[mi];
-  }
-}
-
-struct FusedWs {
-  float* rec_x;
-  float* rec_s;
-  float* rec_key;
-  int32_t* rec_val;
-  int32_t* rec_off;
-  char* pool;
-  size_t pool_bytes, bytes;
-  int64_t nrec;
-};
-static FusedWs fused_ws(void* base, int64_t total_n, int B, int L) {
-  FusedWs w;
-  w.nrec = total_n / REC_ROWS + B;               // = rec_off[B]
-  char* p = static_cast<char*>(base);
-  size_t off = 0;
-  auto take = [&](size_t bytes) {
-    char* q = p + off;
-    off = align_up(off + bytes, 256);
-    return q;
-  };
-  w.rec_x = reinterpret_cast<float*>(take(sizeof(float) * static_cast<size_t>(w.nrec) * L));
-  w.rec_s = reinterpret_cast<float*>(take(sizeof(float) * static_cast<size_t>(w.nrec)));
-  w.rec_key = reinterpret_cast<float*>(take(sizeof(float) * static_cast<size_t>(w.nrec)));
-  w.rec_val = reinterpret_cast<int32_t*>(take(sizeof(int32_t) * static_cast<size_t>(w.nrec)));
-  w.rec_off = reinterpret_cast<int32_t*>(take(sizeof(int32_t) * static_cast<size_t>(B + 1)));
-  w.pool_bytes = pool_ws(nullptr, w.nrec, B, L).bytes;
-  w.pool = take(w.pool_bytes);
-  w.bytes = off;
-  return w;
-}
-
-bool force_simt();
-
 }  // namespace milb200
 
 using namespace milb200;
@@ -658,45 +572,6 @@ int milb200_segment_softmax_pool_fwd(const void* X, const float* scores, const i
                                      argmax, lse, workspace, ws_bytes, st);
   return pool_fwd_t<float>((const float*)X, scores, offsets, B, total_n, L, M, (float*)M_lowp, argmax, lse, workspace,
                            ws_bytes, st);
-}
-
-/* ---- single-pass forward (SURVEY 8f rank 1) ------------------------------------------------------------
- * milb200_gated_score_fwd (with gate_act) + milb200_segment_softmax_pool_fwd in one pass over X: the score GEMM's extra
- * warps reduce every finished tile to softmax-pooling records while it is L2-resident, and the pooling kernel runs over
- * the records (1/32 of the rows).  Same outputs as the two calls; returns MILB200_EUNSUPPORTED (and launches nothing)
- * for shapes / dtypes the fused kernel is not built for — the caller then uses the two calls.                          */
-int milb200_gated_score_pool_supported(int L, int D, int dtype) {
-  return (tc::gated_score_pool_supported(L, D, dtype) && !force_simt()) ? 1 : 0;
-}
-size_t milb200_gated_score_pool_workspace_bytes(int64_t total_n, int B, int L) {
-  if (total_n <= 0 || B <= 0 || L <= 0) return 256;
-  return fused_ws(nullptr, total_n, B, L).bytes;
-}
-int milb200_gated_score_pool_fwd(const void* X, const void* Wcat, const float* bcat, const float* ww, const float* bw,
-                                 const int32_t* offsets, int B, float* scores, void* gate_act, float* M, int32_t* argmax,
-                                 float* lse, int64_t total_n, int L, int D, int dtype, void* workspace, size_t ws_bytes,
-                                 void* stream) {
-  MIL_CHECK_ARG(milb200_gated_score_pool_supported(L, D, dtype), MILB200_EUNSUPPORTED,
-                "gated_score_pool_fwd: not built for L=%d D=%d dtype=%d", L, D, dtype);
-  int rc = pool_check(X, scores, offsets, B, total_n, L, dtype);
-  if (rc) return rc;
-  MIL_CHECK_ARG(Wcat && bcat && ww && bw && gate_act && M, MILB200_EINVAL, "gated_score_pool_fwd: null pointer");
-  MIL_CHECK_ARG(aligned16(Wcat) && aligned16(gate_act), MILB200_EALIGN, "gated_score_pool_fwd: operands must be 16-byte aligned");
-  FusedWs w = fused_ws(workspace, total_n, B, L);
-  MIL_CHECK_ARG(workspace && ws_bytes >= w.bytes, MILB200_EWORKSPACE, "gated_score_pool_fwd: workspace %zu < %zu", ws_bytes, w.bytes);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  k_record_prepare<<<B + 1, 128, 0, st>>>(offsets, B, L, w.rec_off, w.rec_x, w.rec_s, w.rec_key, w.rec_val);
-  MIL_LAUNCH_CHECK();
-  rc = tc::gated_score_pool(X, total_n, L, Wcat, bcat, ww, bw, scores, gate_act, offsets, B, w.rec_x, w.rec_s, w.rec_key,
-                            w.rec_val, st);
-  if (rc) return rc;
-  rc = pool_fwd_t<float>(w.rec_x, w.rec_s, w.rec_off, B, w.nrec, L, M, nullptr, nullptr, lse, w.pool, w.pool_bytes, st);
-  if (rc) return rc;
-  if (argmax) {
-    k_record_argmax<<<B, 128, 0, st>>>(w.rec_off, w.rec_key, w.rec_val, argmax);
-    MIL_LAUNCH_CHECK();
-  }
-  return MILB200_OK;
 }
 
 /* M[b] = sum_i x_i over CSR offsets (no softmax): the reference's dense-batch behaviour (ABMIL.py:56-59 with

@@ -7,11 +7,13 @@
 //                            allocator, warps 4-7 = epilogue.  Epilogues:
 //                              EpiStore   bias + activation (+ rank-1 pooling term) -> bf16/fp32 store
 //                                         (nn.Linear sites: aggregator.py:44,47,66; transformer.py:430-448)
-//                              EpiScore   gated-attention score  (ABMIL.py:52-54), writes 4 B per instance
-//                              EpiDz      its backward: recompute V,U, emit dZ + column sums
+//                              EpiDz      gated-attention backward: recompute V,U, emit dZ + column sums
+//   k_gemm_kmajor_2sm<BN, Epi>  the same on CTA pairs (tcgen05 cta_group::2: one M = 256 MMA, the weight tile
+//                            split between the two CTAs).  Epilogue:
+//                              EpiScoreT  gated-attention score (ABMIL.py:52-54), writes 4 B per instance
+//                                         (+ optionally the gate activations V,U for the backward)
 //   k_gemm_tn                split-K  D[128 x 512] = sum_k A[k, m] B[k, n]  (both operands MN-major):
 //                            dW = dZ^T X of the gate / linear backward.
-#include <cfloat>
 #include <cstdlib>
 
 #include "tc_common.cuh"
@@ -86,8 +88,6 @@ struct EpiCtx {
   int64_t row, M;
   int n0, N, nt, n_tiles, q, half, lane;
   int64_t iter;
-  uint64_t* pfull = nullptr;    // POOL epilogues: score mailbox handshake with the pool warps (two slots)
-  uint64_t* pempty = nullptr;
 };
 
 struct EpiStore {
@@ -112,7 +112,6 @@ struct EpiStore {
   // partial-sector writes per store instruction (the epilogue of a 128 x 256 tile took 5.6 us of a 10 us kernel)
   static constexpr int BOX_BYTES = 32 * 32 * 2;
   static constexpr int STAGING_BYTES = EPI_WARPS * BOX_BYTES;
-  static constexpr int POOL_WARPS = 0;
   __device__ static void prologue(const Params& p, float* esm, int tid) {
     if (p.bias && p.bias_n <= BIAS_CACHE)
       for (int i = tid; i < p.bias_n; i += NUM_THREADS) esm[i] = __ldg(p.bias + i);
@@ -228,14 +227,7 @@ constexpr int GATE_PW = GATE_DH / 2;  // pairs per warp per tile = 48
 // form dZ without re-running this GEMM.  Column order of the saved matrix ("tile-64 order"): gate unit d lives at
 // V -> 128 (d / 64) + d % 64, U -> 128 (d / 64) + 64 + d % 64, i.e. every 128-column tile of the dW GEMM's A operand
 // holds 64 matching (V, U) pairs.  Six [32 rows x 16 cols] TMA-store boxes per warp per half tile.
-//
-// POOL (single-pass forward, SURVEY 8f rank 1): four extra warps turn the scores of every finished 128-row tile into
-// softmax-pooling partials while the tile is still L2-resident — warp w owns rows [32 w, 32 w + 32) of the tile, re-reads
-// them with streaming 128-bit loads (registers only: no shared-memory traffic next to the MMA's) and writes, per
-// (32-row block k, bag b) segment, the record  k + b:  x' = sum_i e^{s_i - m} x_i / l,  s' = m + log l  (l = sum_i e^{s_i - m}).
-// A softmax pool over the records with scores s' is exactly the softmax pool over the instances, so the ordinary pooling
-// kernel finishes the job on ~1/32 of the rows (fp32 records); X is read from HBM once instead of twice.
-template <bool SAVE, bool POOL = false>
+template <bool SAVE>
 struct EpiScoreT {
   struct Params {
     const float* bcat;  // [384] packed order
@@ -243,20 +235,9 @@ struct EpiScoreT {
     const float* bw;    // [1]
     float* scores;
     CUtensorMap tmS;    // SAVE: gate activations [M, 384] bf16; box [32 rows x 48 cols]
-    // POOL
-    const __nv_bfloat16* X;
-    int L;
-    const int32_t* offsets;
-    int B;
-    float* rec_x;       // [records, L]
-    float* rec_s;       // [records]
-    float* rec_key;     // [records] block maximum of the scores (argmax key)
-    int32_t* rec_val;   // [records] index within the bag of the block's first maximum
   };
-  static constexpr int POOL_WARPS = POOL ? 4 : 0;
-  // bias[384] | w[192] | partial[2 parities][4 (h, half)][128 rows] | POOL: score mailbox [2][128]
-  static constexpr int MAIL_OFF = 3 * GATE_D + 2 * 4 * BM;
-  static constexpr int SMEM_FLOATS = MAIL_OFF + (POOL ? 2 * BM : 0);
+  // bias[384] | w[192] | partial[2 parities][4 (h, half)][128 rows]
+  static constexpr int SMEM_FLOATS = 3 * GATE_D + 2 * 4 * BM;
   // staging: ONE [32 x 16] V sub-box + ONE U sub-box per warp (2 KB), recycled for each of the three 16-unit chunks of a
   // half tile.  The main loop is bound by operand supply, so shared memory is better spent on a fifth pipeline stage
   // than on epilogue staging (the epilogue warps wait for the accumulator most of the time anyway).
@@ -337,100 +318,6 @@ struct EpiScoreT {
       if (cx.half == 0) {
         const float sc = ((ps[r] + ps[BM + r]) + (ps[2 * BM + r] + ps[3 * BM + r])) + __ldg(p.bw);
         if (cx.row < cx.M) p.scores[cx.row] = sc;
-        if (POOL) {
-          const int par = static_cast<int>(cx.iter & 1);
-          mbar_wait(cx.pempty + par, static_cast<uint32_t>((cx.iter >> 1) & 1) ^ 1);   // the pool warps took this slot's last tile
-          esm[MAIL_OFF + par * BM + r] = sc;
-          __syncwarp();
-          if (cx.lane == 0) mbar_arrive(cx.pfull + par);
-        }
-      }
-    }
-  }
-  // ---- pool warps (POOL): see the struct comment ----
-  __device__ static void pool_role(const Params& p, const float* esm, uint64_t* pfull, uint64_t* pempty, int w, int lane,
-                                   int rank, int64_t pair0, int64_t n_pairs, int64_t p_tiles, int64_t M) {
-    const int V = p.L / 8;                                   // 16-byte vectors per row (L % 8 == 0, L <= 1024)
-    const uint4* Xv = reinterpret_cast<const uint4*>(p.X);
-    int64_t it = 0;
-    for (int64_t pt = pair0; pt < p_tiles; pt += n_pairs, ++it) {
-      const int64_t row0 = (2 * pt + rank) * BM + 32 * w;
-      const int par = static_cast<int>(it & 1);
-      mbar_wait(pfull + par, static_cast<uint32_t>((it >> 1) & 1));
-      const float s = esm[MAIL_OFF + par * BM + 32 * w + lane];
-      __syncwarp();
-      if (lane == 0) mbar_arrive(pempty + par);              // the value is in a register: the slot may be rewritten
-      if (row0 >= M) continue;
-      const int nrows = (M - row0 < 32) ? static_cast<int>(M - row0) : 32;
-      int b = find_bag(p.offsets, p.B, row0);
-      int r = 0;
-      while (r < nrows) {
-        const int64_t ob = __ldg(p.offsets + b), oe = __ldg(p.offsets + b + 1);
-        const int seg_end = (oe - row0 < nrows) ? static_cast<int>(oe - row0) : nrows;
-        if (seg_end <= r) { ++b; continue; }                 // empty bag (not part of the contract; skip it)
-        const bool valid = lane >= r && lane < seg_end;
-        const float m = warp_max(valid ? s : -FLT_MAX);
-        const float e = valid ? __expf(s - m) : 0.f;
-        const float l = warp_sum(e);
-        const unsigned first = __ballot_sync(0xffffffffu, valid && s == m);
-        float acc[4][8];
-#pragma unroll
-        for (int j = 0; j < 4; ++j)
-#pragma unroll
-          for (int k = 0; k < 8; ++k) acc[j][k] = 0.f;
-        int i = r;
-        for (; i + 3 < seg_end; i += 4) {                    // four rows = 16 128-bit loads per lane in flight
-          uint4 v[4][4];
-#pragma unroll
-          for (int u = 0; u < 4; ++u)
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              const int vec = lane + 32 * j;
-              v[u][j] = vec < V ? ldg_stream(Xv + (row0 + i + u) * V + vec) : make_uint4(0, 0, 0, 0);
-            }
-#pragma unroll
-          for (int u = 0; u < 4; ++u) {
-            const float wu = __shfl_sync(0xffffffffu, e, i + u);
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              float f[8];
-              Vec16<__nv_bfloat16>::unpack(v[u][j], f);
-#pragma unroll
-              for (int k = 0; k < 8; ++k) acc[j][k] = fmaf(wu, f[k], acc[j][k]);
-            }
-          }
-        }
-        for (; i < seg_end; ++i) {
-          const float w0 = __shfl_sync(0xffffffffu, e, i);
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            const int vec = lane + 32 * j;
-            if (vec < V) {
-              float f[8];
-              Vec16<__nv_bfloat16>::unpack(ldg_stream(Xv + (row0 + i) * V + vec), f);
-#pragma unroll
-              for (int k = 0; k < 8; ++k) acc[j][k] = fmaf(w0, f[k], acc[j][k]);
-            }
-          }
-        }
-        const int64_t rec = row0 / 32 + b;
-        const float inv = 1.f / l;
-        float* dst = p.rec_x + rec * p.L;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const int vec = lane + 32 * j;
-          if (vec < V) {
-            *reinterpret_cast<float4*>(dst + vec * 8) = make_float4(acc[j][0] * inv, acc[j][1] * inv, acc[j][2] * inv, acc[j][3] * inv);
-            *reinterpret_cast<float4*>(dst + vec * 8 + 4) = make_float4(acc[j][4] * inv, acc[j][5] * inv, acc[j][6] * inv, acc[j][7] * inv);
-          }
-        }
-        if (lane == 0) {
-          p.rec_s[rec] = m + __logf(l);
-          p.rec_key[rec] = m;
-          p.rec_val[rec] = static_cast<int32_t>(row0 + (__ffs(first) - 1) - ob);
-        }
-        r = seg_end;
-        ++b;
       }
     }
   }
@@ -478,7 +365,6 @@ struct EpiDz {
   static constexpr int SMEM_FLOATS = 3 * GATE_D;
   static constexpr int BOX_BYTES = 32 * GATE_PW * 2;              // one [32 rows x 48 bf16] TMA-store box
   static constexpr int STAGING_BYTES = EPI_WARPS * 2 * BOX_BYTES;  // per warp: dVpre box | dUpre box
-  static constexpr int POOL_WARPS = 0;
   __device__ static void prologue(const Params& p, float* esm, int tid) {
     for (int i = tid; i < 2 * GATE_D; i += NUM_THREADS) esm[i] = __ldg(p.bcat + i);
     for (int i = tid; i < GATE_D; i += NUM_THREADS) esm[2 * GATE_D + i] = __ldg(p.ww + i);
@@ -780,7 +666,7 @@ constexpr size_t kmajor2_smem_bytes() {
 }
 
 template <int BN, class Epi>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS + 32 * Epi::POOL_WARPS, 1)
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1)
 k_gemm_kmajor_2sm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, int64_t M, int N, int K,
                   const __grid_constant__ typename Epi::Params ep) {
   using Cfg = TileCfg<BN>;
@@ -797,11 +683,9 @@ k_gemm_kmajor_2sm(const __grid_constant__ CUtensorMap tmA, const __grid_constant
   uint64_t* tfull_bar = bars + 2 * STAGES;     // [2]       per CTA
   uint64_t* tempty_bar = bars + 2 * STAGES + 2;  // [2]     leader's
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * STAGES + 4);
-  uint64_t* pfull_bar = bars + 2 * STAGES + 5;   // [2] score mailbox filled (pool epilogues only)
-  uint64_t* pempty_bar = pfull_bar + 2;          // [2] score mailbox drained
   uint8_t* staging = smem + STAGES * STAGE_BYTES + BAR_BYTES;
   float* esm = reinterpret_cast<float*>(staging + Epi::STAGING_BYTES);
-  static_assert((2 * STAGES + 9) * 8 <= BAR_BYTES, "barrier block overflow");
+  static_assert((2 * STAGES + 4) * 8 + 8 <= BAR_BYTES, "barrier block overflow");
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t rank = cluster_ctarank();
@@ -823,8 +707,6 @@ k_gemm_kmajor_2sm(const __grid_constant__ CUtensorMap tmA, const __grid_constant
     for (int a = 0; a < 2; ++a) {
       mbar_init(tfull_bar + a, 1);
       mbar_init(tempty_bar + a, 2 * EPI_WARPS);     // one arrival per epilogue warp of BOTH CTAs
-      mbar_init(pfull_bar + a, 4);                  // the four lane-quarter warps that finish a tile's scores
-      mbar_init(pempty_bar + a, 4);                 // the four pool warps
     }
     fence_barrier_init();
   }
@@ -849,9 +731,9 @@ k_gemm_kmajor_2sm(const __grid_constant__ CUtensorMap tmA, const __grid_constant
             uint8_t* sa = stage_base + s * STAGE_BYTES;
             uint8_t* sb = sa + Cfg::A_BYTES;
             if (rank == 0) mbar_arrive_expect_tx(full_bar + s, 2 * STAGE_BYTES);   // both CTAs' bytes land on my barrier
-            // last pass over the tile: evict-first, unless the pool warps are about to re-read it from L2
+            // the A tile is read n_tiles times back to back: keep it in L2 until the last sweep
             tma_load_2d_2sm(sa, &tmA, full_bar + s, kb * BK, static_cast<int32_t>(mt * BM),
-                            Epi::POOL_WARPS > 0 ? kEvictLast : (nt == n_tiles - 1 ? kEvictFirst : kEvictNormal));
+                            nt == n_tiles - 1 ? kEvictFirst : kEvictNormal);
             tma_load_2d_2sm(sb, &tmB, full_bar + s, kb * BK, nt * BN + static_cast<int>(rank) * (BN / 2), kEvictLast);
             if (++s == STAGES) { s = 0; ph ^= 1; }
           }
@@ -894,17 +776,11 @@ k_gemm_kmajor_2sm(const __grid_constant__ CUtensorMap tmA, const __grid_constant
         }
       }
     }
-  } else if (warp >= EPI_WARP0 + EPI_WARPS) {
-    // ===== pool warps (pool epilogues only): pooling partials of every finished tile =====
-    if constexpr (Epi::POOL_WARPS > 0)
-      Epi::pool_role(ep, esm, pfull_bar, pempty_bar, warp - EPI_WARP0 - EPI_WARPS, lane, static_cast<int>(rank), pair0, n_pairs,
-                     p_tiles, M);
   } else if (warp >= EPI_WARP0) {
     // ===== epilogue warps (both CTAs): my 128 rows of the pair's accumulator live in MY tensor memory =====
     const int e = warp - EPI_WARP0;
     Epi epi;
     EpiCtx cx;
-    cx.pfull = pfull_bar; cx.pempty = pempty_bar;
     cx.M = M; cx.N = N; cx.n_tiles = n_tiles; cx.q = e & 3; cx.half = e >> 2; cx.lane = lane;
     int64_t it = 0;
     cx.iter = 0;
@@ -951,18 +827,9 @@ static int launch_kmajor_2sm(const void* A, int64_t M, int K, int64_t lda, const
   MIL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
   const int64_t p_tiles = ((M + BM - 1) / BM + 1) / 2;
   const int pairs = static_cast<int>(p_tiles < sm_count() / 2 ? p_tiles : sm_count() / 2);
-  kern<<<2 * pairs, NUM_THREADS + 32 * Epi::POOL_WARPS, smem, st>>>(tmA, tmB, M, N, K, ep);
+  kern<<<2 * pairs, NUM_THREADS, smem, st>>>(tmA, tmB, M, N, K, ep);
   MIL_LAUNCH_CHECK();
   return MILB200_OK;
-}
-
-static bool gate_2sm() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("MILB200_GATE_2SM");      // default on; =0 selects the single-SM kernel
-    v = (e && e[0] == '0') ? 0 : 1;
-  }
-  return v == 1;
 }
 
 int debug_set_trace(void* dev_ptr) {
@@ -1069,29 +936,11 @@ int gated_score(const void* X, int64_t n, int L, const void* Wcat, const float* 
     ep.bcat = bcat; ep.ww = ww; ep.bw = bw; ep.scores = scores;
     int rc0 = make_tmap_bf16_2d_sw32(&ep.tmS, gate_act, static_cast<uint64_t>(n), 2 * GATE_D, 2 * GATE_D, 32);
     if (rc0) return rc0;
-    if (gate_2sm()) return launch_kmajor_2sm<GATE_BN, EpiScoreT<true>>(X, n, L, L, Wcat, 2 * GATE_D, L, ep, st);
-    return launch_kmajor<GATE_BN, EpiScoreT<true>>(X, n, L, L, Wcat, 2 * GATE_D, L, ep, nullptr, st);
+    return launch_kmajor_2sm<GATE_BN, EpiScoreT<true>>(X, n, L, L, Wcat, 2 * GATE_D, L, ep, st);
   }
   EpiScoreT<false>::Params ep;
   ep.bcat = bcat; ep.ww = ww; ep.bw = bw; ep.scores = scores;
-  if (gate_2sm()) return launch_kmajor_2sm<GATE_BN, EpiScoreT<false>>(X, n, L, L, Wcat, 2 * GATE_D, L, ep, st);
-  return launch_kmajor<GATE_BN, EpiScoreT<false>>(X, n, L, L, Wcat, 2 * GATE_D, L, ep, nullptr, st);
-}
-
-// single-pass forward: scores + saved V,U + softmax-pooling records (see EpiScoreT, POOL)
-bool gated_score_pool_supported(int L, int D, int dtype) {
-  return dtype == MILB200_BF16 && D == GATE_D && L >= 64 && L % 8 == 0 && L <= 1024 && gate_2sm();
-}
-int gated_score_pool(const void* X, int64_t n, int L, const void* Wcat, const float* bcat, const float* ww, const float* bw,
-                     float* scores, void* gate_act, const int32_t* offsets, int B, float* rec_x, float* rec_s,
-                     float* rec_key, int32_t* rec_val, cudaStream_t st) {
-  EpiScoreT<true, true>::Params ep;
-  ep.bcat = bcat; ep.ww = ww; ep.bw = bw; ep.scores = scores;
-  ep.X = static_cast<const __nv_bfloat16*>(X); ep.L = L; ep.offsets = offsets; ep.B = B;
-  ep.rec_x = rec_x; ep.rec_s = rec_s; ep.rec_key = rec_key; ep.rec_val = rec_val;
-  int rc0 = make_tmap_bf16_2d_sw32(&ep.tmS, gate_act, static_cast<uint64_t>(n), 2 * GATE_D, 2 * GATE_D, 32);
-  if (rc0) return rc0;
-  return launch_kmajor_2sm<GATE_BN, EpiScoreT<true, true>>(X, n, L, L, Wcat, 2 * GATE_D, L, ep, st);
+  return launch_kmajor_2sm<GATE_BN, EpiScoreT<false>>(X, n, L, L, Wcat, 2 * GATE_D, L, ep, st);
 }
 
 int gated_dz_max_records() { return sm_count() * EPI_WARPS; }

@@ -20,10 +20,6 @@ bool gemm_store_supported(int64_t M, int N, int K);
 // gate_act (optional): bf16 [n, 384] gate activations V|U in the packed column order, saved for the backward.
 int gated_score(const void* X, int64_t n, int L, const void* Wcat, const float* bcat, const float* ww,
                 const float* bw, float* scores, void* gate_act, cudaStream_t st);
-bool gated_score_pool_supported(int L, int D, int dtype);
-int gated_score_pool(const void* X, int64_t n, int L, const void* Wcat, const float* bcat, const float* ww, const float* bw,
-                     float* scores, void* gate_act, const int32_t* offsets, int B, float* rec_x, float* rec_s,
-                     float* rec_key, int32_t* rec_val, cudaStream_t st);
 
 // Recompute V,U and emit dZ[n, 384] = [dL/dVpre | dL/dUpre] (bf16) for upstream dscores; per-warp column sums
 // (-> dbcat, dww, dbw) are written to colsum_ws[nrec][CS_STRIDE]; *nrec receives the record count.

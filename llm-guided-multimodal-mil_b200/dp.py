@@ -126,18 +126,13 @@ class AbmilTrainer:
             seed = int(torch.randint(0, 2 ** 62, (1,), dtype=torch.int64).item())
             X = F._dropout_raw(X.contiguous(), self.dropout_p, seed, 0)
             mark("dropout")
-        fused = F.gated_scores_pool(X, Wcat, bcat, v["ww"], v["bw"], offsets) if self.save_gate else None
-        if fused is not None:
-            s, act, M, am, _ = fused          # one pass over X: scores, saved V,U and the pool (SURVEY 8f rank 1)
-            mark("gated_score_pool_fwd")
+        if self.save_gate:
+            s, act = F.gated_scores(X, Wcat, bcat, v["ww"], v["bw"], save=True)
         else:
-            if self.save_gate:
-                s, act = F.gated_scores(X, Wcat, bcat, v["ww"], v["bw"], save=True)
-            else:
-                s, act = F.gated_scores(X, Wcat, bcat, v["ww"], v["bw"]), None
-            mark("gated_score_fwd")
-            M, _, am, _ = F.segment_softmax_pool(X, s, offsets)
-            mark("segment_softmax_pool_fwd")
+            s, act = F.gated_scores(X, Wcat, bcat, v["ww"], v["bw"]), None
+        mark("gated_score_fwd")
+        M, _, am, _ = F.segment_softmax_pool(X, s, offsets)
+        mark("segment_softmax_pool_fwd")
         self._saved = (X, offsets, s, act, M, v, seed)
         self.last_argmax, self.last_scores = am, s
         return M

@@ -56,36 +56,6 @@ def gated_scores(X, Wcat, bcat, ww, bw, save=False):
     return (s, act) if save else s
 
 
-def single_pass_enabled():
-    """Opt-in (MILB200_SINGLE_PASS=1): measured slower than the two-kernel forward on B200 (0.71 vs 0.64 ms at cfg 2) — the
-    tile is no longer L2-resident when the pool warps re-read it; DESIGN.md has the ncu figures."""
-    return os.environ.get("MILB200_SINGLE_PASS", "0") == "1"
-
-
-def gated_scores_pool(X, Wcat, bcat, ww, bw, offsets):
-    """Scores, saved gate activations and the softmax pool in ONE pass over X (milb200_gated_score_pool_fwd).
-    Returns (s, act, M, argmax, lse), or None when the fused kernel is not built for this shape / dtype (the caller then
-    uses gated_scores + segment_softmax_pool)."""
-    n, Lf = X.shape
-    D = Wcat.shape[0] // 2
-    code = L.dtype_code(X)
-    lib = L.lib()
-    if not single_pass_enabled() or not lib.milb200_gated_score_pool_supported(Lf, D, code):
-        return None
-    B = offsets.numel() - 1
-    dev = X.device
-    s = torch.empty((n,), dtype=torch.float32, device=dev)
-    act = torch.empty((n, 2 * D), dtype=X.dtype, device=dev)
-    M = torch.empty((B, Lf), dtype=torch.float32, device=dev)
-    am = torch.empty((B,), dtype=torch.int32, device=dev)
-    lse = torch.empty((B,), dtype=torch.float32, device=dev)
-    ws = L.workspace(lib.milb200_gated_score_pool_workspace_bytes(n, B, Lf), dev)
-    L.check(lib.milb200_gated_score_pool_fwd(L.ptr(X), L.ptr(Wcat), L.ptr(bcat), L.ptr(ww), L.ptr(bw), L.ptr(offsets), B,
-                                             L.ptr(s), L.ptr(act), L.ptr(M), L.ptr(am), L.ptr(lse), n, Lf, D, code,
-                                             L.ptr(ws), ws.numel(), L.stream_ptr()), "gated_score_pool_fwd")
-    return s, act, M, am, lse
-
-
 def segment_softmax_pool(X, s, offsets, want_lowp=False):
     """M[b] = sum_i softmax_b(s)_i x_i over CSR offsets.  Returns (M fp32 [B,L], M_lowp|None, argmax int32 [B],
     lse fp32 [B])."""

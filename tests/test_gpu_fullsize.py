@@ -131,12 +131,13 @@ def test_trainer_update_matches_optimizer_oracle(optimizer):
 @pytest.mark.parametrize("total_n,L", [(n, 1024) for n in (1, 2, 127, 128, 129, 255, 256, 257, 383, 385, 512, 513, 1025,
                                                             148 * 256 + 1)] +
                          [(2500, 768), (2500, 512), (777, 256), (3001, 320), (40000, 768)])
-@pytest.mark.parametrize("single_pass", ["0", "1"])
-def test_tile_boundaries_of_the_tensor_core_step(total_n, L, single_pass, monkeypatch):
-    monkeypatch.setenv("MILB200_SINGLE_PASS", single_pass)      # "1": also through the opt-in one-pass forward
+@pytest.mark.parametrize("recompute_gate", ["0", "1"])
+def test_tile_boundaries_of_the_tensor_core_step(total_n, L, recompute_gate):
     """The bench's trainer step (CTA-pair score GEMM with saved V,U, persistent pools, fused dW) at instance counts that
     straddle the 128-row CTA tile, the 256-row pair tile and one full wave of pairs (+1), split into 1-3 ragged bags:
-    pooled vectors, scores, argmax and every parameter gradient against the float64 oracle on the same bf16 operands."""
+    pooled vectors, scores, argmax and every parameter gradient against the float64 oracle on the same bf16 operands.
+    recompute_gate = "1": the trainer saves no gate activations (save_gate=False), so the score GEMM runs without the V,U
+    stores and the backward recomputes them (EpiDz)."""
     from mil_b200.dp import AbmilTrainer
     import mil_b200
     p = mo.procedural_state(mo.abmil_shapes(L), 7)
@@ -148,7 +149,7 @@ def test_tile_boundaries_of_the_tensor_core_step(total_n, L, single_pass, monkey
     g = torch.Generator().manual_seed(total_n)
     X = torch.randn(total_n, L, generator=g).to(torch.bfloat16)
     dM = torch.randn(len(off) - 1, L, generator=g)
-    tr = AbmilTrainer(L, 192, torch.bfloat16, device="cuda")
+    tr = AbmilTrainer(L, 192, torch.bfloat16, device="cuda", save_gate=recompute_gate == "0")
     tr.load_from(m)
     Mt, _ = tr.forward_backward(X.cuda(), torch.from_numpy(off).cuda(), dM.cuda())
     torch.cuda.synchronize()
@@ -176,12 +177,12 @@ def test_tile_boundaries_of_the_tensor_core_step(total_n, L, single_pass, monkey
             assert rel_err(a, b) <= 1e-2, k
 
 
-@pytest.mark.parametrize("single_pass", ["0", "1"])
+@pytest.mark.parametrize("recompute_gate", ["0", "1"])
 @pytest.mark.parametrize("case", ["many_tiny_bags", "one_huge_bag", "huge_then_tiny"])
-def test_extreme_bag_shapes(case, single_pass, monkeypatch):
-    monkeypatch.setenv("MILB200_SINGLE_PASS", single_pass)      # "1": also through the opt-in one-pass forward
+def test_extreme_bag_shapes(case, recompute_gate):
     """Edge cases of the CSR machinery: 3000 bags of 1-3 instances (every CTA slab holds hundreds of bag pieces),
-    one bag spread over every CTA of the persistent pools, and a huge bag followed by tiny ones."""
+    one bag spread over every CTA of the persistent pools, and a huge bag followed by tiny ones.  recompute_gate = "1":
+    the trainer saves no gate activations and the backward recomputes them."""
     from mil_b200.dp import AbmilTrainer
     import mil_b200
     L = 512
@@ -200,7 +201,7 @@ def test_extreme_bag_shapes(case, single_pass, monkeypatch):
     g = torch.Generator().manual_seed(99)
     X = torch.randn(n, L, generator=g).to(torch.bfloat16)
     dM = torch.randn(len(lens), L, generator=g)
-    tr = AbmilTrainer(L, 192, torch.bfloat16, device="cuda")
+    tr = AbmilTrainer(L, 192, torch.bfloat16, device="cuda", save_gate=recompute_gate == "0")
     tr.load_from(m)
     Mt, _ = tr.forward_backward(X.cuda(), torch.from_numpy(off).cuda(), dM.cuda())
     torch.cuda.synchronize()

@@ -125,12 +125,13 @@ def test_cfg2_fullsize_8bag_subset_gradients_vs_oracle():
 # argmax tie rule on EXACT ties
 # ---------------------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
-@pytest.mark.parametrize("single_pass", ["0", "1"])
-def test_argmax_exact_ties_pick_the_first_index(dtype, single_pass, monkeypatch):
+@pytest.mark.parametrize("recompute_gate", ["0", "1"])
+def test_argmax_exact_ties_pick_the_first_index(dtype, recompute_gate, monkeypatch):
     """Duplicated instances have bit-identical scores.  torch.argmax (what the reference's users apply to the attention
     row, and what the float64 oracle restates) returns the FIRST maximal index; the pooling kernel must do the same no
-    matter which warp, CTA slab or bag piece holds the copies."""
-    monkeypatch.setenv("MILB200_SINGLE_PASS", single_pass)
+    matter which warp, CTA slab or bag piece holds the copies.  recompute_gate = "1": the forward keeps no gate
+    activations (the other instantiation of the score kernel)."""
+    monkeypatch.setenv("MILB200_RECOMPUTE_GATE", recompute_gate)
     import mil_b200
     L = 1024 if dtype == torch.bfloat16 else 512
     p = mo.procedural_state(mo.abmil_shapes(L), 5)

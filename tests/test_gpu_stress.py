@@ -24,11 +24,11 @@ def _torch_reference(X, off, Wv, Wu, bv, bu, ww, bw, dM):
     return M.detach(), s.detach(), Wv.grad, Wu.grad
 
 
-@pytest.mark.parametrize("single_pass", ["0", "1"])
+@pytest.mark.parametrize("recompute_gate", ["0", "1"])
 @pytest.mark.parametrize("seed", list(range(24)))
-def test_random_batches_are_repeatable_and_correct(seed, single_pass, monkeypatch):
-    # single_pass = "1": the opt-in one-pass forward (score GEMM + pooling records, milb200_gated_score_pool_fwd)
-    monkeypatch.setenv("MILB200_SINGLE_PASS", single_pass)
+def test_random_batches_are_repeatable_and_correct(seed, recompute_gate):
+    # recompute_gate = "1": no saved gate activations (save_gate=False): score GEMM without the V,U stores, and the
+    # backward recomputes V,U (EpiDz) before the dW GEMM
     import mil_b200
     from mil_b200.dp import AbmilTrainer
     rng = np.random.default_rng(1000 + seed)
@@ -46,7 +46,7 @@ def test_random_batches_are_repeatable_and_correct(seed, single_pass, monkeypatc
     offt = torch.from_numpy(off).cuda()
     outs = []
     for rep in range(2):
-        tr = AbmilTrainer(L, 192, torch.bfloat16, device="cuda")
+        tr = AbmilTrainer(L, 192, torch.bfloat16, device="cuda", save_gate=recompute_gate == "0")
         tr.load_from(m)
         M, _ = tr.forward_backward(X, offt, dM)
         torch.cuda.synchronize()
