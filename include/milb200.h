@@ -67,7 +67,9 @@ size_t milb200_gated_score_workspace_bytes(int64_t total_n, int L, int D, int dt
  * passing it to milb200_gated_score_bwd replaces the recompute GEMM by an elementwise pass (bf16: +0.77 KB/instance of
  * memory for -35 % of the backward time at L = 1024).  fp32 inputs run on the tensor cores as three kind::tf32 MMAs
  * over hi/lo operand splits ("3xTF32", fp32-grade results: <= 1e-5 of the float64 oracle); MILB200_TF32X3=0 in the
- * environment, D % 64 != 0 or L % 16 != 0 select the FFMA kernels.                                                    */
+ * environment, D % 64 != 0 or L % 16 != 0 select the FFMA kernels.  bf16 runs on the tensor cores for D = 192, L >= 64,
+ * L % 16 == 0 (the input-gradient GEMM takes N = L in steps of 16) and on the FFMA kernels otherwise.  The FFMA
+ * backward takes D <= 256.                                                                                             */
 int milb200_gated_score_saves_activations(int L, int D, int dtype);
 int milb200_gated_score_fwd(const void* X, const void* Wcat, const float* bcat, const float* ww,
                             const float* bw, float* scores, void* gate_act, int64_t total_n, int L, int D,
@@ -137,7 +139,8 @@ int milb200_linear_bwd(const void* X, const void* add, const void* W, const void
 
 /* Mixed-precision variant for the head of the fusion path's key stream (fc_pathology, model/aggregator.py:141): X, W bf16
  * on the tensor cores, Y fp32; backward takes fp32 dY (and the fp32 output Y), returns dW / dbias fp32 and dX bf16 (may be
- * NULL).  Tensor-core shapes only (n % 16 == 0, k >= 64, k % 8 == 0).  Workspace (backward only):
+ * NULL).  Tensor-core shapes only (n % 16 == 0, k >= 64, k % 8 == 0; the backward also needs n >= 64 and k % 16 == 0,
+ * since its dX GEMM has N = k and K = n).  Workspace (backward only):
  * milb200_linear_workspace_bytes(m, n, k, MILB200_BF16, 1).                                                          */
 int milb200_linear_f32out_fwd(const void* X, const void* W, const float* bias, float* Y, int64_t m, int n, int k, int act,
                               void* stream);
@@ -312,8 +315,8 @@ int milb200_tape_backward(const milb200_tape_op* ops, int n_ops, const milb200_t
  * outputs: dscores_i = a_i (dM_b . x_i - dM_b . M_b) is computed by extra warps INSIDE the dWcat tensor-core kernel, a few
  * k-blocks ahead of the MMA that consumes it, so X leaves HBM once for the whole backward (the rows the dot products
  * pull into L2 are the rows the kernel's TMA loads read next) and no separate pooling-backward launch exists.
- * dscores fp32[total_n] is written as a by-product.  Unsupported configurations (fp32, D != 192, L > 1024, input
- * gradient wanted): milb200_gated_pool_bwd_supported() == 0 and the caller makes the two calls.                      */
+ * dscores fp32[total_n] is written as a by-product.  Unsupported configurations (fp32, D != 192, L > 1024, L % 16 != 0,
+ * input gradient wanted): milb200_gated_pool_bwd_supported() == 0 and the caller makes the two calls.                */
 int milb200_gated_pool_bwd_supported(int L, int D, int dtype);
 size_t milb200_gated_pool_bwd_workspace_bytes(int64_t total_n, int B, int L, int D);
 int milb200_gated_pool_bwd(const void* X, const float* scores, const int32_t* offsets, int B, const float* dM,

@@ -538,6 +538,11 @@ struct AttPlan {
   int per_cta;      // rows of the big side per CTA
   size_t ws_bytes;  // partial buffers
 };
+// floats of the (max, sum) partials of the many-key forward, rounded up to 16 bytes: the accumulator partials that follow
+// are read as float4 (an odd heads * nq would otherwise leave them 8 bytes off)
+static size_t att_ml_floats(int64_t ctas, int heads, int64_t nq) {
+  return (static_cast<size_t>(ctas) * heads * nq * 2 + 3) / 4 * 4;
+}
 static AttPlan att_plan(int64_t nq, int64_t nk, int heads, int c, int backward) {
   AttPlan p{};
   const int64_t HC = static_cast<int64_t>(heads) * c;
@@ -550,7 +555,7 @@ static AttPlan att_plan(int64_t nq, int64_t nk, int heads, int c, int backward) 
   p.per_cta = static_cast<int>(per);
   p.ctas = static_cast<int>((big + per - 1) / per);
   if (p.t2i) {
-    if (!backward) p.ws_bytes = sizeof(float) * static_cast<size_t>(p.ctas) * heads * nq * (2 + c);
+    if (!backward) p.ws_bytes = sizeof(float) * (att_ml_floats(p.ctas, heads, nq) + static_cast<size_t>(p.ctas) * heads * nq * c);
     else p.ws_bytes = sizeof(float) * static_cast<size_t>(p.ctas) * nq * HC;
   } else {
     p.ws_bytes = backward ? sizeof(float) * static_cast<size_t>(p.ctas) * 2 * nk * HC : 0;
@@ -570,7 +575,7 @@ static int attention_fwd_t(const T* Q, const T* K, const T* V, T* O, float* lse,
    } else {
     MIL_CHECK_ARG(ws && ws_bytes >= p.ws_bytes, MILB200_EWORKSPACE, "attention_fwd: workspace %zu < %zu", ws_bytes, p.ws_bytes);
     float* part_ml = static_cast<float*>(ws);
-    float* part_acc = part_ml + static_cast<size_t>(p.ctas) * heads * nq * 2;
+    float* part_acc = part_ml + att_ml_floats(p.ctas, heads, nq);
     size_t smem = sizeof(float) * (nq * HC + static_cast<size_t>(heads) * 32 * (C + 1));
     auto kern = k_t2i_fwd<T, C>;
     if (smem > 48 * 1024) MIL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));

@@ -388,7 +388,8 @@ static size_t simt_splits(int64_t K) {
 }
 
 static bool tc_gate_ok(int L, int D, int dtype) {
-  return dtype == MILB200_BF16 && D == tc::GATE_D && L >= 64 && L % 8 == 0 && !force_simt();
+  // L % 16: the input-gradient GEMM dX = dZ Wcat (N = L) runs on the tensor-core kernel, which takes N in steps of 16
+  return dtype == MILB200_BF16 && D == tc::GATE_D && L >= 64 && L % 16 == 0 && !force_simt();
 }
 // The tensor-core gate kernels want the packed weight rows in interleaved-halves order (see tc_gemm.cu);
 // milb200_pack_gate_weights asks here so that packer and consumer always agree.
@@ -920,7 +921,7 @@ int milb200_gated_pool_bwd(const void* X, const float* scores, const int32_t* of
   MIL_CHECK_ARG(total_n > 0 && B > 0 && L > 0 && D > 0, MILB200_EINVAL, "gated_pool_bwd: bad shape");
   MIL_CHECK_ARG(total_n < (1ll << 31), MILB200_EINVAL, "gated_pool_bwd: total_n exceeds int32 CSR offsets");
   MIL_CHECK_ARG(milb200_gated_pool_bwd_supported(L, D, dtype), MILB200_EUNSUPPORTED,
-                "gated_pool_bwd: needs bf16, D=%d, L <= 1024 and a multiple of 8 (L=%d D=%d dtype=%d)", tc::GATE_D, L, D, dtype);
+                "gated_pool_bwd: needs bf16, D=%d, L <= 1024 and a multiple of 16 (L=%d D=%d dtype=%d)", tc::GATE_D, L, D, dtype);
   MIL_CHECK_ARG(aligned16(X) && aligned16(gate_act) && aligned16(dscores) && aligned16(dM), MILB200_EALIGN,
                 "gated_pool_bwd: X, gate_act, dscores and dM must be 16-byte aligned");
   cudaStream_t st = static_cast<cudaStream_t>(stream);

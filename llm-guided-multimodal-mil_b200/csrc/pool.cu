@@ -491,7 +491,8 @@ static int pool_fwd_t(const T* X, const float* scores, const int32_t* offsets, i
   const int64_t ctas = (total_n + slab - 1) / slab;
   const size_t smem = sizeof(float) * static_cast<size_t>(POOL_WARPS) * L;
   auto launch = [&](auto kern) -> int {
-    if (smem > 48 * 1024) MIL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    // the kernel's static shared memory (< 1 KB) counts against the same 48 KB default as the dynamic part
+    if (smem + 1024 > 48 * 1024) MIL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kern<<<static_cast<unsigned>(ctas), POOL_THREADS, smem, st>>>(X, scores, offsets, B, total_n, L, V, slab, M, M_lowp,
                                                                  argmax, lse, w.acc, w.ml, w.counters, normalize);
     MIL_LAUNCH_CHECK();
@@ -510,13 +511,13 @@ template <typename T>
 static int pool_bwd_t(const T* X, const float* scores, const int32_t* offsets, int B, int64_t total_n, int L,
                       const float* dM, const float* M, float* dscores, float* attn, void* workspace, size_t ws_bytes,
                       cudaStream_t st) {
+  int V = L * static_cast<int>(sizeof(T)) / 16;
+  int nv = (V + 31) / 32;
+  MIL_CHECK_ARG(nv <= 16, MILB200_EUNSUPPORTED, "pool_bwd: row too long (L=%d)", L);
   PoolWs w = pool_ws(workspace, total_n, B, L);
   MIL_CHECK_ARG(workspace && ws_bytes >= w.bytes, MILB200_EWORKSPACE, "pool_bwd: workspace %zu < %zu", ws_bytes, w.bytes);
   k_pool_bwd_stats<<<B, 1024, 0, st>>>(scores, offsets, L, dM, M, w.stats);
   MIL_LAUNCH_CHECK();
-  int V = L * static_cast<int>(sizeof(T)) / 16;
-  int nv = (V + 31) / 32;
-  MIL_CHECK_ARG(nv <= 16, MILB200_EUNSUPPORTED, "pool_bwd: row too long (L=%d)", L);
   // two CTAs per SM, each a contiguous slab of whole 128-row groups (8 warps x 16 rows)
   int64_t ctas = static_cast<int64_t>(sm_count()) * 2;
   int64_t slab = (total_n + ctas - 1) / ctas;

@@ -51,8 +51,19 @@ def _fro(a, b):
 @pytest.mark.parametrize("nq,nk,c", [(10, 5000, 32), (1, 160, 32), (1, 20000, 32), (16, 333, 32), (5000, 10, 32),
                                      (160, 1, 32), (20000, 1, 32), (10, 10, 64), (1, 1, 64), (7, 17, 32)])
 def test_attention_core_vs_float64(dtype, tol, nq, nk, c):
+    _attention_core_vs_float64(dtype, tol, nq, nk, c, 8)
+
+
+@pytest.mark.parametrize("dtype,tol", [(torch.float32, TOL_F32), (torch.bfloat16, 1e-2)])
+@pytest.mark.parametrize("nq,nk,c", [(10, 5000, 32), (5000, 10, 32), (16, 333, 32), (10, 10, 64), (7, 17, 32)])
+@pytest.mark.parametrize("heads", [1, 3])
+def test_attention_core_few_heads_vs_float64(dtype, tol, nq, nk, c, heads):
+    """The kernels run one warp per head: one and an odd number of heads (CTAs of 32 and 96 threads)."""
+    _attention_core_vs_float64(dtype, tol, nq, nk, c, heads)
+
+
+def _attention_core_vs_float64(dtype, tol, nq, nk, c, H):
     from mil_b200 import functional as F
-    H = 8
     g = torch.Generator(device="cuda").manual_seed(nq * 31 + nk)
     q = torch.randn(nq, H * c, device="cuda", generator=g).to(dtype).requires_grad_(True)
     k = torch.randn(nk, H * c, device="cuda", generator=g).to(dtype).requires_grad_(True)
@@ -78,8 +89,11 @@ def test_attention_rejects_two_large_sides():
 
 
 @pytest.mark.parametrize("dtype,tol", [(torch.float32, TOL_F32), (torch.bfloat16, 1e-2)])
-@pytest.mark.parametrize("m,n,res", [(1, 512, False), (10, 512, True), (5000, 512, True), (77, 64, True), (3, 768, True)])
+@pytest.mark.parametrize("m,n,res", [(1, 512, False), (10, 512, True), (5000, 512, True), (77, 64, True), (3, 768, True),
+                                     (7, 4, True), (5, 8, True), (33, 200, False), (300, 1000, True), (20000, 1024, True)])
 def test_layernorm_vs_float64(dtype, tol, m, n, res):
+    """Widths from one 16-byte vector per row (n = 4 fp32, 8 bf16) to the 1024-element limit, with partial lane groups
+    (n = 200, 1000); rows that are not a multiple of 16 bytes (bf16 n = 4) must be refused."""
     from mil_b200 import functional as F
     g = torch.Generator(device="cuda").manual_seed(m + n)
     x = torch.randn(m, n, device="cuda", generator=g).to(dtype).requires_grad_(True)
@@ -87,6 +101,11 @@ def test_layernorm_vs_float64(dtype, tol, m, n, res):
     ga = (torch.rand(n, device="cuda", generator=g) + 0.5).requires_grad_(True)
     be = torch.randn(n, device="cuda", generator=g).requires_grad_(True)
     dy = torch.randn(m, n, device="cuda", generator=g).to(dtype)
+    if (n * x.element_size()) % 16:
+        import mil_b200
+        with pytest.raises(mil_b200.MilB200Error):
+            F.layernorm(x, ga, be, residual=r)
+        return
     y = F.layernorm(x, ga, be, residual=r)
     (y.float() * dy.float()).sum().backward()
     xd = x.detach().double().requires_grad_(True)
