@@ -117,6 +117,20 @@ int milb200_segment_softmax_pool_bwd(const void* X, const float* scores, const i
                                      float* dscores, float* attn, void* workspace, size_t ws_bytes,
                                      void* stream);
 
+/* The same pair for a caller that knows dM before the forward runs (a training step whose loss gradient does not depend
+ * on M): the forward also writes rowdot[i] = dM_b . x_i (fp32[total_n]) from the rows it streams anyway, and the
+ * backward forms dscores and attn from rowdot without reading X.  M, M_lowp, argmax and lse equal those of
+ * milb200_segment_softmax_pool_fwd, and dscores and attn equal those of milb200_segment_softmax_pool_bwd, bit for bit.
+ * dM, M are [B,L] fp32.  dM, rowdot, dscores and attn must be 4-byte aligned; attn may be NULL.
+ * Workspace of both: milb200_pool_workspace_bytes.                                                      */
+int milb200_segment_softmax_pool_fwd_rowdot(const void* X, const float* scores, const int32_t* offsets, int B,
+                                            int64_t total_n, int L, int dtype, const float* dM, float* M, void* M_lowp,
+                                            int32_t* argmax, float* lse, float* rowdot, void* workspace, size_t ws_bytes,
+                                            void* stream);
+int milb200_segment_softmax_pool_bwd_rowdot(const float* scores, const int32_t* offsets, int B, int64_t total_n, int L,
+                                            const float* dM, const float* M, const float* rowdot, float* dscores,
+                                            float* attn, void* workspace, size_t ws_bytes, void* stream);
+
 /* ---- dense linear layers ------------------------------------------------------------------------
  * Y[m,n] = act(X[m,k] W[n,k]^T + bias[n])  — nn.Linear (+Tanh/ReLU) as used by fc_pathology,
  * fc_CI2CT/fc_CI2Pth (model/aggregator.py:44,47,66), q/k/v/out projections

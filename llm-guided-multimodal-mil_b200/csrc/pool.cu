@@ -23,6 +23,16 @@ template <typename T> __device__ __forceinline__ float exp_t(float x);
 template <> __device__ __forceinline__ float exp_t<float>(float x) { return expf(x); }
 template <> __device__ __forceinline__ float exp_t<__nv_bfloat16>(float x) { return __expf(x); }
 
+// the VN floats of dM_b that line up with 16-byte vector `vec` of a row, from shared memory; 0 past the row (vec >= V)
+template <int VN>
+__device__ __forceinline__ void dm_chunk(const float* dms, int vec, int V, float* d) {
+#pragma unroll
+  for (int k = 0; k < VN; k += 4) {
+    const float4 q = vec < V ? *reinterpret_cast<const float4*>(dms + vec * VN + k) : make_float4(0.f, 0.f, 0.f, 0.f);
+    d[k] = q.x; d[k + 1] = q.y; d[k + 2] = q.z; d[k + 3] = q.w;
+  }
+}
+
 struct PiecePartial {  // published per (CTA, bag) piece
   float m, l;
   int argmax;  // index within the bag
@@ -34,14 +44,22 @@ struct PiecePartial {  // published per (CTA, bag) piece
 // owns the 16-byte vectors j, j+32, ... of a row, two rows in flight — accumulating exp(s_i - max) * x_i in registers,
 // (3) one shared-memory fold across the 8 warps.  A bag inside one slab is finished on the spot; a bag spanning
 // slabs is finished by the CTA that publishes its last piece, folding the partials in piece order (deterministic).
-template <typename T, int NV>
-__global__ void __launch_bounds__(POOL_THREADS)
-k_pool_fwd(const T* __restrict__ X, const float* __restrict__ scores, const int32_t* __restrict__ offsets, int B,
-           int64_t total_n, int L, int V, int64_t slab, float* __restrict__ M, T* __restrict__ M_lowp,
-           int32_t* __restrict__ argmax_out, float* __restrict__ lse_out, float* __restrict__ ws_acc,
-           PiecePartial* __restrict__ ws_ml, unsigned int* __restrict__ counters, int normalize) {
+//
+// ROWDOT: the caller already knows the upstream gradient dM, so the pass also writes rowdot[i] = dM_b . x_i for every
+// row, on the rows it has in registers anyway; the backward then forms the score gradients without reading X again.
+// dM_b is staged once per piece in shared memory next to `red`, and each row's dot is accumulated exactly as k_pool_bwd
+// accumulates it (j then k ascending, masked lanes included in the two-row loop, the same warp_sum), so the gradients do
+// not change by a bit.
+template <typename T, int NV, bool ROWDOT>
+__device__ __forceinline__ void
+pool_fwd_body(const T* __restrict__ X, const float* __restrict__ scores, const int32_t* __restrict__ offsets, int B,
+              int64_t total_n, int L, int V, int64_t slab, float* __restrict__ M, T* __restrict__ M_lowp,
+              int32_t* __restrict__ argmax_out, float* __restrict__ lse_out, float* __restrict__ ws_acc,
+              PiecePartial* __restrict__ ws_ml, unsigned int* __restrict__ counters, int normalize,
+              const float* __restrict__ dM, float* __restrict__ rowdot) {
   constexpr int VN = Vec16<T>::N;
-  extern __shared__ __align__(16) float red[];  // [POOL_WARPS][L]
+  extern __shared__ __align__(16) float red[];  // [POOL_WARPS][L], then (ROWDOT) dM_b [L]
+  float* dms = red + static_cast<int64_t>(POOL_WARPS) * L;
   __shared__ float wred_v[POOL_WARPS];
   __shared__ int wred_i[POOL_WARPS];
   __shared__ float piece_m, piece_l;
@@ -77,6 +95,8 @@ k_pool_fwd(const T* __restrict__ X, const float* __restrict__ scores, const int3
       }
       continue;
     }
+    if (ROWDOT)  // read after the barrier of (1); the previous piece ended with one
+      for (int c = t; c < L; c += POOL_THREADS) dms[c] = __ldg(dM + static_cast<int64_t>(b) * L + c);
 
     // ---- (1) piece max and first argmax ----
     float pm = 0.f;
@@ -134,28 +154,51 @@ k_pool_fwd(const T* __restrict__ X, const float* __restrict__ scores, const int3
           v1[j] = (vec < V) ? ldg_stream(Xv + (rb + i + 1) * V + vec) : make_uint4(0, 0, 0, 0);
         }
         const float w0 = __shfl_sync(0xffffffffu, e, i), w1 = __shfl_sync(0xffffffffu, e, i + 1);
+        float g0 = 0.f, g1 = 0.f;
 #pragma unroll
         for (int j = 0; j < NV; ++j) {
-          float f[VN];
+          float f[VN], d[VN];
+          if (ROWDOT) dm_chunk<VN>(dms, lane + j * 32, V, d);  // one read of dM_b serves both rows
           Vec16<T>::unpack(v0[j], f);
 #pragma unroll
           for (int k = 0; k < VN; ++k) acc[j][k] = fmaf(w0, f[k], acc[j][k]);
+          if (ROWDOT)
+#pragma unroll
+            for (int k = 0; k < VN; ++k) g0 = fmaf(d[k], f[k], g0);
           Vec16<T>::unpack(v1[j], f);
 #pragma unroll
           for (int k = 0; k < VN; ++k) acc[j][k] = fmaf(w1, f[k], acc[j][k]);
+          if (ROWDOT)
+#pragma unroll
+            for (int k = 0; k < VN; ++k) g1 = fmaf(d[k], f[k], g1);
+        }
+        if (ROWDOT) {
+          g0 = warp_sum(g0);
+          g1 = warp_sum(g1);
+          if (lane == 0) { rowdot[rb + i] = g0; rowdot[rb + i + 1] = g1; }
         }
       }
       if (i < nr) {
         const float w0 = __shfl_sync(0xffffffffu, e, i);
+        float g0 = 0.f;
 #pragma unroll
         for (int j = 0; j < NV; ++j) {
           const int vec = lane + j * 32;
           if (vec < V) {
-            float f[VN];
+            float f[VN], d[VN];
             Vec16<T>::unpack(ldg_stream(Xv + (rb + i) * V + vec), f);
 #pragma unroll
             for (int k = 0; k < VN; ++k) acc[j][k] = fmaf(w0, f[k], acc[j][k]);
+            if (ROWDOT) {
+              dm_chunk<VN>(dms, vec, V, d);
+#pragma unroll
+              for (int k = 0; k < VN; ++k) g0 = fmaf(d[k], f[k], g0);
+            }
           }
+        }
+        if (ROWDOT) {
+          g0 = warp_sum(g0);
+          if (lane == 0) rowdot[rb + i] = g0;
         }
       }
     }
@@ -255,13 +298,46 @@ k_pool_fwd(const T* __restrict__ X, const float* __restrict__ scores, const int3
   }
 }
 
+#define MIL_POOL_FWD_PARAMS                                                                                             \
+  const T *__restrict__ X, const float *__restrict__ scores, const int32_t *__restrict__ offsets, int B,               \
+      int64_t total_n, int L, int V, int64_t slab, float *__restrict__ M, T *__restrict__ M_lowp,                      \
+      int32_t *__restrict__ argmax_out, float *__restrict__ lse_out, float *__restrict__ ws_acc,                       \
+      PiecePartial *__restrict__ ws_ml, unsigned int *__restrict__ counters, int normalize
+#define MIL_POOL_FWD_ARGS \
+  X, scores, offsets, B, total_n, L, V, slab, M, M_lowp, argmax_out, lse_out, ws_acc, ws_ml, counters, normalize
+
+template <typename T, int NV>
+__global__ void __launch_bounds__(POOL_THREADS) k_pool_fwd(MIL_POOL_FWD_PARAMS) {
+  pool_fwd_body<T, NV, false>(MIL_POOL_FWD_ARGS, nullptr, nullptr);
+}
+
+// The row dots cost registers (the dM_b chunk, two dots).  Where the plain kernel runs two CTAs per SM (<= 128
+// registers: bf16 NV <= 6, fp32 NV <= 8) the row-dot kernel is held to two as well, so that the HBM-bound pass keeps its
+// bytes in flight; the wider instantiations run one CTA per SM either way.
+template <typename T, int NV>
+constexpr int pool_fwd_rowdot_min_blocks() { return (sizeof(T) == 2 ? NV <= 6 : NV <= 8) ? 2 : 1; }
+
+template <typename T, int NV>
+__global__ void __launch_bounds__(POOL_THREADS, pool_fwd_rowdot_min_blocks<T, NV>())
+k_pool_fwd_rowdot(MIL_POOL_FWD_PARAMS, const float* __restrict__ dM, float* __restrict__ rowdot) {
+  pool_fwd_body<T, NV, true>(MIL_POOL_FWD_ARGS, dM, rowdot);
+}
+#undef MIL_POOL_FWD_PARAMS
+#undef MIL_POOL_FWD_ARGS
+
 // ---- backward ------------------------------------------------------------------------------------
 // stats[b] = (lse_b, dM_b . M_b): softmax statistics are recomputed from the scores, not stored.
+// SWEEP (rowdot[i] = dM_b . x_i, written by the ROWDOT forward): the same CTA then sweeps its bag and writes the score
+// gradients and attention weights: k_pool_bwd's expressions on the same floats, without reading X.  A template flag, so
+// that the statistics-only kernel keeps its registers (two 1024-thread CTAs per SM).
+template <bool SWEEP>
 __global__ void __launch_bounds__(1024)
 k_pool_bwd_stats(const float* __restrict__ scores, const int32_t* __restrict__ offsets, int L,
-                 const float* __restrict__ dM, const float* __restrict__ M, float2* __restrict__ stats) {
+                 const float* __restrict__ dM, const float* __restrict__ M, float2* __restrict__ stats,
+                 const float* __restrict__ rowdot, float* __restrict__ dscores, float* __restrict__ attn) {
   __shared__ float red[32];
   __shared__ float bc;
+  __shared__ float2 bag_stats;
   const int b = blockIdx.x, t = threadIdx.x, lane = t & 31, warp = t >> 5, nt = blockDim.x, nw = blockDim.x >> 5;
   const int64_t ob = offsets[b], oe = offsets[b + 1];
   // the bag's scores stay in registers between the two passes (up to 8 per thread; longer bags re-read from L2)
@@ -307,14 +383,33 @@ k_pool_bwd_stats(const float* __restrict__ scores, const int32_t* __restrict__ o
   if (t == 0) {
     float d = 0.f;
     for (int w = 0; w < nw; ++w) d += red[w];
-    stats[b] = make_float2(oe > ob ? mx + logf(tot) : 0.f, d);
+    bag_stats = make_float2(oe > ob ? mx + logf(tot) : 0.f, d);
+    stats[b] = bag_stats;
+  }
+  if (!SWEEP) return;
+  __syncthreads();
+  const float lse = bag_stats.x, cdot = bag_stats.y;
+#pragma unroll
+  for (int k = 0; k < KEEP; ++k) {
+    const int64_t i = ob + t + static_cast<int64_t>(k) * nt;
+    if (i < oe) {
+      const float a = expf(sc[k] - lse);
+      dscores[i] = a * (rowdot[i] - cdot);
+      if (attn) attn[i] = a;
+    }
+  }
+#pragma unroll 4
+  for (int64_t i = ob + t + static_cast<int64_t>(KEEP) * nt; i < oe; i += nt) {
+    const float a = expf(scores[i] - lse);
+    dscores[i] = a * (rowdot[i] - cdot);
+    if (attn) attn[i] = a;
   }
 }
 
 // (shared with the fused pooling + gate backward, gate.cu)
 int pool_bwd_stats(const float* scores, const int32_t* offsets, int B, int L, const float* dM, const float* M,
                    float2* stats, cudaStream_t st) {
-  k_pool_bwd_stats<<<B, 1024, 0, st>>>(scores, offsets, L, dM, M, stats);
+  k_pool_bwd_stats<false><<<B, 1024, 0, st>>>(scores, offsets, L, dM, M, stats, nullptr, nullptr, nullptr);
   MIL_LAUNCH_CHECK();
   return MILB200_OK;
 }
@@ -477,10 +572,11 @@ static PoolWs pool_ws(void* base, int64_t total_n, int B, int L) {
   return w;
 }
 
+// dM != NULL selects the ROWDOT kernels (rowdot[i] = dM_b . x_i as well)
 template <typename T>
 static int pool_fwd_t(const T* X, const float* scores, const int32_t* offsets, int B, int64_t total_n, int L, float* M,
                       T* M_lowp, int32_t* argmax, float* lse, void* workspace, size_t ws_bytes, cudaStream_t st,
-                      int normalize = 1) {
+                      int normalize = 1, const float* dM = nullptr, float* rowdot = nullptr) {
   const int V = L * static_cast<int>(sizeof(T)) / 16;
   const int nv = (V + 31) / 32;
   MIL_CHECK_ARG(nv <= 16, MILB200_EUNSUPPORTED, "pool: row of %d bytes exceeds the 8 KB limit", L * (int)sizeof(T));
@@ -489,15 +585,27 @@ static int pool_fwd_t(const T* X, const float* scores, const int32_t* offsets, i
   MIL_CUDA(cudaMemsetAsync(w.counters, 0, sizeof(unsigned int) * static_cast<size_t>(B), st));
   const int64_t slab = pool_slab_rows(total_n);
   const int64_t ctas = (total_n + slab - 1) / slab;
-  const size_t smem = sizeof(float) * static_cast<size_t>(POOL_WARPS) * L;
-  auto launch = [&](auto kern) -> int {
+  // per-warp accumulator rows, plus the staged dM_b row of the ROWDOT kernels
+  const size_t smem = sizeof(float) * static_cast<size_t>(POOL_WARPS + (dM ? 1 : 0)) * L;
+  auto launch = [&](auto kern, auto... rowdot_args) -> int {
     // the kernel's static shared memory (< 1 KB) counts against the same 48 KB default as the dynamic part
     if (smem + 1024 > 48 * 1024) MIL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kern<<<static_cast<unsigned>(ctas), POOL_THREADS, smem, st>>>(X, scores, offsets, B, total_n, L, V, slab, M, M_lowp,
-                                                                 argmax, lse, w.acc, w.ml, w.counters, normalize);
+                                                                 argmax, lse, w.acc, w.ml, w.counters, normalize,
+                                                                 rowdot_args...);
     MIL_LAUNCH_CHECK();
     return MILB200_OK;
   };
+  // (the same NV buckets as pool_bwd_t: a row's dot then has the same lane mapping in both kernels)
+  if (dM) {
+    if (nv <= 1) return launch(k_pool_fwd_rowdot<T, 1>, dM, rowdot);
+    if (nv == 2) return launch(k_pool_fwd_rowdot<T, 2>, dM, rowdot);
+    if (nv == 3) return launch(k_pool_fwd_rowdot<T, 3>, dM, rowdot);
+    if (nv == 4) return launch(k_pool_fwd_rowdot<T, 4>, dM, rowdot);
+    if (nv <= 6) return launch(k_pool_fwd_rowdot<T, 6>, dM, rowdot);
+    if (nv <= 8) return launch(k_pool_fwd_rowdot<T, 8>, dM, rowdot);
+    return launch(k_pool_fwd_rowdot<T, 16>, dM, rowdot);
+  }
   if (nv <= 1) return launch(k_pool_fwd<T, 1>);
   if (nv == 2) return launch(k_pool_fwd<T, 2>);
   if (nv == 3) return launch(k_pool_fwd<T, 3>);
@@ -516,7 +624,7 @@ static int pool_bwd_t(const T* X, const float* scores, const int32_t* offsets, i
   MIL_CHECK_ARG(nv <= 16, MILB200_EUNSUPPORTED, "pool_bwd: row too long (L=%d)", L);
   PoolWs w = pool_ws(workspace, total_n, B, L);
   MIL_CHECK_ARG(workspace && ws_bytes >= w.bytes, MILB200_EWORKSPACE, "pool_bwd: workspace %zu < %zu", ws_bytes, w.bytes);
-  k_pool_bwd_stats<<<B, 1024, 0, st>>>(scores, offsets, L, dM, M, w.stats);
+  k_pool_bwd_stats<false><<<B, 1024, 0, st>>>(scores, offsets, L, dM, M, w.stats, nullptr, nullptr, nullptr);
   MIL_LAUNCH_CHECK();
   // two CTAs per SM, each a contiguous slab of whole 128-row groups (8 warps x 16 rows)
   int64_t ctas = static_cast<int64_t>(sm_count()) * 2;
@@ -550,6 +658,8 @@ static int pool_check(const void* X, const float* scores, const int32_t* offsets
   return MILB200_OK;
 }
 
+static bool aligned_f32(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 3u) == 0; }
+
 }  // namespace milb200
 
 using namespace milb200;
@@ -573,6 +683,22 @@ int milb200_segment_softmax_pool_fwd(const void* X, const float* scores, const i
                                      argmax, lse, workspace, ws_bytes, st);
   return pool_fwd_t<float>((const float*)X, scores, offsets, B, total_n, L, M, (float*)M_lowp, argmax, lse, workspace,
                            ws_bytes, st);
+}
+
+int milb200_segment_softmax_pool_fwd_rowdot(const void* X, const float* scores, const int32_t* offsets, int B,
+                                            int64_t total_n, int L, int dtype, const float* dM, float* M, void* M_lowp,
+                                            int32_t* argmax, float* lse, float* rowdot, void* workspace, size_t ws_bytes,
+                                            void* stream) {
+  int rc = pool_check(X, scores, offsets, B, total_n, L, dtype);
+  if (rc) return rc;
+  MIL_CHECK_ARG(M && dM && rowdot, MILB200_EINVAL, "pool_fwd_rowdot: M, dM and rowdot must be non-null");
+  MIL_CHECK_ARG(aligned_f32(dM) && aligned_f32(rowdot), MILB200_EALIGN, "pool_fwd_rowdot: dM and rowdot must be 4-byte aligned");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (dtype == MILB200_BF16)
+    return pool_fwd_t<__nv_bfloat16>((const __nv_bfloat16*)X, scores, offsets, B, total_n, L, M, (__nv_bfloat16*)M_lowp,
+                                     argmax, lse, workspace, ws_bytes, st, 1, dM, rowdot);
+  return pool_fwd_t<float>((const float*)X, scores, offsets, B, total_n, L, M, (float*)M_lowp, argmax, lse, workspace,
+                           ws_bytes, st, 1, dM, rowdot);
 }
 
 /* M[b] = sum_i x_i over CSR offsets (no softmax): the reference's dense-batch behaviour (ABMIL.py:56-59 with
@@ -617,6 +743,24 @@ int milb200_segment_softmax_pool_bwd(const void* X, const float* scores, const i
     return pool_bwd_t<__nv_bfloat16>((const __nv_bfloat16*)X, scores, offsets, B, total_n, L, dM, M, dscores, attn,
                                      workspace, ws_bytes, st);
   return pool_bwd_t<float>((const float*)X, scores, offsets, B, total_n, L, dM, M, dscores, attn, workspace, ws_bytes, st);
+}
+
+int milb200_segment_softmax_pool_bwd_rowdot(const float* scores, const int32_t* offsets, int B, int64_t total_n, int L,
+                                            const float* dM, const float* M, const float* rowdot, float* dscores,
+                                            float* attn, void* workspace, size_t ws_bytes, void* stream) {
+  MIL_CHECK_ARG(scores && offsets && dM && M && rowdot && dscores, MILB200_EINVAL, "pool_bwd_rowdot: null pointer");
+  MIL_CHECK_ARG(aligned_f32(rowdot) && aligned_f32(dscores) && aligned_f32(attn), MILB200_EALIGN,
+                "pool_bwd_rowdot: rowdot, dscores and attn must be 4-byte aligned");
+  MIL_CHECK_ARG(B > 0 && total_n > 0 && L > 0, MILB200_EINVAL, "pool_bwd_rowdot: B=%d total_n=%lld L=%d must be positive",
+                B, (long long)total_n, L);
+  MIL_CHECK_ARG(total_n < (1ll << 31), MILB200_EINVAL, "pool_bwd_rowdot: total_n exceeds int32 CSR offsets");
+  PoolWs w = pool_ws(workspace, total_n, B, L);
+  MIL_CHECK_ARG(workspace && ws_bytes >= w.bytes, MILB200_EWORKSPACE, "pool_bwd_rowdot: workspace %zu < %zu", ws_bytes,
+                w.bytes);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  k_pool_bwd_stats<true><<<B, 1024, 0, st>>>(scores, offsets, L, dM, M, w.stats, rowdot, dscores, attn);
+  MIL_LAUNCH_CHECK();
+  return MILB200_OK;
 }
 
 }  // extern "C"

@@ -111,6 +111,11 @@ class AbmilTrainer:
     # ---- one training step ---------------------------------------------------------------------
     def forward(self, X, offsets):
         """Forward of the pool over one packed CSR batch; keeps what `backward` needs.  Returns M fp32 [B, L]."""
+        return self._forward(X, offsets, None)
+
+    def _forward(self, X, offsets, dM):
+        """`forward`; with the upstream gradient dM already known (forward_backward), the pooling pass also takes the
+        backward's row dots dM_b . x_i from the rows it streams, so that the backward does not read X again."""
         v = self._views(self.params)
         # fp32 master -> compute-dtype operand in the row order the kernels expect (one tiny kernel)
         D = self.D
@@ -131,16 +136,20 @@ class AbmilTrainer:
         else:
             s, act = F.gated_scores(X, Wcat, bcat, v["ww"], v["bw"]), None
         mark("gated_score_fwd")
-        M, _, am, _ = F.segment_softmax_pool(X, s, offsets)
+        if dM is None:
+            M, _, am, _ = F.segment_softmax_pool(X, s, offsets)
+            rowdot = None
+        else:
+            M, _, am, _, rowdot = F.segment_softmax_pool_rowdot(X, s, offsets, dM)
         mark("segment_softmax_pool_fwd")
-        self._saved = (X, offsets, s, act, M, v, seed)
+        self._saved = (X, offsets, s, act, M, v, seed, rowdot)
         self.last_argmax, self.last_scores = am, s
         return M
 
     def backward(self, dM):
         """Backward of the last `forward` given dL/dM [B, L] fp32: parameter gradients go to the flat buffer; returns
         dL/dX (or None when the trainer was built without need_input_grad)."""
-        X, offsets, s, act, M, v, seed = self._saved
+        X, offsets, s, act, M, v, seed, rowdot = self._saved
         self._saved = None
         mark = self.phase_hook or (lambda name: None)
         if act is not None and not self.need_input_grad and F.fused_backward_enabled():
@@ -150,8 +159,13 @@ class AbmilTrainer:
                 self.last_dscores = fused[0]
                 mark("gated_pool_bwd")
                 return None
-        ds, attn = F.segment_softmax_pool_bwd(X, s, offsets, dM, M, want_attn=self.need_input_grad)
-        mark("segment_softmax_pool_bwd")
+        if rowdot is not None:
+            # ds_i = a_i (dM_b . x_i - dM_b . M_b) from the forward's row dots: no pass over X
+            ds, attn = F.segment_softmax_pool_bwd_rowdot(s, offsets, dM, M, rowdot, want_attn=self.need_input_grad)
+            mark("pool_bwd_rowdot")
+        else:
+            ds, attn = F.segment_softmax_pool_bwd(X, s, offsets, dM, M, want_attn=self.need_input_grad)
+            mark("segment_softmax_pool_bwd")
         dX, *_ = F.gated_scores_bwd(X, self._wcat_c, self._bcat_c, v["ww"], v["bw"], ds, attn, dM, offsets,
                                     self.need_input_grad, grad_out=self.grads, gate_act=act)
         mark("gate_bwd")
@@ -164,12 +178,16 @@ class AbmilTrainer:
 
     def forward_backward(self, X, offsets, dM=None):
         """Forward + backward of the pool over one packed CSR batch.  Upstream gradient dM defaults to ones
-        (loss = sum of the pooled vectors).  Returns (M fp32 [B, L], dX or None)."""
-        M = self.forward(X, offsets)
+        (loss = sum of the pooled vectors).  Returns (M fp32 [B, L], dX or None).
+        dM is known before the forward here, so the forward takes the pooling backward's row dots and the backward
+        never re-reads X (one pass over X fewer than `forward` + `backward`, same results bit for bit); the opt-in
+        fused backward (MILB200_FUSED_BWD=1) keeps the two calls."""
         if dM is None:
-            if getattr(self, "_ones", None) is None or self._ones.shape != M.shape:
-                self._ones = torch.ones_like(M)
+            shape = (offsets.numel() - 1, self.L)
+            if getattr(self, "_ones", None) is None or tuple(self._ones.shape) != shape:
+                self._ones = torch.ones(shape, dtype=torch.float32, device=X.device)
             dM = self._ones
+        M = self._forward(X, offsets, None if F.fused_backward_enabled() else dM)
         return M, self.backward(dM)
 
     # ---- latency-optimal exchange: symmetric memory + one kernel (csrc/exchange.cu) ------------------------------------

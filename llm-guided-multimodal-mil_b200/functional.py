@@ -88,6 +88,48 @@ def segment_softmax_pool_bwd(X, s, offsets, dM, M, want_attn):
     return ds, attn
 
 
+def _check_dM(dM, B, Lf):
+    if dM.dtype != torch.float32 or tuple(dM.shape) != (B, Lf):
+        raise L.MilB200Error(f"dM must be fp32 [{B}, {Lf}], got {dM.dtype} {list(dM.shape)}")
+
+
+def segment_softmax_pool_rowdot(X, s, offsets, dM, want_lowp=False):
+    """segment_softmax_pool for a caller that already has dL/dM: the same pass over X also returns
+    rowdot[i] = dM_b . x_i (fp32 [total_n]), which lets segment_softmax_pool_bwd_rowdot skip X.
+    Returns (M, M_lowp|None, argmax, lse, rowdot); the first four equal segment_softmax_pool's bit for bit."""
+    n, Lf = X.shape
+    B = offsets.numel() - 1
+    _check_dM(dM, B, Lf)
+    M = torch.empty((B, Lf), dtype=torch.float32, device=X.device)
+    Ml = torch.empty((B, Lf), dtype=X.dtype, device=X.device) if want_lowp else None
+    am = torch.empty((B,), dtype=torch.int32, device=X.device)
+    lse = torch.empty((B,), dtype=torch.float32, device=X.device)
+    rowdot = torch.empty((n,), dtype=torch.float32, device=X.device)
+    ws = L.workspace(L.lib().milb200_pool_workspace_bytes(n, B, Lf), X.device)
+    L.check(L.lib().milb200_segment_softmax_pool_fwd_rowdot(L.ptr(X), L.ptr(s), L.ptr(offsets), B, n, Lf,
+                                                            L.dtype_code(X), L.ptr(dM), L.ptr(M), L.ptr(Ml), L.ptr(am),
+                                                            L.ptr(lse), L.ptr(rowdot), L.ptr(ws), ws.numel(),
+                                                            L.stream_ptr()),
+            "segment_softmax_pool_fwd_rowdot")
+    return M, Ml, am, lse, rowdot
+
+
+def segment_softmax_pool_bwd_rowdot(s, offsets, dM, M, rowdot, want_attn):
+    """segment_softmax_pool_bwd from the row dots of segment_softmax_pool_rowdot (same dM): no pass over X.
+    Returns (ds, attn|None), equal to segment_softmax_pool_bwd's bit for bit."""
+    n = s.numel()
+    B, Lf = M.shape
+    _check_dM(dM, B, Lf)
+    ds = torch.empty((n,), dtype=torch.float32, device=s.device)
+    attn = torch.empty((n,), dtype=torch.float32, device=s.device) if want_attn else None
+    ws = L.workspace(L.lib().milb200_pool_workspace_bytes(n, B, Lf), s.device)
+    L.check(L.lib().milb200_segment_softmax_pool_bwd_rowdot(L.ptr(s), L.ptr(offsets), B, n, Lf, L.ptr(dM), L.ptr(M),
+                                                            L.ptr(rowdot), L.ptr(ds), L.ptr(attn), L.ptr(ws), ws.numel(),
+                                                            L.stream_ptr()),
+            "segment_softmax_pool_bwd_rowdot")
+    return ds, attn
+
+
 def fused_backward_enabled():
     """MILB200_FUSED_BWD=1 routes the parameter-gradient backward of the gated pool (nn.Module autograd and AbmilTrainer)
     through the mirrored single-pass backward (milb200_gated_pool_bwd).  Built and parity-green; measured at cfg 2 it
