@@ -190,19 +190,22 @@ int milb200_attention_bwd(const void* Q, const void* K, const void* V, const voi
                           int c, int dtype, void* workspace, size_t ws_bytes, void* stream);
 
 /* ---- CLIP-style logits and small losses -----------------------------------------------------------
- * clip/model.py:359-365: logits_per_image = exp(logit_scale) * norm(I) norm(T)^T  ([bi,bt] fp32).    */
+ * clip/model.py:359-365: logits_per_image = exp(logit_scale) * norm(I) norm(T)^T  ([bi,bt] fp32).
+ * d <= 1024, the backward's limit: a wider d is refused here, before anything is launched.           */
 int milb200_clip_logits_fwd(const void* I, const void* T, const float* logit_scale, float* logits,
                             float* inv_norm_i, float* inv_norm_t, int bi, int bt, int d, int dtype,
                             void* stream);
 /* Backward: upstream gradients of logits_per_image ([bi,bt]) and/or logits_per_text ([bt,bi]) — either may be
- * NULL.  dI/dT in `dtype` (may be NULL), dscale[1] = d/d logit_scale (may be NULL).                      */
+ * NULL.  dI/dT in `dtype` (may be NULL), dscale[1] = d/d logit_scale (may be NULL).  One kernel per requested
+ * output; omitted outputs are not written.                                                               */
 int milb200_clip_logits_bwd(const void* I, const void* T, const float* logit_scale, const float* logits,
                             const float* inv_norm_i, const float* inv_norm_t, const float* dlogits_per_image,
                             const float* dlogits_per_text, void* dI, void* dT, float* dscale, int bi, int bt,
                             int d, int dtype, void* stream);
 /* utils.py:277-282 (CLIPloss_v1): logits[i] = out @ feat[:,i,:]^T ([I,b,b]), CE over dim 1 against the
  * identity, mean over I*b.  out[b,d] (dtype), feat[b,I,d] (dtype, frozen).  logits fp32 [I,b,b];
- * lse_ws fp32 [2*I*b] scratch; loss[1]; dout[b,d] fp32 (may be NULL).                                     */
+ * lse_ws fp32 [2*I*b] scratch; loss[1]; dout[b,d] fp32 (may be NULL).  d <= 1024 and b + d <= 12280 (the
+ * feature row and one logits column share 48 KB of shared memory); larger shapes are refused.             */
 int milb200_cliploss_fwd_bwd(const void* out, const void* feat, float* logits, float* lse_ws, float* loss,
                              float* dout, int b, int n_info, int d, int dtype, void* stream);
 /* nn.CosineEmbeddingLoss(a, b, target=+1) (train_ddp.py:102,326): loss[1] = mean_i(1 - cos(a_i, b_i)) and its
@@ -210,7 +213,11 @@ int milb200_cliploss_fwd_bwd(const void* out, const void* feat, float* logits, f
 int milb200_cosine_embedding_fwd_bwd(const void* a, const void* b, float* loss, float* loss_rows_ws, void* da,
                                      void* db, int n, int d, int dtype, void* stream);
 /* sigmoid + BCELoss(mean) of aggregator.py:200 / train_ddp.py:99,319: prob = sigmoid(z),
- * loss = mean BCE(prob, target), dz = (prob - target)/numel.  z,target,prob,dz fp32[n].             */
+ * loss = mean BCE(prob, target) with torch's -100 clamp of both logs, dz = (prob - target)/numel.
+ * z,target,prob,dz fp32[n]; prob, loss and dz may each be NULL.
+ * dz is the derivative of mean BCE(sigmoid(z), target) for every z.  torch's fp32 autograd through sigmoid + BCELoss
+ * agrees only for -27.6 < z < 16.6: where the fp32 prob rounds to 1 (z >= 16.6) it gives 0, because p(1-p) = 0,
+ * and for z <= -27.6 it scales the gradient by p(1-p)/1e-12 (its clamp of the BCE denominator).                  */
 int milb200_sigmoid_bce_fwd_bwd(const float* z, const float* target, float* prob, float* loss, float* dz,
                                 int n, void* stream);
 
@@ -343,8 +350,9 @@ int milb200_gated_pool_bwd(const void* X, const float* scores, const int32_t* of
 int milb200_adam_step(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t n,
                       float lr, float beta1, float beta2, float eps, float weight_decay,
                       float grad_scale, int step, void* stream);
-/* The same update with the step number in device memory (bias corrections computed by the kernel): lets a captured CUDA
- * graph of the whole training step be replayed.  milb200_step_counter_inc adds 1 to the counter (one-thread kernel).   */
+/* The same update with the step number in device memory: lets a captured CUDA graph of the whole training step be
+ * replayed.  Both entry points form the bias corrections 1 - beta^step on the device in one way, so a counter at s
+ * gives the bit-identical result of milb200_adam_step(step = s).  milb200_step_counter_inc adds 1 to the counter (one-thread kernel).   */
 int milb200_adam_step_dev(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, float lr,
                           float beta1, float beta2, float eps, float weight_decay, float grad_scale,
                           const int32_t* step_dev, void* stream);

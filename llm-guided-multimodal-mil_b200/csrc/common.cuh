@@ -140,6 +140,13 @@ __device__ __forceinline__ float tanh_fast(float x) {
 }
 __device__ __forceinline__ float sigmoid_fast(float x) { return fmaf(0.5f, tanh_fast(0.5f * x), 0.5f); }
 
+// Adam's bias correction 1 - beta^step.  Written as -expm1(step * log1p(beta - 1)) (beta - 1 is exact) because
+// 1 - powf(beta, step) cancels: at beta = 0.999, step 2 it keeps only 5 correct digits.  Every Adam kernel computes it
+// here, on the device, so the eager, graphed and fused updates agree bit for bit.
+__device__ __forceinline__ float adam_bias_correction(float beta, int step) {
+  return -expm1f(static_cast<float>(step) * log1pf(beta - 1.f));
+}
+
 // index of the bag that owns global row `row`: largest b with offsets[b] <= row
 __device__ __forceinline__ int find_bag(const int32_t* __restrict__ offsets, int B, int64_t row) {
   int lo = 0, hi = B;  // invariant: offsets[lo] <= row < offsets[hi]

@@ -252,9 +252,13 @@ __global__ void k_ct_tokens_bwd(const T* __restrict__ dtokens, T* __restrict__ d
   dfmap[idx] = from_f32<T>(to_f32<T>(dtokens[static_cast<int64_t>(ti) * c + ci]) / static_cast<float>(hw));
 }
 
+// step_dev != nullptr: the step number is read from device memory (so that a CUDA graph that contains the optimiser
+// can be replayed: the bias corrections must not be baked into the launch parameters); otherwise it is `step`
 __global__ void k_adam(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
                        float* __restrict__ v, int64_t n, float lr, float b1, float b2, float eps, float wd,
-                       float gscale, float bc1, float bc2) {
+                       float gscale, int step, const int32_t* __restrict__ step_dev) {
+  const int s = step_dev ? *step_dev : step;
+  const float bc1 = adam_bias_correction(b1, s), bc2 = adam_bias_correction(b2, s);
   int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   int64_t stride = static_cast<int64_t>(gridDim.x) * blockDim.x;
   for (; i < n; i += stride) {
@@ -265,27 +269,6 @@ __global__ void k_adam(float* __restrict__ p, const float* __restrict__ g, float
     m[i] = mi;
     v[i] = vi;
     float denom = sqrtf(vi) / sqrtf(bc2) + eps;  // torch: (sqrt(v)/sqrt(bias_correction2)) + eps
-    p[i] = pi - (lr / bc1) * (mi / denom);
-  }
-}
-
-// same update with the step number read from device memory (so that a CUDA graph that contains the optimiser can be
-// replayed: the bias corrections must not be baked into the launch parameters)
-__global__ void k_adam_dev(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
-                           int64_t n, float lr, float b1, float b2, float eps, float wd, float gscale,
-                           const int32_t* __restrict__ step_dev) {
-  const float step = static_cast<float>(*step_dev);
-  const float bc1 = 1.f - powf(b1, step), bc2 = 1.f - powf(b2, step);
-  int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
-  int64_t stride = static_cast<int64_t>(gridDim.x) * blockDim.x;
-  for (; i < n; i += stride) {
-    float pi = p[i];
-    float gi = fmaf(wd, pi, g[i] * gscale);
-    float mi = fmaf(b1, m[i], (1.f - b1) * gi);
-    float vi = fmaf(b2, v[i], (1.f - b2) * gi * gi);
-    m[i] = mi;
-    v[i] = vi;
-    float denom = sqrtf(vi) / sqrtf(bc2) + eps;
     p[i] = pi - (lr / bc1) * (mi / denom);
   }
 }
@@ -577,11 +560,9 @@ int milb200_adam_step(float* param, const float* grad, float* exp_avg, float* ex
                       void* stream) {
   MIL_CHECK_ARG(param && grad && exp_avg && exp_avg_sq && n >= 0 && step >= 1, MILB200_EINVAL, "adam_step: bad arguments");
   if (n == 0) return MILB200_OK;
-  float bc1 = 1.f - powf(beta1, static_cast<float>(step));
-  float bc2 = 1.f - powf(beta2, static_cast<float>(step));
   unsigned blocks = static_cast<unsigned>(std::min<int64_t>((n + 255) / 256, 148 * 8));
   k_adam<<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2,
-                                                                eps, weight_decay, grad_scale, bc1, bc2);
+                                                                eps, weight_decay, grad_scale, step, nullptr);
   MIL_LAUNCH_CHECK();
   return MILB200_OK;
 }
@@ -601,8 +582,8 @@ int milb200_adam_step_dev(float* param, const float* grad, float* exp_avg, float
   MIL_CHECK_ARG(param && grad && exp_avg && exp_avg_sq && n >= 0 && step_dev, MILB200_EINVAL, "adam_step_dev: bad arguments");
   if (n == 0) return MILB200_OK;
   unsigned blocks = static_cast<unsigned>(std::min<int64_t>((n + 255) / 256, 148 * 8));
-  k_adam_dev<<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2,
-                                                                    eps, weight_decay, grad_scale, step_dev);
+  k_adam<<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2,
+                                                                eps, weight_decay, grad_scale, 0, step_dev);
   MIL_LAUNCH_CHECK();
   return MILB200_OK;
 }

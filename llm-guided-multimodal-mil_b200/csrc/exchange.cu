@@ -65,13 +65,13 @@ __global__ void __launch_bounds__(XCH_THREADS)
 k_allreduce_update(float* __restrict__ p, float* __restrict__ g_local, float* g_mc, uint32_t* const* __restrict__ pads,
                    const int rank, const int world, const int slot0, float* __restrict__ m, float* __restrict__ v,
                    const int64_t n, const int64_t chunk4, const int optimizer, const float lr, const float b1, const float b2,
-                   const float eps, const float wd, const float gscale, float bc1, float bc2,
+                   const float eps, const float wd, const float gscale, const int step,
                    const int32_t* __restrict__ step_dev) {
-  if (step_dev != nullptr && optimizer == 0) {      // replayable graphs: the step number lives in device memory
-    const float step = static_cast<float>(*step_dev);
-    bc1 = 1.f - powf(b1, step);
-    bc2 = 1.f - powf(b2, step);
-  }
+  // replayable graphs: the step number lives in device memory.  The bias corrections are formed as milb200_adam_step
+  // forms them, so the fused and the separate update agree bit for bit.
+  const int s = (step_dev != nullptr && optimizer == 0) ? *step_dev : step;
+  const float bc1 = optimizer != 0 ? 1.f : adam_bias_correction(b1, s);
+  const float bc2 = optimizer != 0 ? 1.f : adam_bias_correction(b2, s);
   peer_barrier(pads, rank, world, slot0);
   {
     const int64_t lo = rank * chunk4, hi = min((n + 3) / 4, lo + chunk4);
@@ -169,11 +169,9 @@ int milb200_allreduce_update_symm(float* param, float* grad_local, void* grad_mu
     return MILB200_OK;
   }
   int blocks = static_cast<int>(std::min<int64_t>(XCH_MAX_BLOCKS, std::max<int64_t>(1, (n + XCH_THREADS * 8 - 1) / (XCH_THREADS * 8))));
-  const float bc1 = optimizer != 0 ? 1.f : 1.f - powf(beta1, static_cast<float>(step));
-  const float bc2 = optimizer != 0 ? 1.f : 1.f - powf(beta2, static_cast<float>(step));
   k_allreduce_update<<<blocks, XCH_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(
       param, grad_local, static_cast<float*>(grad_multicast), reinterpret_cast<uint32_t* const*>(signal_pads_dev), rank, world,
-      pad_slot0, exp_avg, exp_avg_sq, n, chunk4, optimizer, lr, beta1, beta2, eps, weight_decay, grad_scale, bc1, bc2,
+      pad_slot0, exp_avg, exp_avg_sq, n, chunk4, optimizer, lr, beta1, beta2, eps, weight_decay, grad_scale, step,
       step_dev);
   MIL_LAUNCH_CHECK();
   return MILB200_OK;

@@ -195,6 +195,8 @@ static int ln_ctas(int64_t m) {
 // ---------------------------------------------------------------------------------------------------
 // CLIP cosine logits
 // ---------------------------------------------------------------------------------------------------
+constexpr int CLIP_MAX_D = 1024;  // k_clip_bwd_side: 4 columns per thread of 256
+
 template <typename T>
 __global__ void k_inv_norm(const T* __restrict__ A, int rows, int d, float* __restrict__ inv) {
   const int lane = threadIdx.x & 31;
@@ -232,7 +234,7 @@ k_clip_bwd_side(const T* __restrict__ A, const T* __restrict__ Bm, const float* 
   const int i = blockIdx.x;
   const float sc = expf(ls[0]);
   const float ia = inv_a[i];
-  float g[4] = {0.f, 0.f, 0.f, 0.f};  // d <= 1024 with 256 threads
+  float g[4] = {0.f, 0.f, 0.f, 0.f};  // d <= CLIP_MAX_D with 256 threads
   for (int j = 0; j < nb; ++j) {
     // image side: G[i, j] = dli[i, j] + dlt[j, i]   (dli is [bi, bt], dlt is [bt, bi])
     // text side (transpose): row i is a text row: G^T[i, j] = dli[j, i] + dlt[i, j]
@@ -288,6 +290,7 @@ k_clip_dscale(const float* __restrict__ logits, const float* __restrict__ dli, c
 // CLIPloss_v1: logits[i][r][c] = out[r] . feat[c][i]; CE over r (dim 1) against the identity, mean over I*b
 // ---------------------------------------------------------------------------------------------------
 // one CTA per (i, c) column: logits column, its log-sum-exp, loss contribution
+constexpr size_t CLIPLOSS_STATIC_SMEM = 8 * sizeof(float);  // red[8]
 template <typename T>
 __global__ void __launch_bounds__(256)
 k_cliploss_cols(const T* __restrict__ out, const T* __restrict__ feat, float* __restrict__ logits, float* __restrict__ lse,
@@ -295,7 +298,7 @@ k_cliploss_cols(const T* __restrict__ out, const T* __restrict__ feat, float* __
   extern __shared__ float sm[];  // f[d] | col[b]
   float* f = sm;
   float* col = sm + d;
-  __shared__ float red[8];
+  __shared__ float red[CLIPLOSS_STATIC_SMEM / sizeof(float)];
   const int i = blockIdx.x / b, c = blockIdx.x % b;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   for (int k = threadIdx.x; k < d; k += 256) f[k] = to_f32<T>(feat[(static_cast<int64_t>(c) * n_info + i) * d + k]);
@@ -463,6 +466,8 @@ int milb200_clip_logits_fwd(const void* I, const void* T, const float* logit_sca
                             float* inv_norm_t, int bi, int bt, int d, int dtype, void* stream) {
   MIL_CHECK_ARG(I && T && logit_scale && logits && inv_norm_i && inv_norm_t, MILB200_EINVAL, "clip_logits_fwd: null pointer");
   MIL_CHECK_ARG(bi > 0 && bt > 0 && d > 0, MILB200_EINVAL, "clip_logits_fwd: bad shape");
+  // the backward keeps a row in four registers per thread of a 256-thread CTA: refuse here what it cannot take
+  MIL_CHECK_ARG(d <= CLIP_MAX_D, MILB200_EUNSUPPORTED, "clip_logits_fwd: d=%d > %d unsupported", d, CLIP_MAX_D);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   int64_t pairs = static_cast<int64_t>(bi) * bt;
   if (dtype == MILB200_BF16) {
@@ -487,7 +492,7 @@ int milb200_clip_logits_bwd(const void* I, const void* T, const float* logit_sca
                             int dtype, void* stream) {
   MIL_CHECK_ARG(I && T && logit_scale && logits && inv_norm_i && inv_norm_t, MILB200_EINVAL, "clip_logits_bwd: null pointer");
   MIL_CHECK_ARG(dlogits_per_image || dlogits_per_text, MILB200_EINVAL, "clip_logits_bwd: no upstream gradient");
-  MIL_CHECK_ARG(bi > 0 && bt > 0 && d > 0 && d <= 1024, MILB200_EUNSUPPORTED, "clip_logits_bwd: d=%d unsupported", d);
+  MIL_CHECK_ARG(bi > 0 && bt > 0 && d > 0 && d <= CLIP_MAX_D, MILB200_EUNSUPPORTED, "clip_logits_bwd: d=%d unsupported", d);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (dtype == MILB200_BF16) {
     if (dI) k_clip_bwd_side<__nv_bfloat16><<<bi, 256, 0, st>>>((const __nv_bfloat16*)I, (const __nv_bfloat16*)T, logit_scale,
@@ -503,7 +508,9 @@ int milb200_clip_logits_bwd(const void* I, const void* T, const float* logit_sca
                                                        dlogits_per_image, dlogits_per_text, bt, bi, d, 1, (float*)dT);
   }
   if (dscale) k_clip_dscale<<<1, 256, 0, st>>>(logits, dlogits_per_image, dlogits_per_text, bi, bt, dscale);
-  count_launch(2);
+  const int launched = (dI ? 1 : 0) + (dT ? 1 : 0) + (dscale ? 1 : 0);
+  if (launched == 0) return MILB200_OK;
+  count_launch(launched - 1);
   MIL_LAUNCH_CHECK();
   return MILB200_OK;
 }
@@ -512,10 +519,14 @@ int milb200_cliploss_fwd_bwd(const void* out, const void* feat, float* logits, f
                              int b, int n_info, int d, int dtype, void* stream) {
   MIL_CHECK_ARG(out && feat && logits && lse_ws && loss, MILB200_EINVAL, "cliploss: null pointer");
   MIL_CHECK_ARG(b > 0 && n_info > 0 && d > 0 && d <= 1024, MILB200_EUNSUPPORTED, "cliploss: bad shape b=%d I=%d d=%d", b, n_info, d);
+  // k_cliploss_cols stages feat[c][i] and one logits column in dynamic shared memory, next to its static red[8]; the
+  // two together must fit the 48 KB every launch gets without an opt-in
+  const size_t smem = sizeof(float) * (static_cast<size_t>(d) + b);
+  MIL_CHECK_ARG(smem + CLIPLOSS_STATIC_SMEM <= 48 * 1024, MILB200_EUNSUPPORTED,
+                "cliploss: b + d = %d exceeds %d", b + d, static_cast<int>((48 * 1024 - CLIPLOSS_STATIC_SMEM) / sizeof(float)));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   float* lse = lse_ws;                 // [I*b]
   float* loss_part = lse_ws + n_info * b;  // [I*b]
-  size_t smem = sizeof(float) * (d + b);
   if (dtype == MILB200_BF16) {
     k_cliploss_cols<__nv_bfloat16><<<n_info * b, 256, smem, st>>>((const __nv_bfloat16*)out, (const __nv_bfloat16*)feat, logits,
                                                                   lse, loss_part, b, n_info, d);
