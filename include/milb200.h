@@ -331,19 +331,12 @@ int milb200_tape_backward(const milb200_tape_op* ops, int n_ops, const milb200_t
                           const float* p_f32, float* g_f32, const void* arena, size_t arena_bytes, void* workspace,
                           size_t ws_bytes, int dtype, const milb200_segments* segs, void* stream);
 
-/* ---- mirrored single-pass backward of the gated pool (autograd of ABMIL.py:52-59 in one pass over X) -----------
- * = milb200_segment_softmax_pool_bwd (attn == NULL) + milb200_gated_score_bwd (gate_act given, dX == NULL) with the same
- * outputs: dscores_i = a_i (dM_b . x_i - dM_b . M_b) is computed by extra warps INSIDE the dWcat tensor-core kernel, a few
- * k-blocks ahead of the MMA that consumes it, so X leaves HBM once for the whole backward (the rows the dot products
- * pull into L2 are the rows the kernel's TMA loads read next) and no separate pooling-backward launch exists.
- * dscores fp32[total_n] is written as a by-product.  Unsupported configurations (fp32, D != 192, L > 1024, L % 16 != 0,
- * input gradient wanted): milb200_gated_pool_bwd_supported() == 0 and the caller makes the two calls.                */
+/* ---- single-pass backward of the gated pool: removed ------------------------------------------------------------
+ * The mirrored single-pass backward (the pooling backward inside the dWcat tensor-core kernel) was slower than the
+ * two-call backward once the pooling backward's row dots moved into the pool forward, and was removed (DESIGN §5c).
+ * Always returns 0: callers take the two-call backward, milb200_segment_softmax_pool_bwd (or its _rowdot form) followed
+ * by milb200_gated_score_bwd.                                                                                      */
 int milb200_gated_pool_bwd_supported(int L, int D, int dtype);
-size_t milb200_gated_pool_bwd_workspace_bytes(int64_t total_n, int B, int L, int D);
-int milb200_gated_pool_bwd(const void* X, const float* scores, const int32_t* offsets, int B, const float* dM,
-                           const float* M, const float* ww, const void* gate_act, int64_t total_n, int L, int D,
-                           int dtype, float* dscores, float* dWcat, float* dbcat, float* dww, float* dbw,
-                           void* workspace, size_t ws_bytes, void* stream);
 
 /* ---- optimiser (train_ddp.py:111-118): fused Adam over one flat fp32 buffer -----------------------
  * g is first scaled by grad_scale (1/world after the NCCL sum = DDP's average).                      */

@@ -36,8 +36,6 @@ SIGNATURES = {
     "milb200_gated_score_bwd": (_i, [_p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _i, _i64, _i, _i, _i,
                                      _p, _p, _p, _p, _p, _p, _sz, _p]),
     "milb200_gated_pool_bwd_supported": (_i, [_i, _i, _i]),
-    "milb200_gated_pool_bwd_workspace_bytes": (_sz, [_i64, _i, _i, _i]),
-    "milb200_gated_pool_bwd": (_i, [_p, _p, _p, _i, _p, _p, _p, _p, _i64, _i, _i, _i, _p, _p, _p, _p, _p, _p, _sz, _p]),
     "milb200_profile_enable": (None, [_i]),
     "milb200_debug_trace": (_i, [_p]),
     "milb200_profile_read": (_i, [_p, _i]),

@@ -20,8 +20,6 @@ size_t smallm_ws_bytes(int64_t m, int k);
 int splitk_reduce_gate(const float* part, int splits, int D, int L, int dh, float* out, cudaStream_t st);
 int splitk_reduce_gate64(const float* part, int splits, int D, int L, float* out, cudaStream_t st);
 int transpose2d(const void* in, void* out, int rows, int cols, int dtype, cudaStream_t st);
-int pool_bwd_stats(const float* scores, const int32_t* offsets, int B, int L, const float* dM, const float* M,
-                   float2* stats, cudaStream_t st);
 
 constexpr int64_t SIMT_ROW_CHUNK = 32768;
 
@@ -889,71 +887,8 @@ int milb200_gated_score_bwd(const void* X, const void* Wcat, const float* bcat, 
                               dWcat, dbcat, dww, dbw, (float*)dX, ws, w, st);
 }
 
-// ---- mirrored single-pass backward: pooling backward + gate backward in one pass over X ---------------------
-struct GatePoolBwdWs {
-  size_t gate, stats, total;
-};
-static GatePoolBwdWs gate_pool_bwd_ws(int64_t total_n, int B, int L, int D) {
-  GatePoolBwdWs w{};
-  w.gate = 0;
-  size_t off = gate_ws(total_n, L, D, MILB200_BF16, 1).total;
-  w.stats = align_up(off, 256);
-  off = w.stats + sizeof(float2) * static_cast<size_t>(B);
-  w.total = align_up(off, 256) + 256;
-  return w;
-}
-
-int milb200_gated_pool_bwd_supported(int L, int D, int dtype) {
-  return (tc_gate_ok(L, D, dtype) && tc::gemm_tn_gate_pool_supported(L)) ? 1 : 0;
-}
-
-size_t milb200_gated_pool_bwd_workspace_bytes(int64_t total_n, int B, int L, int D) {
-  if (total_n <= 0 || B <= 0 || L <= 0 || D <= 0) return 256;
-  return gate_pool_bwd_ws(total_n, B, L, D).total;
-}
-
-int milb200_gated_pool_bwd(const void* X, const float* scores, const int32_t* offsets, int B, const float* dM,
-                           const float* M, const float* ww, const void* gate_act, int64_t total_n, int L, int D,
-                           int dtype, float* dscores, float* dWcat, float* dbcat, float* dww, float* dbw, void* workspace,
-                           size_t ws_bytes, void* stream) {
-  MIL_CHECK_ARG(X && scores && offsets && dM && M && ww && gate_act && dscores && dWcat && dbcat && dww && dbw,
-                MILB200_EINVAL, "gated_pool_bwd: null pointer");
-  MIL_CHECK_ARG(total_n > 0 && B > 0 && L > 0 && D > 0, MILB200_EINVAL, "gated_pool_bwd: bad shape");
-  MIL_CHECK_ARG(total_n < (1ll << 31), MILB200_EINVAL, "gated_pool_bwd: total_n exceeds int32 CSR offsets");
-  MIL_CHECK_ARG(milb200_gated_pool_bwd_supported(L, D, dtype), MILB200_EUNSUPPORTED,
-                "gated_pool_bwd: needs bf16, D=%d, L <= 1024 and a multiple of 16 (L=%d D=%d dtype=%d)", tc::GATE_D, L, D, dtype);
-  MIL_CHECK_ARG(aligned16(X) && aligned16(gate_act) && aligned16(dscores) && aligned16(dM), MILB200_EALIGN,
-                "gated_pool_bwd: X, gate_act, dscores and dM must be 16-byte aligned");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  GatePoolBwdWs pw = gate_pool_bwd_ws(total_n, B, L, D);
-  MIL_CHECK_ARG(workspace && ws_bytes >= pw.total, MILB200_EWORKSPACE, "gated_pool_bwd: workspace %zu < %zu", ws_bytes, pw.total);
-  char* ws = static_cast<char*>(workspace);
-  GateWs w = gate_ws(total_n, L, D, dtype, 1);
-  float* colsum = reinterpret_cast<float*>(ws + w.colsum);
-  float* part = reinterpret_cast<float*>(ws + w.part);
-  float2* stats = reinterpret_cast<float2*>(ws + pw.stats);
-  g_prof_n = 0;
-  prof_mark(st);
-  int rc = pool_bwd_stats(scores, offsets, B, L, dM, M, stats, st);
-  if (rc) return rc;
-  tc::TnGatePool gp{};
-  gp.scores = scores;
-  gp.offsets = offsets;
-  gp.B = B;
-  gp.dM = dM;
-  gp.stats = stats;
-  int splits = 0;
-  rc = tc::gemm_tn_gate(gate_act, dscores, ww, X, L, total_n, L, part, &splits, colsum, st, &gp);
-  if (rc) return rc;
-  prof_mark(st);
-  k_colsum_finalize_tn<<<(3 * D + 1 + 255) / 256, 256, 0, st>>>(colsum, splits, tc::gemm_tn_gate_record_floats(), dbcat, dww,
-                                                                dbw, D);
-  MIL_LAUNCH_CHECK();
-  rc = splitk_reduce_gate64(part, splits, D, L, dWcat, st);
-  if (rc) return rc;
-  prof_mark(st);
-  return MILB200_OK;
-}
+// The mirrored single-pass backward was removed (DESIGN §5c): callers take the two-call backward.
+int milb200_gated_pool_bwd_supported(int /*L*/, int /*D*/, int /*dtype*/) { return 0; }
 
 // ---- dense linear ------------------------------------------------------------------------------------
 size_t milb200_linear_workspace_bytes(int64_t m, int n, int k, int dtype, int backward) {

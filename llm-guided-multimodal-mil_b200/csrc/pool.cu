@@ -406,14 +406,6 @@ k_pool_bwd_stats(const float* __restrict__ scores, const int32_t* __restrict__ o
   }
 }
 
-// (shared with the fused pooling + gate backward, gate.cu)
-int pool_bwd_stats(const float* scores, const int32_t* offsets, int B, int L, const float* dM, const float* M,
-                   float2* stats, cudaStream_t st) {
-  k_pool_bwd_stats<false><<<B, 1024, 0, st>>>(scores, offsets, L, dM, M, stats, nullptr, nullptr, nullptr);
-  MIL_LAUNCH_CHECK();
-  return MILB200_OK;
-}
-
 constexpr int BWD_ROWS_PER_WARP = 16;
 
 template <typename T, int NV>

@@ -1107,58 +1107,28 @@ k_gemm_tn(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUten
 // and the 16-byte chunk pc of both boxes), fence the async proxy and release the stage to the MMA warp.  (Fetching
 // V,U with ordinary loads instead serialises: the proxy fence drains the thread's outstanding global loads.)
 // Column sums (-> dbcat, dww, dbw) ride along in registers; CTAs of n-tile 0 publish them per (split, m-tile).
-//
-// Mirrored single-pass backward (TnGatePool::fused): the pooling backward runs INSIDE this kernel.  Eight "g" warps per
-// CTA (two more warpgroups) compute ds_i = a_i (dM_b . x_i - dM_b . M_b) for rows the split consumes a few stages
-// later: the 32-row k-blocks of a split are dealt round-robin to its (m-tile, n-tile) CTAs, g warp (q, hh) takes column
-// quarter q of rows 16 hh .. 16 hh + 15 of its CTA's block (16 loads of 16 bytes per lane in flight, then straight-line
-// dot products and a halving butterfly), the quarters meet in shared memory where warp 2 finishes the rows, and ds
-// goes to HBM.  The V,U producer warp of EVERY CTA of the split reads ds eight blocks at a time and forwards it to
-// shared memory — a word is valid once it differs from the sentinel the launcher filled ds with, so the cross-CTA
-// hand-over needs no flags and no fences.  The g warps run `lead` blocks ahead of their own CTA's V,U producer and warp
-// 2 prefetches the block after that into L2.  All CTAs are co-resident (grid <= SM count, one CTA per SM), which the
-// hand-over relies on; a value that never arrives traps after TNG_SPIN_LIMIT polls instead of hanging.
-// Measured (cfg 2, 671 070 rows): 0.65 ms against 0.23 (k_pool_bwd) + 0.45 ms for the two kernels; ncu shows the g
-// warps limited by the issue rate of one warp per scheduler next to the transform warps (eight g warps with two
-// transform groups instead of three is what made it pay: 0.92 -> 0.65 ms), and X still leaves HBM ~1.7 times (L2 hit
-// rate 43 %: the window between the g read and the three TMA reads does not survive the V,U / X streams of 144 CTAs).
+// Warps: 0 X producer, 1 MMA issuer, 2 TMEM allocator, 3 raw V,U / ds producer, 4.. transform and accumulator epilogue.
+// A variant that also ran the pooling backward inside this kernel was built, measured and removed (DESIGN §5c).
 // ---------------------------------------------------------------------------------------------
 constexpr int TNG_MT = 2 * GATE_D / BM;   // 3 m-tiles of 128 columns = 64 (V, U) pairs each
 constexpr int TNG_REC = 200;              // record: dVpre[64] | dUpre[64] | ds*V*U[64] | sum ds | pad
 constexpr int TNG_ASTAGES = 8;            // A ring (8 KB per stage): raw V,U land and are transformed well ahead of the MMA
 constexpr int TNG_BSTAGES = 4;            // B ring (32 KB per stage)
-constexpr int TNG_BAR_BYTES = 512;
-constexpr int TNG_XW = 8;                 // transform warps: two groups of four alternate over the stages (round 1 used three
-                                          // groups at 111 registers; with the stage ring of 8 and 96 registers two groups keep
-                                          // the pace: 0.447 vs 0.470 ms, and the third group's registers feed the g warps)
-constexpr int TNG_GW = 8;                 // g warps (two more warpgroups): the pooling backward's dot products
+constexpr int TNG_BAR_BYTES = 384;        // a multiple of 128: keeps ds_s 128-byte aligned
+constexpr int TNG_XW = 8;                 // transform warps: two groups of four alternate over the stages (measured: three
+                                          // groups at 111 registers 0.470 ms, two groups at 96 with the stage ring of 8 0.447 ms)
 constexpr int TNG_DS_SLOTS = 32;          // ds ring (stages): refilled eight stages at a time, ahead of the A ring
 constexpr int TNG_DS_CHUNK = 8;
-constexpr int TNG_GBUF = 4;               // buffers of per-quarter partial dot products between the g warps and warp 2
-constexpr uint32_t TNG_SENTINEL = 0xFFFFFFFFu;  // "ds not computed yet" (a NaN payload no arithmetic produces)
-constexpr int TNG_THREADS = (EPI_WARP0 + TNG_XW + TNG_GW) * 32;
-constexpr uint32_t TNG_SPIN_LIMIT = 1u << 26;   // a lost flag traps instead of hanging the GPU
+constexpr int TNG_THREADS = (EPI_WARP0 + TNG_XW) * 32;
 constexpr int TNG_RED_BYTES = static_cast<int>(sizeof(float)) * TNG_XW * 8 * 25;      // 9600: keeps ds_s 128-byte aligned
 constexpr size_t TNG_SMEM = 1024 + static_cast<size_t>(TNG_ASTAGES) * TN_A_BYTES + static_cast<size_t>(TNG_BSTAGES) * TN_B_BYTES +
-                            TNG_BAR_BYTES + TNG_RED_BYTES + TNG_DS_SLOTS * TN_BK * sizeof(float) + TNG_GBUF * 4 * 32 * sizeof(float);
+                            TNG_BAR_BYTES + TNG_RED_BYTES + TNG_DS_SLOTS * TN_BK * sizeof(float);
 static_assert(TNG_SMEM <= 232448 && TNG_RED_BYTES % 128 == 0, "fused dW kernel smem budget");
-
-__device__ __forceinline__ void ld_volatile_v4(const float* p, uint32_t* v) {
-  asm volatile("ld.volatile.global.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]) : "l"(p) : "memory");
-}
-__device__ __forceinline__ uint32_t ld_volatile_u32(const float* p) {
-  uint32_t v;
-  asm volatile("ld.volatile.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ void prefetch_l2_bulk(const void* p, int bytes) {
-  asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(p), "r"(bytes) : "memory");
-}
 
 __global__ void __launch_bounds__(TNG_THREADS, 1)
 k_gemm_tn_gate(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-               const float* ds, const float* __restrict__ ww, int64_t Kr, int No, int n_tiles,
-               int kb_per_split, float* __restrict__ part, float* __restrict__ rec_ws, const TnGatePool gp) {
+               const float* __restrict__ ds, const float* __restrict__ ww, int64_t Kr, int No, int n_tiles,
+               int kb_per_split, float* __restrict__ part, float* __restrict__ rec_ws) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* a_ring = smem;                                          // [TNG_ASTAGES][V box | U box]
@@ -1170,14 +1140,10 @@ k_gemm_tn_gate(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   uint64_t* bfull_bar = bars + 3 * TNG_ASTAGES;
   uint64_t* bempty_bar = bars + 3 * TNG_ASTAGES + TNG_BSTAGES;
   uint64_t* tfull_bar = bars + 3 * TNG_ASTAGES + 2 * TNG_BSTAGES;
-  uint64_t* gfull_bar = tfull_bar + 1;                             // partial dot products of a block written (8 g warps)
-  uint64_t* gempty_bar = gfull_bar + TNG_GBUF;                     // ... and consumed by warp 2
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(gempty_bar + TNG_GBUF);
-  volatile int* prog = reinterpret_cast<volatile int*>(tmem_slot + 2);  // stage the V,U producer is issuing (g-warp throttle)
-  static_assert((3 * TNG_ASTAGES + 2 * TNG_BSTAGES + 1 + 2 * TNG_GBUF) * 8 + 16 <= TNG_BAR_BYTES, "barrier block overflow");
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tfull_bar + 1);
+  static_assert((3 * TNG_ASTAGES + 2 * TNG_BSTAGES + 1) * 8 + 4 <= TNG_BAR_BYTES, "barrier block overflow");
   float* red = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(bars) + TNG_BAR_BYTES);  // [8 warps][8 pc][25]
   float* ds_s = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(red) + TNG_RED_BYTES);   // [TNG_DS_SLOTS][32]
-  float* gpart = ds_s + TNG_DS_SLOTS * TN_BK;                                                  // [2][4 quarters][32 rows]
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   constexpr int Mo = 2 * GATE_D;
@@ -1195,7 +1161,6 @@ k_gemm_tn_gate(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     prefetch_tmap(&tmB);
   }
   if (warp == 1 && lane == 0) {
-    *prog = 0;
     for (int s = 0; s < TNG_ASTAGES; ++s) {
       mbar_init(araw_bar + s, 1);
       mbar_init(afull_bar + s, 4);               // one arrival per warp of the group that transforms the stage
@@ -1206,14 +1171,6 @@ k_gemm_tn_gate(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       mbar_init(bempty_bar + s, 1);
     }
     mbar_init(tfull_bar, 1);
-    for (int s = 0; s < TNG_GBUF; ++s) {
-      mbar_init(gfull_bar + s, TNG_GW);
-      mbar_init(gempty_bar + s, 1);
-    }
-    for (int s = 0; s < TNG_GBUF; ++s) {
-      mbar_init(gfull_bar + s, TNG_GW);
-      mbar_init(gempty_bar + s, 1);
-    }
     fence_barrier_init();
   }
   if (warp == 2) tmem_alloc(tmem_slot, 512);
@@ -1239,65 +1196,46 @@ k_gemm_tn_gate(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   } else if (warp == 3) {
     // ===== raw V,U / ds producer: runs up to TNG_ASTAGES stages ahead of the MMA =====
     // ds goes through the warp's registers into a 32-stage ring, eight stages per refill (one L2 round trip amortised
-    // over eight stages).  In the fused mode a value is valid once it differs from the sentinel the launcher filled the
-    // buffer with: every 32-bit word validates itself, so neither side needs a fence.
-    uint32_t nx[8];
+    // over eight stages); the next chunk's loads are in flight while the current eight stages are issued.
+    float nx[8];
     bool have_next = false;
-    const bool tr = g_trace != nullptr && blockIdx.x == 0 && lane == 0;
-    uint32_t t_refetch = 0, t_aempty = 0, t_chunks = 0;
-    auto fetch = [&](int ii, uint32_t* v) {              // 8 ds values of this lane for the chunk that starts at stage ii
+    auto fetch = [&](int ii, float* v) {                 // 8 ds values of this lane for the chunk that starts at stage ii
       const int nst = (nkb - ii) < TNG_DS_CHUNK ? (nkb - ii) : TNG_DS_CHUNK;
       const int64_t r = (kb0 + ii) * TN_BK + lane * 8;
 #pragma unroll
-      for (int e = 0; e < 8; ++e) v[e] = 0u;
+      for (int e = 0; e < 8; ++e) v[e] = 0.f;
       if (lane < nst * 4) {
         if (r + 7 < Kr) {
-          ld_volatile_v4(ds + r, v);
-          ld_volatile_v4(ds + r + 4, v + 4);
+          const float4 a = __ldg(reinterpret_cast<const float4*>(ds + r));
+          const float4 b = __ldg(reinterpret_cast<const float4*>(ds + r + 4));
+          v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w;
+          v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
         } else {
 #pragma unroll
           for (int e = 0; e < 8; ++e)
-            if (r + e < Kr) v[e] = ld_volatile_u32(ds + r + e);
+            if (r + e < Kr) v[e] = __ldg(ds + r + e);
         }
       }
     };
     for (int i = 0; i < nkb; ++i) {
       if ((i & (TNG_DS_CHUNK - 1)) == 0) {
-        if (gp.fused && lane == 0) *prog = i;
-        uint32_t v[8];
+        float v[8];
         if (have_next) {
 #pragma unroll
           for (int e = 0; e < 8; ++e) v[e] = nx[e];
         } else {
           fetch(i, v);
         }
-        if (gp.fused) {
-          uint32_t spins = 0;
-          for (;;) {
-            bool ready = true;
-#pragma unroll
-            for (int e = 0; e < 8; ++e) ready = ready && (v[e] != TNG_SENTINEL);
-            if (ready) break;
-            __nanosleep(64);
-            if (++spins > TNG_SPIN_LIMIT) asm volatile("trap;");
-            fetch(i, v);
-            ++t_refetch;
-          }
-        }
-        ++t_chunks;
-        uint32_t* dst = reinterpret_cast<uint32_t*>(ds_s) + (i % TNG_DS_SLOTS) * TN_BK + lane * 8;
-        *reinterpret_cast<uint4*>(dst) = make_uint4(v[0], v[1], v[2], v[3]);
-        *reinterpret_cast<uint4*>(dst + 4) = make_uint4(v[4], v[5], v[6], v[7]);
+        float* dst = ds_s + (i % TNG_DS_SLOTS) * TN_BK + lane * 8;
+        *reinterpret_cast<float4*>(dst) = make_float4(v[0], v[1], v[2], v[3]);
+        *reinterpret_cast<float4*>(dst + 4) = make_float4(v[4], v[5], v[6], v[7]);
         __syncwarp();
         have_next = i + TNG_DS_CHUNK < nkb;
         if (have_next) fetch(i + TNG_DS_CHUNK, nx);     // in flight while the next eight stages are issued
       }
       if (lane == 0) {
-        if (gp.fused) *prog = i;
         const int s = i % TNG_ASTAGES;
-        const uint32_t c0 = static_cast<uint32_t>(clock64());
         mbar_wait(aempty_bar + s, static_cast<uint32_t>((i / TNG_ASTAGES) & 1) ^ 1);
-        t_aempty += static_cast<uint32_t>(clock64()) - c0;
         uint8_t* sa = a_ring + s * TN_A_BYTES;
         const int32_t krow = static_cast<int32_t>((kb0 + i) * TN_BK);
         mbar_arrive_expect_tx(araw_bar + s, TN_A_BYTES);   // (release: the ring refill above is visible to the waiters)
@@ -1306,176 +1244,6 @@ k_gemm_tn_gate(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       }
       __syncwarp();
     }
-    if (tr) { g_trace[0] = t_chunks; g_trace[1] = t_refetch; g_trace[2] = t_aempty; }
-  } else if (warp == 2) {
-    // ===== epilogue of the pooling backward (fused mode only): ds of the 32 rows of every block the g warps reduced =====
-    if (gp.fused) {
-      const int tiles_ps = TNG_MT * n_tiles;
-      const int64_t ldb = gp.ldx * 2;                             // row pitch of X in bytes
-      int it = 0;
-      for (int i = tile; i < nkb; i += tiles_ps, ++it) {
-        const int64_t row0 = (kb0 + i) * TN_BK;
-        // the CTA's next block -> L2, so that the g warps' loads pay an L2 hit (one bulk prefetch per 8 KB of rows)
-        if (i + tiles_ps < nkb) {
-          const int64_t rn = row0 + static_cast<int64_t>(tiles_ps) * TN_BK;
-          if (lane < 8 && rn + 4 * lane < Kr && gp.ldx == No) {
-            const int64_t rows = (Kr - (rn + 4 * lane)) < 4 ? (Kr - (rn + 4 * lane)) : 4;
-            prefetch_l2_bulk(reinterpret_cast<const uint8_t*>(gp.X) + (rn + 4 * lane) * ldb, static_cast<int>(rows * ldb));
-          }
-        }
-        const int64_t rr = row0 + lane;
-        float sc = 0.f;
-        float2 st = make_float2(0.f, 0.f);
-        if (rr < Kr) {
-          sc = __ldg(gp.scores + rr);
-          st = __ldg(gp.stats + find_bag(gp.offsets, gp.B, rr));
-        }
-        mbar_wait(gfull_bar + (it % TNG_GBUF), static_cast<uint32_t>((it / TNG_GBUF) & 1));   // the four quarters of block `it`
-        const float* pp = gpart + (it % TNG_GBUF) * (4 * 32);
-        const float g = (pp[lane] + pp[32 + lane]) + (pp[64 + lane] + pp[96 + lane]);
-        __syncwarp();
-        if (lane == 0) mbar_arrive(gempty_bar + (it % TNG_GBUF));                              // buffer free again
-        if (rr < Kr) gp.ds_out[rr] = expf(sc - st.x) * (g - st.y);
-      }
-    }
-  } else if (warp >= EPI_WARP0 + TNG_XW) {
-    // ===== g warps: the pooling backward for the k-blocks this CTA owns (fused mode only) =====
-    // Warp q owns the q-th quarter of the columns (one 16-byte chunk per lane and row: 8 registers of dM instead of
-    // 32), four rounds of eight rows per block, double-buffered in registers: the loads of round r + 1 are in flight
-    // while round r is reduced (eight straight-line dot products and a 9-shuffle halving butterfly).  The four partial
-    // dot products of a row meet in shared memory (a ring of four buffers with full / empty mbarriers), where warp 2 picks
-    // them up, so the g warps wait neither for each other nor for the per-row epilogue.
-    if (gp.fused) {
-      const int gw = warp - (EPI_WARP0 + TNG_XW);
-      const int q = gw & 3, hh = gw >> 2;                          // column quarter, row half of the block
-      const int tiles_ps = TNG_MT * n_tiles;
-      const int V = No >> 3;                                       // 16-byte chunks per row (<= 128)
-      const int vec = q * 32 + lane;
-      const bool col_ok = vec < V;
-      const int64_t ldv = gp.ldx >> 3;
-      const uint4* Xv = reinterpret_cast<const uint4*>(gp.X) + vec;
-      int b = -1;
-      int64_t bag_end = -1;
-      float dm[8];
-      auto load_dm = [&](int bag) {
-        if (vec < V) {
-          const float4 d0 = __ldg(reinterpret_cast<const float4*>(gp.dM + static_cast<int64_t>(bag) * No + vec * 8));
-          const float4 d1 = __ldg(reinterpret_cast<const float4*>(gp.dM + static_cast<int64_t>(bag) * No + vec * 8 + 4));
-          dm[0] = d0.x; dm[1] = d0.y; dm[2] = d0.z; dm[3] = d0.w;
-          dm[4] = d1.x; dm[5] = d1.y; dm[6] = d1.z; dm[7] = d1.w;
-        } else {
-#pragma unroll
-          for (int k = 0; k < 8; ++k) dm[k] = 0.f;
-        }
-      };
-      auto dot8 = [&](const uint4& xv) {
-        float f[8];
-        Vec16<__nv_bfloat16>::unpack(xv, f);
-        float g0 = 0.f, g1 = 0.f;
-#pragma unroll
-        for (int k = 0; k < 8; k += 2) {
-          g0 = fmaf(dm[k], f[k], g0);
-          g1 = fmaf(dm[k + 1], f[k + 1], g1);
-        }
-        return g0 + g1;
-      };
-      auto load8 = [&](uint4* x, int64_t r0) {
-#pragma unroll
-        for (int u = 0; u < 8; ++u)
-          x[u] = (col_ok && r0 + u < Kr) ? ldg_stream(Xv + (r0 + u) * ldv) : make_uint4(0u, 0u, 0u, 0u);
-      };
-      auto reduce8 = [&](const uint4* x, int64_t r0, float* dst) {     // dst[0..8): this quarter's partial sums of rows r0..r0+7
-        float p[8];
-        if (r0 < Kr) {
-          if (b < 0) {
-            b = find_bag(gp.offsets, gp.B, r0);
-            bag_end = __ldg(gp.offsets + b + 1);
-            load_dm(b);
-          }
-          while (r0 >= bag_end) {
-            ++b;
-            bag_end = __ldg(gp.offsets + b + 1);
-            if (r0 < bag_end) load_dm(b);
-          }
-        }
-        if (r0 + 7 < bag_end) {                                   // the 8 rows lie inside one bag (bag_end <= Kr)
-#pragma unroll
-          for (int u = 0; u < 8; ++u) p[u] = dot8(x[u]);
-        } else {                                                  // a bag boundary (or the end of the rows) inside them
-#pragma unroll
-          for (int u = 0; u < 8; ++u) {
-            p[u] = 0.f;
-            if (r0 + u < Kr) {
-              while (r0 + u >= bag_end) {
-                ++b;
-                bag_end = __ldg(gp.offsets + b + 1);
-                if (r0 + u < bag_end) load_dm(b);
-              }
-              p[u] = dot8(x[u]);
-            }
-          }
-        }
-        // 8 row sums over the 32 lanes with a halving butterfly (9 shuffles instead of 40): after three halving steps
-        // lane l holds row 4*b4 + 2*b3 + b2 (bits of l) summed over 8 lanes; two more steps add the remaining four lanes
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-          const bool up = (lane & 16) != 0;
-          const float send = up ? p[k] : p[k + 4];
-          const float keep = up ? p[k + 4] : p[k];
-          p[k] = keep + __shfl_xor_sync(0xffffffffu, send, 16);
-        }
-#pragma unroll
-        for (int k = 0; k < 2; ++k) {
-          const bool up = (lane & 8) != 0;
-          const float send = up ? p[k] : p[k + 2];
-          const float keep = up ? p[k + 2] : p[k];
-          p[k] = keep + __shfl_xor_sync(0xffffffffu, send, 8);
-        }
-        {
-          const bool up = (lane & 4) != 0;
-          const float send = up ? p[0] : p[1];
-          const float keep = up ? p[1] : p[0];
-          p[0] = keep + __shfl_xor_sync(0xffffffffu, send, 4);
-        }
-        p[0] += __shfl_xor_sync(0xffffffffu, p[0], 2);
-        p[0] += __shfl_xor_sync(0xffffffffu, p[0], 1);
-        if ((lane & 3) == 0) dst[lane >> 2] = p[0];
-      };
-      int it = 0;
-      const bool tr = g_trace != nullptr && blockIdx.x == 0 && lane == 0 && gw == 0;
-      uint32_t t_thr = 0, t_rounds = 0, t_fin = 0;
-      for (int i = tile; i < nkb; i += tiles_ps, ++it) {
-        const int64_t row0 = (kb0 + i) * TN_BK + hh * 16;
-        const uint32_t c0 = static_cast<uint32_t>(clock64());
-        {
-          uint32_t spins = 0;
-          const uint32_t prog_addr = smem_u32(const_cast<int*>(prog));
-          for (;;) {
-            int pv;
-            asm volatile("ld.volatile.shared.s32 %0, [%1];" : "=r"(pv) : "r"(prog_addr) : "memory");
-            if (pv + gp.lead >= i) break;
-            __nanosleep(256);
-            if (++spins > TNG_SPIN_LIMIT) asm volatile("trap;");
-          }
-        }
-        const uint32_t c1 = static_cast<uint32_t>(clock64());
-        t_thr += c1 - c0;
-        uint4 xa[8], xb[8];
-        load8(xa, row0);
-        load8(xb, row0 + 8);
-        mbar_wait(gempty_bar + (it % TNG_GBUF), static_cast<uint32_t>((it / TNG_GBUF) & 1) ^ 1);   // buffer consumed
-        float* pp = gpart + (it % TNG_GBUF) * (4 * 32) + q * 32 + hh * 16;
-        const uint32_t c1b = static_cast<uint32_t>(clock64());
-        t_fin += c1b - c1;
-        reduce8(xa, row0, pp);
-        reduce8(xb, row0 + 8, pp + 8);
-        const uint32_t c2 = static_cast<uint32_t>(clock64());
-        t_rounds += c2 - c1b;
-        __syncwarp();
-        if (lane == 0) mbar_arrive(gfull_bar + (it % TNG_GBUF));                               // partials of block `it` written
-      }
-      if (tr) { g_trace[4] = t_thr; g_trace[5] = t_rounds; g_trace[6] = t_fin; g_trace[7] = it; }
-    }
   } else if (warp == 1) {
     if (nkb > 0) {
       constexpr uint32_t idesc = umma_idesc_bf16(BM, 256, 1, 1);
@@ -1483,17 +1251,10 @@ k_gemm_tn_gate(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       const uint32_t d_hi = static_cast<uint32_t>(desc0 >> 32);
       const uint32_t a_lo0 = static_cast<uint32_t>(desc0);
       const uint32_t b_lo0 = a_lo0 + ((TNG_ASTAGES * TN_A_BYTES) >> 4);
-      const bool tr = g_trace != nullptr && blockIdx.x == 0 && lane == 0;
-      uint32_t t_af = 0, t_bf = 0;
-      const uint32_t cs = static_cast<uint32_t>(clock64());
       for (int i = 0; i < nkb; ++i) {
         const int sa = i % TNG_ASTAGES, sb = i % TNG_BSTAGES;
-        const uint32_t c0 = static_cast<uint32_t>(clock64());
         mbar_wait(afull_bar + sa, static_cast<uint32_t>((i / TNG_ASTAGES) & 1));
-        const uint32_t c1 = static_cast<uint32_t>(clock64());
         mbar_wait(bfull_bar + sb, static_cast<uint32_t>((i / TNG_BSTAGES) & 1));
-        t_af += c1 - c0;
-        t_bf += static_cast<uint32_t>(clock64()) - c1;
         tc_fence_after();
         if (elect_one()) {
           const uint32_t ao = a_lo0 + static_cast<uint32_t>(sa) * (TN_A_BYTES >> 4);
@@ -1511,7 +1272,6 @@ k_gemm_tn_gate(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         }
         __syncwarp();
       }
-      if (tr) { g_trace[8] = t_af; g_trace[9] = t_bf; g_trace[10] = static_cast<uint32_t>(clock64()) - cs; g_trace[11] = nkb; }
     }
   } else if (warp >= EPI_WARP0) {
     // ===== in-place V,U -> dV,dU transform (main loop), then the accumulator epilogue =====
@@ -1631,20 +1391,9 @@ k_gemm_tn_gate(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 int gemm_tn_gate_max_records() { return sm_count(); }  // splits * 3 m-tiles <= resident CTAs
 int gemm_tn_gate_record_floats() { return TNG_REC; }
 
-bool gemm_tn_gate_pool_supported(int No) { return No <= 1024 && No % 8 == 0; }
-
-static int tng_lead() {
-  static const int v = [] {
-    const char* e = getenv("MILB200_TNG_LEAD");
-    int x = e ? atoi(e) : 0;
-    return x >= 8 ? x : 24;
-  }();
-  return v;
-}
-
 // part[s][384 (tile-64 order)][No] partial dWcat; rec_ws[splits * 3][TNG_REC] column-sum records
 int gemm_tn_gate(const void* VU, const float* ds, const float* ww, const void* X, int64_t ldx, int64_t Kr, int No,
-                 float* part, int* splits_out, float* rec_ws, cudaStream_t st, const TnGatePool* pool) {
+                 float* part, int* splits_out, float* rec_ws, cudaStream_t st) {
   constexpr int Mo = 2 * GATE_D;
   MIL_CHECK_ARG(gemm_tn_supported(Mo, No), MILB200_EUNSUPPORTED, "tc gemm_tn_gate: unsupported No=%d", No);
   MIL_CHECK_ARG((reinterpret_cast<uintptr_t>(ds) & 15) == 0, MILB200_EALIGN, "tc gemm_tn_gate: ds must be 16-byte aligned");
@@ -1661,23 +1410,9 @@ int gemm_tn_gate(const void* VU, const float* ds, const float* ww, const void* X
   const int kb_per_split = static_cast<int>((total_kb + splits - 1) / splits);
   splits = static_cast<int>((total_kb + kb_per_split - 1) / kb_per_split);
   if (splits_out) *splits_out = splits;
-  TnGatePool gp{};
-  if (pool) {
-    MIL_CHECK_ARG(gemm_tn_gate_pool_supported(No) && ldx % 8 == 0, MILB200_EUNSUPPORTED,
-                  "tc gemm_tn_gate: fused pooling backward needs No <= 1024 (No=%d)", No);
-    // the cross-CTA hand-over of ds needs every CTA resident at once
-    MIL_CHECK_ARG(TNG_MT * n_tiles * splits <= sm_count(), MILB200_EUNSUPPORTED, "tc gemm_tn_gate: grid exceeds the SM count");
-    gp = *pool;
-    gp.X = X;
-    gp.ldx = ldx;
-    gp.ds_out = const_cast<float*>(ds);
-    if (gp.lead < 8) gp.lead = tng_lead();
-    gp.fused = 1;
-    MIL_CUDA(cudaMemsetAsync(gp.ds_out, 0xFF, sizeof(float) * static_cast<size_t>(Kr), st));   // TNG_SENTINEL everywhere
-  }
   MIL_CUDA(cudaFuncSetAttribute(k_gemm_tn_gate, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(TNG_SMEM)));
   k_gemm_tn_gate<<<TNG_MT * n_tiles * splits, TNG_THREADS, TNG_SMEM, st>>>(tmA, tmB, ds, ww, Kr, No, n_tiles, kb_per_split,
-                                                                           part, rec_ws, gp);
+                                                                           part, rec_ws);
   MIL_LAUNCH_CHECK();
   return MILB200_OK;
 }

@@ -34,24 +34,9 @@ int gemm_tn_splitk(const void* A, int64_t lda, const void* B, int64_t ldb, int64
 int gemm_tn_max_splits(int Mo, int No);
 // Gate backward without materialising dZ: dWcat partials from the saved V,U (tile-64 column order), ds and ww; see
 // k_gemm_tn_gate.  part rows are in tile-64 order; rec_ws receives splits*3 column-sum records of record_floats().
-// With `pool` != nullptr the kernel also runs the pooling backward (the mirrored single-pass backward): ds is then an
-// OUTPUT (fp32[Kr], 16-byte aligned) computed from scores, stats[b] = (lse_b, dM_b . M_b) and dM by extra warps of
-// the same kernel.  Needs No <= 1024 (gemm_tn_gate_pool_supported).
-struct TnGatePool {
-  const void* X;            // filled by gemm_tn_gate
-  int64_t ldx;
-  const float* scores;
-  const int32_t* offsets;
-  int B;
-  const float* dM;          // [B, No] fp32
-  const float2* stats;
-  float* ds_out;            // filled by gemm_tn_gate
-  int fused;                // filled by gemm_tn_gate
-  int lead;                 // k-blocks the g warps may run ahead of their CTA's V,U producer (0: default)
-};
+// ds fp32[Kr] must be 16-byte aligned.
 int gemm_tn_gate(const void* VU, const float* ds, const float* ww, const void* X, int64_t ldx, int64_t Kr, int No,
-                 float* part, int* splits, float* rec_ws, cudaStream_t st, const TnGatePool* pool = nullptr);
-bool gemm_tn_gate_pool_supported(int No);
+                 float* part, int* splits, float* rec_ws, cudaStream_t st);
 int gemm_tn_gate_max_records();
 int gemm_tn_gate_record_floats();
 // 3xTF32 tensor-core products for fp32 operands (kind::tf32 MMAs over hi/lo splits, fp32-grade results); operands are

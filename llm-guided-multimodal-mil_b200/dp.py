@@ -152,13 +152,6 @@ class AbmilTrainer:
         X, offsets, s, act, M, v, seed, rowdot = self._saved
         self._saved = None
         mark = self.phase_hook or (lambda name: None)
-        if act is not None and not self.need_input_grad and F.fused_backward_enabled():
-            # mirrored single-pass backward: the pooling backward runs inside the dW kernel (one pass over X)
-            fused = F.gated_pool_bwd(X, s, offsets, dM, M, v["ww"], act, grad_out=self.grads)
-            if fused is not None:
-                self.last_dscores = fused[0]
-                mark("gated_pool_bwd")
-                return None
         if rowdot is not None:
             # ds_i = a_i (dM_b . x_i - dM_b . M_b) from the forward's row dots: no pass over X
             ds, attn = F.segment_softmax_pool_bwd_rowdot(s, offsets, dM, M, rowdot, want_attn=self.need_input_grad)
@@ -180,14 +173,13 @@ class AbmilTrainer:
         """Forward + backward of the pool over one packed CSR batch.  Upstream gradient dM defaults to ones
         (loss = sum of the pooled vectors).  Returns (M fp32 [B, L], dX or None).
         dM is known before the forward here, so the forward takes the pooling backward's row dots and the backward
-        never re-reads X (one pass over X fewer than `forward` + `backward`, same results bit for bit); the opt-in
-        fused backward (MILB200_FUSED_BWD=1) keeps the two calls."""
+        never re-reads X (one pass over X fewer than `forward` + `backward`, same results bit for bit)."""
         if dM is None:
             shape = (offsets.numel() - 1, self.L)
             if getattr(self, "_ones", None) is None or tuple(self._ones.shape) != shape:
                 self._ones = torch.ones(shape, dtype=torch.float32, device=X.device)
             dM = self._ones
-        M = self._forward(X, offsets, None if F.fused_backward_enabled() else dM)
+        M = self._forward(X, offsets, dM)
         return M, self.backward(dM)
 
     # ---- latency-optimal exchange: symmetric memory + one kernel (csrc/exchange.cu) ------------------------------------

@@ -3,8 +3,6 @@ launches on the current CUDA stream; nothing is computed with eager PyTorch ops 
 tiny parameter vectors and views/slices of the gradient buffers."""
 from __future__ import annotations
 
-import os
-
 import torch
 
 from . import _lib as L
@@ -130,43 +128,6 @@ def segment_softmax_pool_bwd_rowdot(s, offsets, dM, M, rowdot, want_attn):
     return ds, attn
 
 
-def fused_backward_enabled():
-    """MILB200_FUSED_BWD=1 routes the parameter-gradient backward of the gated pool (nn.Module autograd and AbmilTrainer)
-    through the mirrored single-pass backward (milb200_gated_pool_bwd).  Built and parity-green; measured at cfg 2 it
-    saves 0.03 ms of a 1.33 ms step (0.65 vs 0.68 ms for the backward), so the two-kernel backward — whose kernels each
-    sit at their own roofline — stays the default."""
-    return os.environ.get("MILB200_FUSED_BWD", "0") == "1"
-
-
-def gated_pool_bwd(X, s, offsets, dM, M, ww, gate_act, grad_out=None):
-    """Pooling backward + gate backward in ONE pass over X (milb200_gated_pool_bwd): parameter gradients only.
-    Returns (ds, dWcat, dbcat, dww, dbw), or None when the fused kernel does not cover the shape / dtype (the caller
-    then uses segment_softmax_pool_bwd + gated_scores_bwd)."""
-    n, Lf = X.shape
-    D = gate_act.shape[1] // 2
-    code = L.dtype_code(X)
-    lib = L.lib()
-    if not lib.milb200_gated_pool_bwd_supported(Lf, D, code):
-        return None
-    B = offsets.numel() - 1
-    need = 2 * D * Lf + 2 * D + D + 1
-    if grad_out is None:
-        grad_out = torch.empty((need,), dtype=torch.float32, device=X.device)
-    elif grad_out.numel() != need or grad_out.dtype != torch.float32:
-        raise L.MilB200Error("gated_pool_bwd: grad_out must be fp32 with 2D*L+3D+1 elements")
-    dWcat = grad_out[:2 * D * Lf].view(2 * D, Lf)
-    dbcat = grad_out[2 * D * Lf:2 * D * Lf + 2 * D]
-    dww = grad_out[2 * D * Lf + 2 * D:2 * D * Lf + 3 * D]
-    dbw = grad_out[2 * D * Lf + 3 * D:]
-    ds = torch.empty((n,), dtype=torch.float32, device=X.device)
-    dM = dM.contiguous()
-    ws = L.workspace(lib.milb200_gated_pool_bwd_workspace_bytes(n, B, Lf, D), X.device)
-    L.check(lib.milb200_gated_pool_bwd(L.ptr(X), L.ptr(s), L.ptr(offsets), B, L.ptr(dM), L.ptr(M), L.ptr(ww),
-                                       L.ptr(gate_act), n, Lf, D, code, L.ptr(ds), L.ptr(dWcat), L.ptr(dbcat),
-                                       L.ptr(dww), L.ptr(dbw), L.ptr(ws), ws.numel(), L.stream_ptr()), "gated_pool_bwd")
-    return ds, dWcat, dbcat, dww, dbw
-
-
 def gated_scores_bwd(X, Wcat, bcat, ww, bw, ds, attn, dM, offsets, need_dx, grad_out=None, gate_act=None):
     """Backward of gated_scores (+ the pooling term of dX).  `grad_out`, if given, is a flat fp32 buffer of
     2D*L + 2D + D + 1 elements (laid out dWcat | dbcat | dww | dbw) that the kernels write in place — the
@@ -222,14 +183,9 @@ class _AbmilPoolCSR(torch.autograd.Function):
         D = ctx.D
         need_dx = ctx.needs_input_grad[0]
         dM = _f32(dM_out).contiguous()
-        fused = (gated_pool_bwd(X, s, offsets, dM, M, wwf, act)
-                 if (act is not None and not need_dx and fused_backward_enabled()) else None)
-        if fused is not None:
-            dX, (_, dWcat, dbcat, dww, dbw) = None, fused      # one pass over X (mirrored single-pass backward)
-        else:
-            ds, attn = segment_softmax_pool_bwd(X, s, offsets, dM, M, want_attn=need_dx)
-            dX, dWcat, dbcat, dww, dbw = gated_scores_bwd(X, Wcat, bcat, wwf, bwf, ds, attn, dM, offsets, need_dx,
-                                                          gate_act=act)
+        ds, attn = segment_softmax_pool_bwd(X, s, offsets, dM, M, want_attn=need_dx)
+        dX, dWcat, dbcat, dww, dbw = gated_scores_bwd(X, Wcat, bcat, wwf, bwf, ds, attn, dM, offsets, need_dx,
+                                                      gate_act=act)
         dt = ctx.param_dtypes
         return (dX, None, dWcat[:D].to(dt[0]), dbcat[:D].to(dt[1]), dWcat[D:].to(dt[2]), dbcat[D:].to(dt[3]),
                 dww.view(1, D).to(dt[4]), dbw.view(1).to(dt[5]), None)

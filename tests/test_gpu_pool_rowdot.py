@@ -3,8 +3,9 @@
 
 The row-dot forward must return the plain forward's M, M_lowp, argmax and lse, and the row-dot backward the plain
 backward's ds and attn, bit for bit, at every vector width the pool kernels are instantiated for and on bag layouts that
-straddle their row slabs or hold empty bags.  forward_backward(X, offsets, dM) must give the same gradients, dX, scores
-and argmax as forward() followed by backward(dM), which keeps the two-pass backward."""
+straddle their row slabs or hold empty bags; empty bags change no output or gradient of the other bags.
+forward_backward(X, offsets, dM) must give the same gradients, dX, scores and argmax as forward() followed by
+backward(dM), which keeps the two-pass backward."""
 import ctypes as C
 
 import numpy as np
@@ -132,6 +133,44 @@ def test_rowdot_pool_rejects_null_and_misaligned_pointers(F):
     _expect_rejected(F, lambda: F.segment_softmax_pool_rowdot(Xw, s, offt, torch.randn(B, 4104, device="cuda")))
 
 
+@pytest.mark.parametrize("dtype", [torch.bfloat16, torch.float32])
+def test_empty_bags_have_defined_outputs_and_zero_gradient_share(F, dtype):
+    """Zero-length bags at the start, in the middle (also exactly on a slab boundary of the persistent pool kernel) and at
+    the end of a packed batch: pooled vector 0, argmax -1, lse -inf; the other bags and every gradient are what the batch
+    without the empty bags gives, through the pooling backward and the gate backward (with and without dX)."""
+    L, D = 1024, 192
+    lens_full = [0, 0, 700, 0, 4096, 0, 33, 0]
+    lens = [l for l in lens_full if l > 0]
+    off_full = _csr(lens_full)
+    off = _csr(lens)
+    gen = torch.Generator(device="cuda").manual_seed(13)
+    X = torch.randn(sum(lens), L, device="cuda", generator=gen).to(dtype)
+    Wv = torch.randn(D, L, device="cuda", generator=gen) * 0.03
+    Wu = torch.randn(D, L, device="cuda", generator=gen) * 0.03
+    bv = torch.zeros(D, device="cuda")
+    ww = torch.randn(D, device="cuda", generator=gen) * 0.3
+    bw = torch.zeros(1, device="cuda")
+    Wcat, bcat = F.pack_gate_weights(Wv, bv, Wu, bv, dtype)
+    s, act = F.gated_scores(X, Wcat, bcat, ww, bw, save=True)
+    M, _, am, lse = F.segment_softmax_pool(X, s, off)
+    Mf, _, amf, lsef = F.segment_softmax_pool(X, s, off_full)
+    keep = torch.tensor([i for i, l in enumerate(lens_full) if l > 0], device="cuda")
+    gone = torch.tensor([i for i, l in enumerate(lens_full) if l == 0], device="cuda")
+    assert torch.equal(Mf[keep], M) and torch.equal(amf[keep], am) and torch.equal(lsef[keep], lse)
+    assert float(Mf[gone].abs().max()) == 0.0 and bool((amf[gone] == -1).all()) and bool(torch.isinf(lsef[gone]).all())
+    dMf = torch.randn(len(lens_full), L, device="cuda", generator=gen)
+    dM = dMf[keep].contiguous()
+    ds, attn = F.segment_softmax_pool_bwd(X, s, off, dM, M, want_attn=True)
+    dsf, attnf = F.segment_softmax_pool_bwd(X, s, off_full, dMf, Mf, want_attn=True)
+    assert torch.equal(ds, dsf) and torch.equal(attn, attnf)
+    for need_dx in (False, True):
+        a = F.gated_scores_bwd(X, Wcat, bcat, ww, bw, ds, attn, dM, off, need_dx, gate_act=act)
+        b = F.gated_scores_bwd(X, Wcat, bcat, ww, bw, dsf, attnf, dMf, off_full, need_dx, gate_act=act)
+        assert (a[0] is None) == (b[0] is None) == (not need_dx)
+        for name, x, y in zip(("dX", "dWcat", "dbcat", "dww", "dbw"), a, b):
+            assert x is None or torch.equal(x, y), (name, need_dx)
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 # AbmilTrainer: forward_backward (row dots) against forward + backward (two passes)
 # ---------------------------------------------------------------------------------------------------------------------
@@ -180,18 +219,6 @@ def test_forward_backward_equals_forward_then_backward(dtype, L, save_gate, need
         assert torch.equal(dXa, dXb)
     else:
         assert dXa is None and dXb is None
-
-
-def test_fused_backward_opt_in_keeps_two_calls(monkeypatch):
-    monkeypatch.setenv("MILB200_FUSED_BWD", "1")
-    lens = [300, 17, 900]
-    offt = _csr(lens)
-    X = torch.randn(sum(lens), 1024, device="cuda").bfloat16()
-    tr = _trainer(torch.bfloat16, 1024)
-    names = _phases(tr)
-    tr.forward_backward(X, offt)
-    torch.cuda.synchronize()
-    assert "gated_pool_bwd" in names and "pool_bwd_rowdot" not in names
 
 
 def test_graphed_step_equals_eager_step():

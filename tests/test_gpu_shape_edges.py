@@ -158,7 +158,7 @@ def _gated_pool(F, dtype, L, D, lens, seed):
     s, act = F.gated_scores(X, Wcat, bcat, ww, bw, save=True)
     M, Ml, am, lse = F.segment_softmax_pool(X, s, offt, want_lowp=dtype != torch.float32)
     ds, attn = F.segment_softmax_pool_bwd(X, s, offt, dM, M, want_attn=True)
-    got = {"s": s, "M": M, "M_lowp": Ml, "argmax": am, "lse": lse, "ds": ds, "attn": attn}
+    got = {"s": s, "M": M, "M_lowp": Ml, "argmax": am, "lse": lse, "ds": ds, "attn": attn, "act": act}
     runs = {"saved+dX": (act, True), "saved": (act, False), "recompute+dX": (None, True), "recompute": (None, False)}
     seen = set()
     for name, (ga, need_dx) in runs.items():
@@ -167,10 +167,6 @@ def _gated_pool(F, dtype, L, D, lens, seed):
         seen.add((ga is None, need_dx))
         dX, dWcat, dbcat, dww, dbw = F.gated_scores_bwd(X, Wcat, bcat, ww, bw, ds, attn, dM, offt, need_dx, gate_act=ga)
         got[name] = [t.clone() if t is not None else None for t in (dX, dWcat, dbcat, dww, dbw)]
-    if act is not None and F.L.lib().milb200_gated_pool_bwd_supported(L, D, F.L.dtype_code(X)):
-        ds_f, dWcat, dbcat, dww, dbw = F.gated_pool_bwd(X, s, offt, dM, M, ww, act)
-        got["fused"] = [None, dWcat, dbcat, dww, dbw]
-        got["fused_ds"] = ds_f
     torch.cuda.synchronize()
 
     q = (lambda t: t.to(dtype).to(F64))
@@ -202,7 +198,7 @@ def _check_gated_pool(got, ref, offt, bag, dtype, lens):
     _check_argmax(got["argmax"], got["s"], ref["s"], offt, bag)
     dscale = float(ref["ds"].abs().max()) if not singles else 1.0
     n = int(sum(lens))
-    for run in ("saved+dX", "saved", "recompute+dX", "recompute", "fused"):
+    for run in ("saved+dX", "saved", "recompute+dX", "recompute"):
         if run not in got:
             continue
         dX, dWcat, dbcat, dww, dbw = got[run]
@@ -214,17 +210,23 @@ def _check_gated_pool(got, ref, offt, bag, dtype, lens):
             else:
                 _close(f"{run} {k}", t, ref[k], tol)
         assert abs(float(dbw) - float(ref["dbw"])) <= 2e-5 * math.sqrt(n) * dscale + 1e-6, (run, "dbw", float(dbw))
-    for k in ("ds", "fused_ds"):
-        if k in got:
-            _close_ds(k, got[k], ref["ds"], ref["ds_scale"], tol)
+    _close_ds("ds", got["ds"], ref["ds"], ref["ds_scale"], tol)
 
 
 # bf16, D = 192, L % 16 == 0: the tensor-core path.  L = 64 is one K block, 80 / 144 / 208 / 1008 end in a partial K block,
 # 1040 gives the TN GEMM a third 512-column tile with 16 valid columns, 1536 / 2048 run the pool's NV = 6 / 8.  Row counts: 1, one short m-tile,
 # +-1 around the 128-row tile and the 256-row CTA pair, an odd tile count (385 = 3 tiles + 1 row), and a batch past a
 # full wave of 74 CTA pairs (2 x 18944 + 129 rows).
+# The saved-activation dW kernel (k_gemm_tn_gate) splits the 32-row k-blocks over 49 / 24 / 6 splits (L <= 512 / <= 1024
+# / 4096 on 148 SMs) and stages ds eight k-blocks at a time in a 32-block ring: splits of exactly 8 and 9 k-blocks
+# (512 x 49*8*32, 512 x 49*9*32), a ring that wraps once or twice (1024 x 24*33*32, 768 x 24*64*32 + 5), a last split
+# shorter than one ds chunk (1024 x 24*8*32 + 1) and fewer than 8 rows (256 x 7).  L = 96 / 112 end the accumulator
+# epilogue in a full / half 32-column chunk, 528 puts 16 columns in a second 512-column tile at L <= 1024, and 4096 runs
+# eight 512-column tiles with the pool's NV = 16.
 TC_CASES = [(64, 1), (80, 31), (144, 127), (208, 128), (1008, 129), (1040, 256), (1536, 257), (2048, 385),
-            (80, 2 * 18944 + 129), (1040, 2 * 18944 + 129)]
+            (80, 2 * 18944 + 129), (1040, 2 * 18944 + 129),
+            (512, 49 * 8 * 32), (512, 49 * 9 * 32), (1024, 24 * 33 * 32), (768, 24 * 64 * 32 + 5), (1024, 24 * 8 * 32 + 1),
+            (256, 7), (96, 2), (112, 33), (528, 300), (4096, 40)]
 
 
 @pytest.mark.parametrize("L,n", TC_CASES)
@@ -232,8 +234,7 @@ def test_gated_pool_tensor_core_path_any_L(F, L, n):
     lens = _lens(n)
     got, ref, offt, bag = _gated_pool(F, torch.bfloat16, L, 192, lens, seed=L + n)
     assert got["saved"][1] is not None
-    if L <= 1024:
-        assert "fused" in got, "the fused backward must cover bf16, D = 192, L <= 1024"
+    assert got["act"] is not None, "the tensor-core forward must save the gate activations"
     _check_gated_pool(got, ref, offt, bag, torch.bfloat16, lens)
 
 
@@ -249,7 +250,8 @@ FFMA_CASES = [(torch.float32, 64, 56), (torch.float32, 100, 96), (torch.float32,
 def test_gated_pool_ffma_path_any_D(F, dtype, D, L):
     lens = _lens(700)
     got, ref, offt, bag = _gated_pool(F, dtype, L, D, lens, seed=D * 7 + L)
-    assert "fused" not in got
+    if dtype == torch.bfloat16:
+        assert got["act"] is None, "bf16 gate activations are saved by the tensor-core forward only"
     _check_gated_pool(got, ref, offt, bag, dtype, lens)
 
 
