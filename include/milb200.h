@@ -131,6 +131,26 @@ int milb200_segment_softmax_pool_bwd_rowdot(const float* scores, const int32_t* 
                                             const float* dM, const float* M, const float* rowdot, float* dscores,
                                             float* attn, void* workspace, size_t ws_bytes, void* stream);
 
+/* The same pair for a linear head on the pooled vector, z_b = W (s_b * M_b) + c with W [C,L] fp32 and s_b an optional
+ * per-bag column scale (the head's dropout mask times 1/(1-p); NULL = all ones): dM_b = s_b * (W^T dz_b) is not known
+ * before the forward, but its row dots are a combination of C dots that are,
+ *   hdot[i*C + c] = (W_c * s_b) . x_i     (fp32 [total_n, C]),
+ * and the backward forms dM_b . x_i = sum_c dz[b,c] hdot[i*C + c] from them without reading X.  col_scale is [B,L] fp32.
+ * M, M_lowp, argmax and lse equal those of milb200_segment_softmax_pool_fwd bit for bit.  The backward takes dz [B,C] and
+ * dM = s_b * (W^T dz_b) [B,L] (for dM_b . M_b); with C = 1, W = dM_b (one bag) and dz = 1 it is the _rowdot backward.
+ * W, col_scale, hdot, dz, dscores and attn must be 4-byte aligned; attn may be NULL.  1 <= C <= 8 (C = 0 is EINVAL, larger
+ * C EUNSUPPORTED); C > 4 needs a bf16 row of at most 1536 elements (EUNSUPPORTED).  The forward stages the C vectors in
+ * shared memory, (8 + C') * L * 4 bytes with C' = C rounded up to 1, 2, 4 or 8, which must stay within 226 KB
+ * (EUNSUPPORTED otherwise, e.g. bf16 L = 4096 with C > 4).  Both are refused before any launch.
+ * Workspace of both: milb200_pool_workspace_bytes.                                                      */
+int milb200_segment_softmax_pool_fwd_headdot(const void* X, const float* scores, const int32_t* offsets, int B,
+                                             int64_t total_n, int L, int dtype, const float* W, int C,
+                                             const float* col_scale, float* M, void* M_lowp, int32_t* argmax, float* lse,
+                                             float* hdot, void* workspace, size_t ws_bytes, void* stream);
+int milb200_segment_softmax_pool_bwd_headdot(const float* scores, const int32_t* offsets, int B, int64_t total_n, int L,
+                                             int C, const float* dz, const float* dM, const float* M, const float* hdot,
+                                             float* dscores, float* attn, void* workspace, size_t ws_bytes, void* stream);
+
 /* ---- dense linear layers ------------------------------------------------------------------------
  * Y[m,n] = act(X[m,k] W[n,k]^T + bias[n])  — nn.Linear (+Tanh/ReLU) as used by fc_pathology,
  * fc_CI2CT/fc_CI2Pth (model/aggregator.py:44,47,66), q/k/v/out projections

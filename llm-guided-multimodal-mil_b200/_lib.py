@@ -44,6 +44,9 @@ SIGNATURES = {
     "milb200_segment_softmax_pool_bwd": (_i, [_p, _p, _p, _i, _i64, _i, _i, _p, _p, _p, _p, _p, _sz, _p]),
     "milb200_segment_softmax_pool_fwd_rowdot": (_i, [_p, _p, _p, _i, _i64, _i, _i, _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
     "milb200_segment_softmax_pool_bwd_rowdot": (_i, [_p, _p, _i, _i64, _i, _p, _p, _p, _p, _p, _p, _sz, _p]),
+    "milb200_segment_softmax_pool_fwd_headdot": (_i, [_p, _p, _p, _i, _i64, _i, _i, _p, _i, _p, _p, _p, _p, _p, _p, _p, _sz,
+                                                     _p]),
+    "milb200_segment_softmax_pool_bwd_headdot": (_i, [_p, _p, _i, _i64, _i, _i, _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
     "milb200_segment_sum_fwd": (_i, [_p, _p, _i, _i64, _i, _i, _p, _p, _p, _sz, _p]),
     "milb200_bag_broadcast": (_i, [_p, _p, _p, _i, _i64, _i, _i, _p, _p]),
     "milb200_dropout": (_i, [_p, _p, _i64, _f, C.c_uint64, C.c_uint64, _i, _p]),

@@ -9,6 +9,7 @@
 // in piece order, so the result is deterministic.
 #include <algorithm>
 #include <cfloat>
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -18,12 +19,15 @@ constexpr int POOL_THREADS = 256;
 constexpr int POOL_WARPS = POOL_THREADS / 32;
 constexpr int POOL_BLK = 16;         // rows a warp owns at a time (one score per lane 0..15)
 constexpr int POOL_MIN_SLAB = 256;   // rows per CTA at least (512 KB of bf16 x 1024)
+constexpr int POOL_MAX_DOTS = 8;     // row dots per row of the row-dot forward (widest NC bucket)
+constexpr size_t POOL_SMEM_LIMIT = 227 * 1024;  // dynamic + static shared memory of one CTA (sm_100)
 
 template <typename T> __device__ __forceinline__ float exp_t(float x);
 template <> __device__ __forceinline__ float exp_t<float>(float x) { return expf(x); }
 template <> __device__ __forceinline__ float exp_t<__nv_bfloat16>(float x) { return __expf(x); }
 
-// the VN floats of dM_b that line up with 16-byte vector `vec` of a row, from shared memory; 0 past the row (vec >= V)
+// the VN floats of a staged dot vector that line up with 16-byte vector `vec` of a row, from shared memory; 0 past the
+// row (vec >= V)
 template <int VN>
 __device__ __forceinline__ void dm_chunk(const float* dms, int vec, int V, float* d) {
 #pragma unroll
@@ -45,20 +49,27 @@ struct PiecePartial {  // published per (CTA, bag) piece
 // (3) one shared-memory fold across the 8 warps.  A bag inside one slab is finished on the spot; a bag spanning
 // slabs is finished by the CTA that publishes its last piece, folding the partials in piece order (deterministic).
 //
-// ROWDOT: the caller already knows the upstream gradient dM, so the pass also writes rowdot[i] = dM_b . x_i for every
-// row, on the rows it has in registers anyway; the backward then forms the score gradients without reading X again.
-// dM_b is staged once per piece in shared memory next to `red`, and each row's dot is accumulated exactly as k_pool_bwd
-// accumulates it (j then k ascending, masked lanes included in the two-row loop, the same warp_sum), so the gradients do
-// not change by a bit.
-template <typename T, int NV, bool ROWDOT>
+// NC > 0 (row dots): the caller already knows what the upstream gradient is made of, so the pass also writes C dots per
+// row, dots[i * C + c] = v_bc . x_i, on the rows it has in registers anyway; the backward then forms the score gradients
+// without reading X again.  v_bc[l] = dv[b * dv_bag_stride + c * L + l] * (col_scale ? col_scale[b * L + l] : 1):
+//   - the _rowdot form is C = 1 with dv = dM (stride L, no scale): dots[i] = dM_b . x_i;
+//   - the _headdot form takes dv = a linear head's W [C, L] (stride 0) and col_scale = the head's dropout scale s_b, so
+//     that dM_b . x_i = sum_c dz_bc dots[i * C + c] once the head's dz exists.
+// NC is C rounded up to a bucket {1, 2, 4, 8}; vectors C..NC-1 are staged as zeros and their dots are not written.  The
+// vectors are staged once per piece in shared memory next to `red`; one shared-memory read of a chunk serves both rows of
+// the two-row loop.  Each dot is accumulated exactly as k_pool_bwd accumulates dM_b . x_i (j then k ascending, masked
+// lanes included in the two-row loop, the same warp_sum), so the C = 1 gradients do not change by a bit.
+template <typename T, int NV, int NC>
 __device__ __forceinline__ void
 pool_fwd_body(const T* __restrict__ X, const float* __restrict__ scores, const int32_t* __restrict__ offsets, int B,
               int64_t total_n, int L, int V, int64_t slab, float* __restrict__ M, T* __restrict__ M_lowp,
               int32_t* __restrict__ argmax_out, float* __restrict__ lse_out, float* __restrict__ ws_acc,
               PiecePartial* __restrict__ ws_ml, unsigned int* __restrict__ counters, int normalize,
-              const float* __restrict__ dM, float* __restrict__ rowdot) {
+              const float* __restrict__ dv, int64_t dv_bag_stride, const float* __restrict__ col_scale, int C,
+              float* __restrict__ dots) {
   constexpr int VN = Vec16<T>::N;
-  extern __shared__ __align__(16) float red[];  // [POOL_WARPS][L], then (ROWDOT) dM_b [L]
+  constexpr int ND = NC > 0 ? NC : 1;           // (array extent; no dot is formed when NC == 0)
+  extern __shared__ __align__(16) float red[];  // [POOL_WARPS][L], then (NC > 0) the dot vectors [NC][L]
   float* dms = red + static_cast<int64_t>(POOL_WARPS) * L;
   __shared__ float wred_v[POOL_WARPS];
   __shared__ int wred_i[POOL_WARPS];
@@ -95,8 +106,20 @@ pool_fwd_body(const T* __restrict__ X, const float* __restrict__ scores, const i
       }
       continue;
     }
-    if (ROWDOT)  // read after the barrier of (1); the previous piece ended with one
-      for (int c = t; c < L; c += POOL_THREADS) dms[c] = __ldg(dM + static_cast<int64_t>(b) * L + c);
+    // read after the barrier of (1); the previous piece ended with one
+#pragma unroll
+    for (int c = 0; c < NC; ++c) {
+      float* dst = dms + static_cast<int64_t>(c) * L;
+      const float* src = dv + static_cast<int64_t>(b) * dv_bag_stride + static_cast<int64_t>(c) * L;
+      if (c >= C) {
+        for (int l = t; l < L; l += POOL_THREADS) dst[l] = 0.f;
+      } else if (col_scale) {
+        const float* cs = col_scale + static_cast<int64_t>(b) * L;
+        for (int l = t; l < L; l += POOL_THREADS) dst[l] = __ldg(src + l) * __ldg(cs + l);
+      } else {
+        for (int l = t; l < L; l += POOL_THREADS) dst[l] = __ldg(src + l);  // (independent loads: the loop unrolls)
+      }
+    }
 
     // ---- (1) piece max and first argmax ----
     float pm = 0.f;
@@ -154,51 +177,96 @@ pool_fwd_body(const T* __restrict__ X, const float* __restrict__ scores, const i
           v1[j] = (vec < V) ? ldg_stream(Xv + (rb + i + 1) * V + vec) : make_uint4(0, 0, 0, 0);
         }
         const float w0 = __shfl_sync(0xffffffffu, e, i), w1 = __shfl_sync(0xffffffffu, e, i + 1);
-        float g0 = 0.f, g1 = 0.f;
+        float g0[ND], g1[ND];
+#pragma unroll
+        for (int c = 0; c < ND; ++c) g0[c] = g1[c] = 0.f;
 #pragma unroll
         for (int j = 0; j < NV; ++j) {
-          float f[VN], d[VN];
-          if (ROWDOT) dm_chunk<VN>(dms, lane + j * 32, V, d);  // one read of dM_b serves both rows
-          Vec16<T>::unpack(v0[j], f);
+          if constexpr (NC <= 1) {
+            // no dots, or one: the staged chunk is held across both rows, each row unpacked once into the same registers
+            float f[VN], d[VN];
+            if (NC == 1) dm_chunk<VN>(dms, lane + j * 32, V, d);  // one read serves both rows
+            Vec16<T>::unpack(v0[j], f);
 #pragma unroll
-          for (int k = 0; k < VN; ++k) acc[j][k] = fmaf(w0, f[k], acc[j][k]);
-          if (ROWDOT)
+            for (int k = 0; k < VN; ++k) acc[j][k] = fmaf(w0, f[k], acc[j][k]);
+            if (NC == 1)
 #pragma unroll
-            for (int k = 0; k < VN; ++k) g0 = fmaf(d[k], f[k], g0);
-          Vec16<T>::unpack(v1[j], f);
+              for (int k = 0; k < VN; ++k) g0[0] = fmaf(d[k], f[k], g0[0]);
+            Vec16<T>::unpack(v1[j], f);
 #pragma unroll
-          for (int k = 0; k < VN; ++k) acc[j][k] = fmaf(w1, f[k], acc[j][k]);
-          if (ROWDOT)
+            for (int k = 0; k < VN; ++k) acc[j][k] = fmaf(w1, f[k], acc[j][k]);
+            if (NC == 1)
 #pragma unroll
-            for (int k = 0; k < VN; ++k) g1 = fmaf(d[k], f[k], g1);
+              for (int k = 0; k < VN; ++k) g1[0] = fmaf(d[k], f[k], g1[0]);
+          } else {
+            // several: both rows unpacked once, the staged vectors streamed past them one chunk at a time (holding NC
+            // chunks instead would cost NC * VN registers)
+            float f0[VN], f1[VN];
+            Vec16<T>::unpack(v0[j], f0);
+#pragma unroll
+            for (int k = 0; k < VN; ++k) acc[j][k] = fmaf(w0, f0[k], acc[j][k]);
+            Vec16<T>::unpack(v1[j], f1);
+#pragma unroll
+            for (int k = 0; k < VN; ++k) acc[j][k] = fmaf(w1, f1[k], acc[j][k]);
+#pragma unroll
+            for (int c = 0; c < NC; ++c) {
+              float d[VN];
+              dm_chunk<VN>(dms + static_cast<int64_t>(c) * L, lane + j * 32, V, d);  // one read serves both rows
+#pragma unroll
+              for (int k = 0; k < VN; ++k) g0[c] = fmaf(d[k], f0[k], g0[c]);
+#pragma unroll
+              for (int k = 0; k < VN; ++k) g1[c] = fmaf(d[k], f1[k], g1[c]);
+            }
+          }
         }
-        if (ROWDOT) {
-          g0 = warp_sum(g0);
-          g1 = warp_sum(g1);
-          if (lane == 0) { rowdot[rb + i] = g0; rowdot[rb + i + 1] = g1; }
+        if constexpr (NC == 1) {  // (C == 1)
+          g0[0] = warp_sum(g0[0]);
+          g1[0] = warp_sum(g1[0]);
+          if (lane == 0) { dots[rb + i] = g0[0]; dots[rb + i + 1] = g1[0]; }
+        } else if constexpr (NC > 1) {
+          float o0 = 0.f, o1 = 0.f;  // lane c writes dot c of both rows
+#pragma unroll
+          for (int c = 0; c < NC; ++c) {
+            g0[c] = warp_sum(g0[c]);
+            g1[c] = warp_sum(g1[c]);
+            if (lane == c) { o0 = g0[c]; o1 = g1[c]; }
+          }
+          if (lane < C) { dots[(rb + i) * C + lane] = o0; dots[(rb + i + 1) * C + lane] = o1; }
         }
       }
       if (i < nr) {
         const float w0 = __shfl_sync(0xffffffffu, e, i);
-        float g0 = 0.f;
+        float g0[ND];
+#pragma unroll
+        for (int c = 0; c < ND; ++c) g0[c] = 0.f;
 #pragma unroll
         for (int j = 0; j < NV; ++j) {
           const int vec = lane + j * 32;
           if (vec < V) {
-            float f[VN], d[VN];
+            float f[VN];
             Vec16<T>::unpack(ldg_stream(Xv + (rb + i) * V + vec), f);
 #pragma unroll
             for (int k = 0; k < VN; ++k) acc[j][k] = fmaf(w0, f[k], acc[j][k]);
-            if (ROWDOT) {
-              dm_chunk<VN>(dms, vec, V, d);
 #pragma unroll
-              for (int k = 0; k < VN; ++k) g0 = fmaf(d[k], f[k], g0);
+            for (int c = 0; c < NC; ++c) {
+              float d[VN];
+              dm_chunk<VN>(dms + static_cast<int64_t>(c) * L, vec, V, d);
+#pragma unroll
+              for (int k = 0; k < VN; ++k) g0[c] = fmaf(d[k], f[k], g0[c]);
             }
           }
         }
-        if (ROWDOT) {
-          g0 = warp_sum(g0);
-          if (lane == 0) rowdot[rb + i] = g0;
+        if constexpr (NC == 1) {
+          g0[0] = warp_sum(g0[0]);
+          if (lane == 0) dots[rb + i] = g0[0];
+        } else if constexpr (NC > 1) {
+          float o0 = 0.f;
+#pragma unroll
+          for (int c = 0; c < NC; ++c) {
+            g0[c] = warp_sum(g0[c]);
+            if (lane == c) o0 = g0[c];
+          }
+          if (lane < C) dots[(rb + i) * C + lane] = o0;
         }
       }
     }
@@ -308,35 +376,45 @@ pool_fwd_body(const T* __restrict__ X, const float* __restrict__ scores, const i
 
 template <typename T, int NV>
 __global__ void __launch_bounds__(POOL_THREADS) k_pool_fwd(MIL_POOL_FWD_PARAMS) {
-  pool_fwd_body<T, NV, false>(MIL_POOL_FWD_ARGS, nullptr, nullptr);
+  pool_fwd_body<T, NV, 0>(MIL_POOL_FWD_ARGS, nullptr, 0, nullptr, 0, nullptr);
 }
 
-// The row dots cost registers (the dM_b chunk, two dots).  Where the plain kernel runs two CTAs per SM (<= 128
-// registers: bf16 NV <= 6, fp32 NV <= 8) the row-dot kernel is held to two as well, so that the HBM-bound pass keeps its
-// bytes in flight; the wider instantiations run one CTA per SM either way.
-template <typename T, int NV>
-constexpr int pool_fwd_rowdot_min_blocks() { return (sizeof(T) == 2 ? NV <= 6 : NV <= 8) ? 2 : 1; }
+// The row dots cost registers (the staged chunk, two dots per vector).  Where the plain kernel runs two CTAs per SM
+// (<= 128 registers: bf16 NV <= 6, fp32 NV <= 8) the one-dot kernel is held to two as well, so that the HBM-bound pass
+// keeps its bytes in flight; the wider instantiations run one CTA per SM either way.  More dots per row keep two CTAs
+// only where they fit in 128 registers without spilling (ptxas -v, CUDA 12.9); elsewhere they run one CTA per SM.
+template <typename T, int NV, int NC>
+constexpr int pool_fwd_rowdot_min_blocks() {
+  constexpr bool two = sizeof(T) == 2 ? NV <= 6 : NV <= 8;
+  constexpr bool fits = NC == 1 || (NC <= 4 && NV <= (sizeof(T) == 2 ? 4 : 6)) || (NC == 8 && NV <= (sizeof(T) == 2 ? 1 : 4));
+  return two && fits ? 2 : 1;
+}
 
-template <typename T, int NV>
-__global__ void __launch_bounds__(POOL_THREADS, pool_fwd_rowdot_min_blocks<T, NV>())
-k_pool_fwd_rowdot(MIL_POOL_FWD_PARAMS, const float* __restrict__ dM, float* __restrict__ rowdot) {
-  pool_fwd_body<T, NV, true>(MIL_POOL_FWD_ARGS, dM, rowdot);
+template <typename T, int NV, int NC>
+__global__ void __launch_bounds__(POOL_THREADS, pool_fwd_rowdot_min_blocks<T, NV, NC>())
+k_pool_fwd_rowdot(MIL_POOL_FWD_PARAMS, const float* __restrict__ dv, int64_t dv_bag_stride,
+                  const float* __restrict__ col_scale, int C, float* __restrict__ dots) {
+  pool_fwd_body<T, NV, NC>(MIL_POOL_FWD_ARGS, dv, dv_bag_stride, col_scale, C, dots);
 }
 #undef MIL_POOL_FWD_PARAMS
 #undef MIL_POOL_FWD_ARGS
 
 // ---- backward ------------------------------------------------------------------------------------
 // stats[b] = (lse_b, dM_b . M_b): softmax statistics are recomputed from the scores, not stored.
-// SWEEP (rowdot[i] = dM_b . x_i, written by the ROWDOT forward): the same CTA then sweeps its bag and writes the score
-// gradients and attention weights: k_pool_bwd's expressions on the same floats, without reading X.  A template flag, so
-// that the statistics-only kernel keeps its registers (two 1024-thread CTAs per SM).
+// SWEEP (row dots written by the row-dot forward): the same CTA then sweeps its bag and writes the score gradients and
+// attention weights without reading X, from g_i = dM_b . x_i:
+//   - dz == NULL (_rowdot): g_i = rowdot[i], and the expressions are k_pool_bwd's on the same floats;
+//   - dz [B, C] (_headdot): g_i = sum_c dz[b, c] * rowdot[i * C + c], c ascending.
+// A template flag, so that the statistics-only kernel keeps its registers (two 1024-thread CTAs per SM).
 template <bool SWEEP>
 __global__ void __launch_bounds__(1024)
 k_pool_bwd_stats(const float* __restrict__ scores, const int32_t* __restrict__ offsets, int L,
                  const float* __restrict__ dM, const float* __restrict__ M, float2* __restrict__ stats,
-                 const float* __restrict__ rowdot, float* __restrict__ dscores, float* __restrict__ attn) {
+                 const float* __restrict__ rowdot, float* __restrict__ dscores, float* __restrict__ attn,
+                 const float* __restrict__ dz = nullptr, int C = 1) {
   __shared__ float red[32];
   __shared__ float bc;
+  __shared__ float dzs[POOL_MAX_DOTS];
   __shared__ float2 bag_stats;
   const int b = blockIdx.x, t = threadIdx.x, lane = t & 31, warp = t >> 5, nt = blockDim.x, nw = blockDim.x >> 5;
   const int64_t ob = offsets[b], oe = offsets[b + 1];
@@ -387,21 +465,28 @@ k_pool_bwd_stats(const float* __restrict__ scores, const int32_t* __restrict__ o
     stats[b] = bag_stats;
   }
   if (!SWEEP) return;
+  if (dz && t < C) dzs[t] = dz[static_cast<int64_t>(b) * C + t];
   __syncthreads();
   const float lse = bag_stats.x, cdot = bag_stats.y;
+  auto row_dot = [&](int64_t i) {
+    if (!dz) return rowdot[i];
+    float g = 0.f;
+    for (int c = 0; c < C; ++c) g = fmaf(dzs[c], rowdot[i * C + c], g);
+    return g;
+  };
 #pragma unroll
   for (int k = 0; k < KEEP; ++k) {
     const int64_t i = ob + t + static_cast<int64_t>(k) * nt;
     if (i < oe) {
       const float a = expf(sc[k] - lse);
-      dscores[i] = a * (rowdot[i] - cdot);
+      dscores[i] = a * (row_dot(i) - cdot);
       if (attn) attn[i] = a;
     }
   }
 #pragma unroll 4
   for (int64_t i = ob + t + static_cast<int64_t>(KEEP) * nt; i < oe; i += nt) {
     const float a = expf(scores[i] - lse);
-    dscores[i] = a * (rowdot[i] - cdot);
+    dscores[i] = a * (row_dot(i) - cdot);
     if (attn) attn[i] = a;
   }
 }
@@ -564,23 +649,40 @@ static PoolWs pool_ws(void* base, int64_t total_n, int B, int L) {
   return w;
 }
 
-// dM != NULL selects the ROWDOT kernels (rowdot[i] = dM_b . x_i as well)
+// NC bucket of C row dots per row (0: no dots)
+static int pool_dot_bucket(int C) { return C <= 0 ? 0 : C == 1 ? 1 : C == 2 ? 2 : C <= 4 ? 4 : 8; }
+
+// per-warp accumulator rows, plus the staged dot vectors of the row-dot kernels
+static size_t pool_fwd_smem_bytes(int L, int C) {
+  return sizeof(float) * static_cast<size_t>(POOL_WARPS + pool_dot_bucket(C)) * L;
+}
+
+// dv != NULL selects the row-dot kernels: C dots per row, dots[i * C + c] = v_bc . x_i (see pool_fwd_body)
 template <typename T>
 static int pool_fwd_t(const T* X, const float* scores, const int32_t* offsets, int B, int64_t total_n, int L, float* M,
                       T* M_lowp, int32_t* argmax, float* lse, void* workspace, size_t ws_bytes, cudaStream_t st,
-                      int normalize = 1, const float* dM = nullptr, float* rowdot = nullptr) {
+                      int normalize = 1, const float* dv = nullptr, int64_t dv_bag_stride = 0,
+                      const float* col_scale = nullptr, int C = 0, float* dots = nullptr) {
   const int V = L * static_cast<int>(sizeof(T)) / 16;
   const int nv = (V + 31) / 32;
   MIL_CHECK_ARG(nv <= 16, MILB200_EUNSUPPORTED, "pool: row of %d bytes exceeds the 8 KB limit", L * (int)sizeof(T));
+  if (!dv) C = 0;
+  MIL_CHECK_ARG(C <= POOL_MAX_DOTS, MILB200_EUNSUPPORTED, "pool_fwd: %d row dots per row exceed the limit of %d", C,
+                POOL_MAX_DOTS);
+  // eight dots per row on a bf16 row of more than 6 vectors per lane do not fit in 255 registers without spilling
+  MIL_CHECK_ARG(!(sizeof(T) == 2 && nv > 6 && C > 4), MILB200_EUNSUPPORTED,
+                "pool_fwd: more than 4 row dots per row need a bf16 row of at most 1536 elements (L=%d)", L);
+  const size_t smem = pool_fwd_smem_bytes(L, C);
+  // the kernel's static shared memory (< 1 KB) counts against the same limits as the dynamic part
+  MIL_CHECK_ARG(smem + 1024 <= POOL_SMEM_LIMIT, MILB200_EUNSUPPORTED,
+                "pool_fwd: L=%d with %d row dots per row needs %zu bytes of shared memory (limit %zu)", L, C, smem + 1024,
+                POOL_SMEM_LIMIT);
   PoolWs w = pool_ws(workspace, total_n, B, L);
   MIL_CHECK_ARG(workspace && ws_bytes >= w.bytes, MILB200_EWORKSPACE, "pool_fwd: workspace %zu < %zu", ws_bytes, w.bytes);
   MIL_CUDA(cudaMemsetAsync(w.counters, 0, sizeof(unsigned int) * static_cast<size_t>(B), st));
   const int64_t slab = pool_slab_rows(total_n);
   const int64_t ctas = (total_n + slab - 1) / slab;
-  // per-warp accumulator rows, plus the staged dM_b row of the ROWDOT kernels
-  const size_t smem = sizeof(float) * static_cast<size_t>(POOL_WARPS + (dM ? 1 : 0)) * L;
   auto launch = [&](auto kern, auto... rowdot_args) -> int {
-    // the kernel's static shared memory (< 1 KB) counts against the same 48 KB default as the dynamic part
     if (smem + 1024 > 48 * 1024) MIL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kern<<<static_cast<unsigned>(ctas), POOL_THREADS, smem, st>>>(X, scores, offsets, B, total_n, L, V, slab, M, M_lowp,
                                                                  argmax, lse, w.acc, w.ml, w.counters, normalize,
@@ -589,14 +691,30 @@ static int pool_fwd_t(const T* X, const float* scores, const int32_t* offsets, i
     return MILB200_OK;
   };
   // (the same NV buckets as pool_bwd_t: a row's dot then has the same lane mapping in both kernels)
-  if (dM) {
-    if (nv <= 1) return launch(k_pool_fwd_rowdot<T, 1>, dM, rowdot);
-    if (nv == 2) return launch(k_pool_fwd_rowdot<T, 2>, dM, rowdot);
-    if (nv == 3) return launch(k_pool_fwd_rowdot<T, 3>, dM, rowdot);
-    if (nv == 4) return launch(k_pool_fwd_rowdot<T, 4>, dM, rowdot);
-    if (nv <= 6) return launch(k_pool_fwd_rowdot<T, 6>, dM, rowdot);
-    if (nv <= 8) return launch(k_pool_fwd_rowdot<T, 8>, dM, rowdot);
-    return launch(k_pool_fwd_rowdot<T, 16>, dM, rowdot);
+  auto launch_dots = [&](auto nc) -> int {
+    constexpr int NC = decltype(nc)::value;
+    if constexpr (sizeof(T) == 2 && NC > 4) {  // (refused above past NV = 6)
+      if (nv <= 1) return launch(k_pool_fwd_rowdot<T, 1, NC>, dv, dv_bag_stride, col_scale, C, dots);
+      if (nv == 2) return launch(k_pool_fwd_rowdot<T, 2, NC>, dv, dv_bag_stride, col_scale, C, dots);
+      if (nv == 3) return launch(k_pool_fwd_rowdot<T, 3, NC>, dv, dv_bag_stride, col_scale, C, dots);
+      if (nv == 4) return launch(k_pool_fwd_rowdot<T, 4, NC>, dv, dv_bag_stride, col_scale, C, dots);
+      return launch(k_pool_fwd_rowdot<T, 6, NC>, dv, dv_bag_stride, col_scale, C, dots);
+    } else {
+      if (nv <= 1) return launch(k_pool_fwd_rowdot<T, 1, NC>, dv, dv_bag_stride, col_scale, C, dots);
+      if (nv == 2) return launch(k_pool_fwd_rowdot<T, 2, NC>, dv, dv_bag_stride, col_scale, C, dots);
+      if (nv == 3) return launch(k_pool_fwd_rowdot<T, 3, NC>, dv, dv_bag_stride, col_scale, C, dots);
+      if (nv == 4) return launch(k_pool_fwd_rowdot<T, 4, NC>, dv, dv_bag_stride, col_scale, C, dots);
+      if (nv <= 6) return launch(k_pool_fwd_rowdot<T, 6, NC>, dv, dv_bag_stride, col_scale, C, dots);
+      if (nv <= 8) return launch(k_pool_fwd_rowdot<T, 8, NC>, dv, dv_bag_stride, col_scale, C, dots);
+      return launch(k_pool_fwd_rowdot<T, 16, NC>, dv, dv_bag_stride, col_scale, C, dots);
+    }
+  };
+  switch (pool_dot_bucket(C)) {
+    case 1: return launch_dots(std::integral_constant<int, 1>());
+    case 2: return launch_dots(std::integral_constant<int, 2>());
+    case 4: return launch_dots(std::integral_constant<int, 4>());
+    case 8: return launch_dots(std::integral_constant<int, 8>());
+    default: break;
   }
   if (nv <= 1) return launch(k_pool_fwd<T, 1>);
   if (nv == 2) return launch(k_pool_fwd<T, 2>);
@@ -688,9 +806,27 @@ int milb200_segment_softmax_pool_fwd_rowdot(const void* X, const float* scores, 
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (dtype == MILB200_BF16)
     return pool_fwd_t<__nv_bfloat16>((const __nv_bfloat16*)X, scores, offsets, B, total_n, L, M, (__nv_bfloat16*)M_lowp,
-                                     argmax, lse, workspace, ws_bytes, st, 1, dM, rowdot);
+                                     argmax, lse, workspace, ws_bytes, st, 1, dM, L, nullptr, 1, rowdot);
   return pool_fwd_t<float>((const float*)X, scores, offsets, B, total_n, L, M, (float*)M_lowp, argmax, lse, workspace,
-                           ws_bytes, st, 1, dM, rowdot);
+                           ws_bytes, st, 1, dM, L, nullptr, 1, rowdot);
+}
+
+int milb200_segment_softmax_pool_fwd_headdot(const void* X, const float* scores, const int32_t* offsets, int B,
+                                             int64_t total_n, int L, int dtype, const float* W, int C,
+                                             const float* col_scale, float* M, void* M_lowp, int32_t* argmax, float* lse,
+                                             float* hdot, void* workspace, size_t ws_bytes, void* stream) {
+  int rc = pool_check(X, scores, offsets, B, total_n, L, dtype);
+  if (rc) return rc;
+  MIL_CHECK_ARG(M && W && hdot, MILB200_EINVAL, "pool_fwd_headdot: M, W and hdot must be non-null");
+  MIL_CHECK_ARG(C >= 1, MILB200_EINVAL, "pool_fwd_headdot: C=%d must be positive", C);
+  MIL_CHECK_ARG(aligned_f32(W) && aligned_f32(hdot) && aligned_f32(col_scale), MILB200_EALIGN,
+                "pool_fwd_headdot: W, col_scale and hdot must be 4-byte aligned");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (dtype == MILB200_BF16)
+    return pool_fwd_t<__nv_bfloat16>((const __nv_bfloat16*)X, scores, offsets, B, total_n, L, M, (__nv_bfloat16*)M_lowp,
+                                     argmax, lse, workspace, ws_bytes, st, 1, W, 0, col_scale, C, hdot);
+  return pool_fwd_t<float>((const float*)X, scores, offsets, B, total_n, L, M, (float*)M_lowp, argmax, lse, workspace,
+                           ws_bytes, st, 1, W, 0, col_scale, C, hdot);
 }
 
 /* M[b] = sum_i x_i over CSR offsets (no softmax): the reference's dense-batch behaviour (ABMIL.py:56-59 with
@@ -751,6 +887,27 @@ int milb200_segment_softmax_pool_bwd_rowdot(const float* scores, const int32_t* 
                 w.bytes);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   k_pool_bwd_stats<true><<<B, 1024, 0, st>>>(scores, offsets, L, dM, M, w.stats, rowdot, dscores, attn);
+  MIL_LAUNCH_CHECK();
+  return MILB200_OK;
+}
+
+int milb200_segment_softmax_pool_bwd_headdot(const float* scores, const int32_t* offsets, int B, int64_t total_n, int L,
+                                             int C, const float* dz, const float* dM, const float* M, const float* hdot,
+                                             float* dscores, float* attn, void* workspace, size_t ws_bytes, void* stream) {
+  MIL_CHECK_ARG(scores && offsets && dz && dM && M && hdot && dscores, MILB200_EINVAL, "pool_bwd_headdot: null pointer");
+  MIL_CHECK_ARG(C >= 1, MILB200_EINVAL, "pool_bwd_headdot: C=%d must be positive", C);
+  MIL_CHECK_ARG(C <= POOL_MAX_DOTS, MILB200_EUNSUPPORTED, "pool_bwd_headdot: C=%d exceeds the limit of %d", C,
+                POOL_MAX_DOTS);
+  MIL_CHECK_ARG(aligned_f32(dz) && aligned_f32(hdot) && aligned_f32(dscores) && aligned_f32(attn), MILB200_EALIGN,
+                "pool_bwd_headdot: dz, hdot, dscores and attn must be 4-byte aligned");
+  MIL_CHECK_ARG(B > 0 && total_n > 0 && L > 0, MILB200_EINVAL, "pool_bwd_headdot: B=%d total_n=%lld L=%d must be positive",
+                B, (long long)total_n, L);
+  MIL_CHECK_ARG(total_n < (1ll << 31), MILB200_EINVAL, "pool_bwd_headdot: total_n exceeds int32 CSR offsets");
+  PoolWs w = pool_ws(workspace, total_n, B, L);
+  MIL_CHECK_ARG(workspace && ws_bytes >= w.bytes, MILB200_EWORKSPACE, "pool_bwd_headdot: workspace %zu < %zu", ws_bytes,
+                w.bytes);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  k_pool_bwd_stats<true><<<B, 1024, 0, st>>>(scores, offsets, L, dM, M, w.stats, hdot, dscores, attn, dz, C);
   MIL_LAUNCH_CHECK();
   return MILB200_OK;
 }

@@ -128,6 +128,52 @@ def segment_softmax_pool_bwd_rowdot(s, offsets, dM, M, rowdot, want_attn):
     return ds, attn
 
 
+def segment_softmax_pool_headdot(X, s, offsets, W, col_scale=None, want_lowp=False):
+    """segment_softmax_pool for a caller that feeds M (times an optional per-bag column scale, e.g. a dropout mask) to a
+    linear head W fp32 [C, L], C <= 8: the same pass over X also returns the head's row dots
+    hdot[i, c] = (W_c * col_scale_b) . x_i (fp32 [total_n, C]), which let segment_softmax_pool_bwd_headdot skip X once the
+    head's dz exists.  Returns (M, M_lowp|None, argmax, lse, hdot); the first four equal segment_softmax_pool's bit for bit."""
+    n, Lf = X.shape
+    B = offsets.numel() - 1
+    if W.dtype != torch.float32 or W.dim() != 2 or W.shape[1] != Lf:
+        raise L.MilB200Error(f"W must be fp32 [C, {Lf}], got {W.dtype} {list(W.shape)}")
+    if col_scale is not None:
+        _check_dM(col_scale, B, Lf)
+    C = W.shape[0]
+    M = torch.empty((B, Lf), dtype=torch.float32, device=X.device)
+    Ml = torch.empty((B, Lf), dtype=X.dtype, device=X.device) if want_lowp else None
+    am = torch.empty((B,), dtype=torch.int32, device=X.device)
+    lse = torch.empty((B,), dtype=torch.float32, device=X.device)
+    hdot = torch.empty((n, C), dtype=torch.float32, device=X.device)
+    ws = L.workspace(L.lib().milb200_pool_workspace_bytes(n, B, Lf), X.device)
+    L.check(L.lib().milb200_segment_softmax_pool_fwd_headdot(L.ptr(X), L.ptr(s), L.ptr(offsets), B, n, Lf,
+                                                             L.dtype_code(X), L.ptr(W), C, L.ptr(col_scale), L.ptr(M),
+                                                             L.ptr(Ml), L.ptr(am), L.ptr(lse), L.ptr(hdot), L.ptr(ws),
+                                                             ws.numel(), L.stream_ptr()),
+            "segment_softmax_pool_fwd_headdot")
+    return M, Ml, am, lse, hdot
+
+
+def segment_softmax_pool_bwd_headdot(s, offsets, dz, dM, M, hdot, want_attn):
+    """segment_softmax_pool_bwd from the head's row dots of segment_softmax_pool_headdot: dz fp32 [B, C] is the gradient
+    of the head's output, dM = col_scale * (W^T dz) fp32 [B, L] the gradient of M.  No pass over X.
+    Returns (ds, attn|None)."""
+    n = s.numel()
+    B, Lf = M.shape
+    _check_dM(dM, B, Lf)
+    C = hdot.shape[1]
+    if dz.dtype != torch.float32 or tuple(dz.shape) != (B, C) or tuple(hdot.shape) != (n, C):
+        raise L.MilB200Error(f"dz must be fp32 [{B}, {C}] and hdot [{n}, {C}]")
+    ds = torch.empty((n,), dtype=torch.float32, device=s.device)
+    attn = torch.empty((n,), dtype=torch.float32, device=s.device) if want_attn else None
+    ws = L.workspace(L.lib().milb200_pool_workspace_bytes(n, B, Lf), s.device)
+    L.check(L.lib().milb200_segment_softmax_pool_bwd_headdot(L.ptr(s), L.ptr(offsets), B, n, Lf, C, L.ptr(dz), L.ptr(dM),
+                                                             L.ptr(M), L.ptr(hdot), L.ptr(ds), L.ptr(attn), L.ptr(ws),
+                                                             ws.numel(), L.stream_ptr()),
+            "segment_softmax_pool_bwd_headdot")
+    return ds, attn
+
+
 def gated_scores_bwd(X, Wcat, bcat, ww, bw, ds, attn, dM, offsets, need_dx, grad_out=None, gate_act=None):
     """Backward of gated_scores (+ the pooling term of dX).  `grad_out`, if given, is a flat fp32 buffer of
     2D*L + 2D + D + 1 elements (laid out dWcat | dbcat | dww | dbw) that the kernels write in place — the
