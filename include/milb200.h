@@ -408,6 +408,27 @@ int milb200_pack_bags_host(const void* const* bag_ptrs, const int64_t* bag_rows,
                            int src_dtype, void* dst, int dst_dtype, int64_t dst_capacity_rows, int32_t* offsets,
                            int n_threads);
 
+/* ---- feeder, device side: a slide set resident in HBM (dataset.py:366-393) ------------------------------------------
+ * The slides are stored back to back in one device matrix store[total_rows, L]; slide s is rows
+ * [slide_start[s], slide_start[s+1]) (int64, device).  A batch is built with two calls on the same stream:
+ *
+ * milb200_select_rows: bag b of the batch is slide ids[b] (int32, device) and keeps k_b = offsets[b+1] - offsets[b] of
+ * its n rows (offsets int32 [n_bags+1], device, offsets[0] = 0).  Writes the bag's store row numbers to
+ * src_rows[offsets[b] .. offsets[b+1]) (int64, device): all n rows in order when k_b = n, otherwise a uniformly random
+ * k_b-subset in increasing order (the augmentation of dataset.py:375-381).  The subset is the k_b rows with the smallest
+ * 64-bit keys Philox4x32-10(counter = (row, slide id, epoch, rank), key = seed), ties broken by the lower row number: a
+ * pure function of (seed, epoch, rank, slide id, k_b), whatever the batch size or the bag's position in the batch.
+ * Caller's contract (device contents, not checked here): ids within the slide table, 1 <= k_b <= n for every bag, and
+ * src_rows holding offsets[n_bags] entries.  A bag outside it gets no rows written.
+ *
+ * milb200_gather_rows: dst[r, :] = store[src_rows[r], :] for r < n_rows, a byte copy of fp32 or bf16 rows (dtype).
+ * L * sizeof(dtype) must be a multiple of 16 (MILB200_EUNSUPPORTED otherwise) and store / dst 16-byte aligned;
+ * addresses are 64-bit, so the store may exceed 2^31 elements.  Contract: every src_rows[r] indexes a row of the store. */
+int milb200_select_rows(const int64_t* slide_start, const int32_t* ids, const int32_t* offsets, int n_bags,
+                        uint64_t seed, uint32_t epoch, uint32_t rank, int64_t* src_rows, void* stream);
+int milb200_gather_rows(const void* store, const int64_t* src_rows, int64_t n_rows, int L, int dtype, void* dst,
+                        void* stream);
+
 #ifdef __cplusplus
 }
 #endif

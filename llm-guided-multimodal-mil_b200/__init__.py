@@ -10,7 +10,7 @@ from .abmil import ABMIL, ABMIL_v2
 from . import model
 from . import clip_loss
 from . import feeder
-from .feeder import PackedBagFeeder, pack_bags_host
+from .feeder import PackedBagFeeder, ResidentBagFeeder, pack_bags_host
 from .fusion_trainer import FusionTrainer
 from .clip_loss import CLIPLogits, CLIPloss_v1
 from .model.sam.transformer import Attention, TwoWayAttentionBlock, TwoWayTransformer

@@ -83,6 +83,8 @@ SIGNATURES = {
     "milb200_pack_bags_offsets": (_i, [_p, _p, _i, _p, _p]),
     "milb200_pack_bags_host": (_i, [_p, _p, _p, _p, _p, _i, _i, _i, _p, _i, _i64, _p, _i]),
     "milb200_sigmoid_bce_fwd_bwd": (_i, [_p, _p, _p, _p, _p, _i, _p]),
+    "milb200_select_rows": (_i, [_p, _p, _p, _i, C.c_uint64, C.c_uint32, C.c_uint32, _p, _p]),
+    "milb200_gather_rows": (_i, [_p, _p, _i64, _i, _i, _p, _p]),
 }
 
 

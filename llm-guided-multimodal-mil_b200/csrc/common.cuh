@@ -147,6 +147,20 @@ __device__ __forceinline__ float adam_bias_correction(float beta, int step) {
   return -expm1f(static_cast<float>(step) * log1pf(beta - 1.f));
 }
 
+// Philox4x32-10 counter-based generator (dropout masks in core.cu, the feeder's row sampler in resident.cu): a pure
+// function of (counter, key), so a mask or a subset is regenerated instead of stored.
+__device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    const uint32_t hi0 = __umulhi(0xD2511F53u, ctr.x), lo0 = 0xD2511F53u * ctr.x;
+    const uint32_t hi1 = __umulhi(0xCD9E8D57u, ctr.z), lo1 = 0xCD9E8D57u * ctr.z;
+    ctr = make_uint4(hi1 ^ ctr.y ^ key.x, lo1, hi0 ^ ctr.w ^ key.y, lo0);
+    key.x += 0x9E3779B9u;
+    key.y += 0xBB67AE85u;
+  }
+  return ctr;
+}
+
 // index of the bag that owns global row `row`: largest b with offsets[b] <= row
 __device__ __forceinline__ int find_bag(const int32_t* __restrict__ offsets, int B, int64_t row) {
   int lo = 0, hi = B;  // invariant: offsets[lo] <= row < offsets[hi]

@@ -361,20 +361,6 @@ int transpose2d(const void* in, void* out, int rows, int cols, int dtype, cudaSt
   return MILB200_OK;
 }
 
-// Philox4x32-10 counter-based generator: element i takes word (i & 3) of block (i >> 2), so the mask is a
-// pure function of (seed, offset, i) and the backward regenerates it instead of storing it.
-__device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
-#pragma unroll
-  for (int r = 0; r < 10; ++r) {
-    const uint32_t hi0 = __umulhi(0xD2511F53u, ctr.x), lo0 = 0xD2511F53u * ctr.x;
-    const uint32_t hi1 = __umulhi(0xCD9E8D57u, ctr.z), lo1 = 0xCD9E8D57u * ctr.z;
-    ctr = make_uint4(hi1 ^ ctr.y ^ key.x, lo1, hi0 ^ ctr.w ^ key.y, lo0);
-    key.x += 0x9E3779B9u;
-    key.y += 0xBB67AE85u;
-  }
-  return ctr;
-}
-
 // One Philox call (128 random bits) serves EIGHT elements (16 bits each: keep-probability resolution 2^-16) and one
 // 128-bit (bf16) / two 128-bit (fp32) loads and stores; counter = index of the 8-element group (+ offset).
 template <typename T>

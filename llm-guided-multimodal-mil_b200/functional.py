@@ -684,3 +684,43 @@ class _CosineEmbeddingLoss(torch.autograd.Function):
 
 def cosine_embedding_loss(a, b):
     return _CosineEmbeddingLoss.apply(a, b)
+
+
+# --------------------------------------------------------------------------------------------------
+# resident feeder: row selection and row gather on the device      (reference: dataset.py:366-393)
+# --------------------------------------------------------------------------------------------------
+
+
+def select_rows(slide_start, ids, offsets, n_rows, seed, epoch=0, rank=0, out=None):
+    """Store rows of one batch -> int64 [n_rows] (n_rows = offsets[-1], known to the caller).  Bag b is slide ids[b]
+    (int32) keeping offsets[b+1] - offsets[b] (int32) of its slide_start (int64 [S+1]) rows: all of them in order, or a
+    uniformly random subset in increasing order, a pure function of (seed, epoch, rank, slide id, count).  The device
+    contents are the caller's contract (milb200.h): ids in range, 1 <= count <= rows for every bag."""
+    if slide_start.dtype != torch.int64 or ids.dtype != torch.int32 or offsets.dtype != torch.int32:
+        raise L.MilB200Error("select_rows: slide_start must be int64, ids and offsets int32")
+    B = ids.numel()
+    if offsets.numel() != B + 1:
+        raise L.MilB200Error(f"select_rows: offsets has {offsets.numel()} entries for {B} bags")
+    if out is None:
+        out = torch.empty((int(n_rows),), dtype=torch.int64, device=ids.device)
+    elif out.dtype != torch.int64 or out.numel() < int(n_rows):
+        raise L.MilB200Error(f"select_rows: out must be int64 with at least {int(n_rows)} entries")
+    L.check(L.lib().milb200_select_rows(L.ptr(slide_start), L.ptr(ids), L.ptr(offsets), B, int(seed) & (2**64 - 1),
+                                        int(epoch) & 0xffffffff, int(rank) & 0xffffffff, L.ptr(out), L.stream_ptr()),
+            "select_rows")
+    return out[:int(n_rows)]
+
+
+def gather_rows(store, src_rows, out=None):
+    """out[r] = store[src_rows[r]] for every r of src_rows (int64, indices into the rows of store [rows, L], fp32 or
+    bf16; each must be a row of the store).  A byte copy; L * itemsize must be a multiple of 16."""
+    if store.dim() != 2 or src_rows.dtype != torch.int64:
+        raise L.MilB200Error("gather_rows: store must be [rows, L] and src_rows int64")
+    n = src_rows.numel()
+    if out is None:
+        out = torch.empty((n, store.shape[1]), dtype=store.dtype, device=store.device)
+    elif out.dtype != store.dtype or out.dim() != 2 or out.shape[1] != store.shape[1] or out.shape[0] < n:
+        raise L.MilB200Error(f"gather_rows: out must be {store.dtype} [>= {n}, {store.shape[1]}]")
+    L.check(L.lib().milb200_gather_rows(L.ptr(store), L.ptr(src_rows), n, store.shape[1], L.dtype_code(store),
+                                        L.ptr(out), L.stream_ptr()), "gather_rows")
+    return out[:n]
