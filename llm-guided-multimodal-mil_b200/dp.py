@@ -6,7 +6,7 @@ gradient buckets, hooks or unused-parameter bitmaps.
 
 Flat layout (fp32), chosen so that [Wv; Wu] is the contiguous Wcat operand the kernels want:
     Wv (D*L) | Wu (D*L) | bv (D) | bu (D) | ww (D) | bw (1)
-and, with a linear classifier head of C classes (head_classes = C), after padding to 16 bytes:
+and, with a linear classifier head of C classes (head_classes = C), after padding to 32 bytes:
     head.weight (C*L) | head.bias (C)
 """
 from __future__ import annotations
@@ -36,8 +36,9 @@ def shard_bags(lengths, rank, world, balance=True):
 
 
 def _head_offset(L_feat, D):
-    """First element of the head in the flat buffer: the pool's parameters rounded up to 16 bytes."""
-    return (2 * D * L_feat + 3 * D + 1 + 3) // 4 * 4
+    """First element of the head in the flat buffer: the pool's parameters rounded up to 32 bytes (8 elements, the
+    granule of FusionTrainer's flat layout, which embeds this one)."""
+    return (2 * D * L_feat + 3 * D + 1 + 7) // 8 * 8
 
 
 def flat_layout(L_feat, D, C=0):
@@ -252,19 +253,23 @@ class AbmilTrainer:
                                ones=torch.ones((B, self.L), dtype=f32, device=dev) if self.head_p > 0.0 else None)
         return b
 
-    def forward_backward_labels(self, X, offsets, labels):
+    def forward_backward_labels(self, X, offsets, labels, loss=None):
         """Forward + backward of pool -> head -> sigmoid -> BCE (mean over B*C, train_ddp.py:99,319) against labels fp32
         [B, C] (one-hot), all on the device.  The pooling pass takes the head's C row dots, so X is read by the score GEMM,
         the pooling pass and the dW GEMM only (as in forward_backward).  Gradients of the pool and of the head go to the
         flat buffer.  Returns (loss [1], prob [B, C]): device tensors that the next step with the same B overwrites.  The
-        pooled vectors M [B, L] are left in `last_pooled`, and dL/dX (need_input_grad) in `last_dX`."""
+        BCE is written into `loss` instead when it is given (a one-element fp32 device tensor, e.g. one entry of a caller's
+        loss vector).  The pooled vectors M [B, L] are left in `last_pooled`, and dL/dX (need_input_grad) in `last_dX`."""
         if not self.C:
             raise ValueError("forward_backward_labels needs a trainer built with head_classes > 0")
         B = offsets.numel() - 1
         if labels.dtype != torch.float32 or tuple(labels.shape) != (B, self.C) or not labels.is_contiguous():
             raise ValueError(f"labels must be a contiguous fp32 [{B}, {self.C}] tensor")
+        if loss is not None and (loss.dtype != torch.float32 or loss.numel() != 1):
+            raise ValueError("loss must be a one-element fp32 tensor")
         lib, Lf, C = L.lib(), self.L, self.C
         b = self._head_bufs(B)
+        loss = b["loss"] if loss is None else loss
         M = self._forward(X, offsets, None, head=True)
         v, g, seed_h = self._views(self.params), self._views(self.grads), self._seed_h
         mark = self.phase_hook or (lambda name: None)
@@ -272,7 +277,7 @@ class AbmilTrainer:
         lws = L.workspace(lib.milb200_linear_workspace_bytes(B, C, Lf, L.F32, 1), self.device)
         L.check(lib.milb200_linear_fwd(L.ptr(Mh), None, L.ptr(v["head_w"]), L.ptr(v["head_b"]), L.ptr(b["z"]), B, C, Lf,
                                        L.ACT_NONE, L.F32, L.ptr(lws), lws.numel(), L.stream_ptr()), "head linear_fwd")
-        L.check(lib.milb200_sigmoid_bce_fwd_bwd(L.ptr(b["z"]), L.ptr(labels), L.ptr(b["prob"]), L.ptr(b["loss"]),
+        L.check(lib.milb200_sigmoid_bce_fwd_bwd(L.ptr(b["z"]), L.ptr(labels), L.ptr(b["prob"]), L.ptr(loss),
                                                 L.ptr(b["dz"]), B * C, L.stream_ptr()), "sigmoid_bce")
         L.check(lib.milb200_linear_bwd(L.ptr(Mh), None, L.ptr(v["head_w"]), L.ptr(b["z"]), L.ptr(b["dz"]), L.ptr(b["dMh"]),
                                        L.ptr(g["head_w"]), L.ptr(g["head_b"]), B, C, Lf, L.ACT_NONE, L.F32, 0, L.ptr(lws),
@@ -281,7 +286,7 @@ class AbmilTrainer:
         dM = b["dMh"] if seed_h is None else F._dropout_raw(b["dMh"], self.head_p, seed_h, 0)
         mark("head")
         self.last_pooled, self.last_dX = M, self._backward(dM, b["dz"])
-        return b["loss"], b["prob"]
+        return loss, b["prob"]
 
     def step_labels(self, X, offsets, labels):
         """forward_backward_labels + exchange + optimiser.  Returns (loss [1], prob [B, C]) on the device."""

@@ -6,8 +6,10 @@
 
 without the autograd graph: every parameter of the branch lives in ONE flat fp32 buffer (fusion-program parameters |
 gated pool | head), the backward kernels write into ONE flat gradient buffer, DDP's exchange is ONE all-reduce and the
-optimiser ONE kernel — the same design as `dp.AbmilTrainer`, which this class embeds for the gated pool.  `load_from` /
-`store_to` move parameters from / to the reference-shaped module, so checkpoints keep the reference's state_dict.
+optimiser ONE kernel — the same design as `dp.AbmilTrainer`, which this class embeds for the gated pool, the head and
+the BCE: the program's packed bag goes through `AbmilTrainer.forward_backward_labels`, whose pooling pass takes the
+head's row dots, so the pool's backward does not read the bag again.  `load_from` / `store_to` move parameters from /
+to the reference-shaped module, so checkpoints keep the reference's state_dict.  The head takes 1..8 classes.
 
 With one clinical-text token per patient (the reference's active prompt configuration) the step runs the COLLAPSED
 program (csrc/xfusion.cu: no projected image tokens, the CT bag and the pathology bag as segments of one launch set,
@@ -28,8 +30,7 @@ import ctypes as C
 import torch
 
 from . import _lib as L
-from . import functional as F
-from .dp import AbmilTrainer
+from .dp import AbmilTrainer, flat_layout
 from .model.sam.transformer import _use_collapsed
 
 
@@ -53,26 +54,26 @@ class FusionTrainer:
         self.train_mode = bool(train_mode)
         self.E = model.embedding_dim
         self.C = model.fc[1].weight.shape[0]
+        if not 1 <= self.C <= 8:
+            raise ValueError(f"FusionTrainer trains 1..8 classes (the pooling pass takes up to 8 head row dots per row), "
+                             f"got num_classes = {self.C}")
         self.collapsed = self.T == 1 and _use_collapsed()
         self.tape = model._fusion_tape_v2() if self.collapsed else model._fusion_tape(single_token=(self.T == 1))
         c = self.tape._freeze()
         self.n_tape = c["total"]
-        D = model.aggregator.attention_V[0].weight.shape[0]
-        self.n_pool = 2 * D * self.E + 3 * D + 1
+        # the gated pool, the head and the BCE run through AbmilTrainer's labelled step on views of the same flat buffers
+        # (its instances are the program's output, so it also gives the gradient of the packed bag)
+        self.pool = AbmilTrainer(self.E, model.aggregator.attention_V[0].weight.shape[0], compute_dtype, device=self.device,
+                                 need_input_grad=True, head_classes=self.C,
+                                 dropout_p=(model.aggregator.dropout1.p if self.train_mode else 0.0),
+                                 head_dropout=(model.fc[0].p if self.train_mode else 0.0))
         up8 = lambda n: (n + 7) // 8 * 8
         self.o_pool = up8(self.n_tape)
-        self.o_head_w = up8(self.o_pool + self.n_pool)
-        self.o_head_b = up8(self.o_head_w + self.C * self.E)
-        self.numel = up8(self.o_head_b + self.C)
+        self.numel = up8(self.o_pool + self.pool.numel)
         z = lambda: torch.zeros(self.numel, dtype=torch.float32, device=self.device)
         self.params, self.grads, self.exp_avg, self.exp_avg_sq = z(), z(), z(), z()
-        # the gated pool runs through AbmilTrainer on views of the same flat buffers (its instances are the program's
-        # output, so it also returns the gradient of the packed bag)
-        self.pool = AbmilTrainer(self.E, D, compute_dtype, device=self.device, need_input_grad=True,
-                                 dropout_p=(model.aggregator.dropout1.p if self.train_mode else 0.0))
-        sl = slice(self.o_pool, self.o_pool + self.n_pool)
+        sl = slice(self.o_pool, self.o_pool + self.pool.numel)
         self.pool.params, self.pool.grads = self.params[sl], self.grads[sl]
-        self.head_p = float(model.fc[0].p) if self.train_mode else 0.0
         self.wc = torch.empty(self.n_tape, dtype=compute_dtype, device=self.device) if compute_dtype != torch.float32 else None
         self.step_count = 0
         self._buf = {}
@@ -80,36 +81,32 @@ class FusionTrainer:
 
     # ---- parameters <-> module ----------------------------------------------------------------------------------
     def _module_tensors(self):
-        """(flat offset, tensor) for every parameter outside the pool, in flat-buffer order."""
+        """(flat offset, tensor) for every parameter of the fusion program, in flat-buffer order."""
         c = self.tape._freeze()
-        out = [(off, p) for p, off in zip(self.tape.params, c["offsets"])]
-        out.append((self.o_head_w, self.model.fc[1].weight))
-        out.append((self.o_head_b, self.model.fc[1].bias))
-        return out
+        return [(off, p) for p, off in zip(self.tape.params, c["offsets"])]
 
     @torch.no_grad()
     def load_from(self, model=None):
         for off, p in self._module_tensors():
             self.params[off:off + p.numel()].copy_(p.detach().reshape(-1))
-        self.pool.load_from(self.model.aggregator)
+        self.pool.load_from(self.model.aggregator, head=self.model.fc[1])
         self._refresh_compute_copy()
 
     @torch.no_grad()
     def store_to(self, model=None):
         for off, p in self._module_tensors():
             p.copy_(self.params[off:off + p.numel()].view(p.shape))
-        self.pool.store_to(self.model.aggregator)
+        self.pool.store_to(self.model.aggregator, head=self.model.fc[1])
 
     def named_grads(self):
-        """{state_dict name: gradient view} for the tests (program / head parameters by module name; pool under aggregator.*)."""
-        names = {id(p): n for n, p in self.model.named_parameters()}
+        """{state_dict name: gradient view} for the tests (program parameters by module name, the pool under aggregator.*,
+        the head under fc.1.*)."""
+        params = dict(self.model.named_parameters())
+        names = {id(p): n for n, p in params.items()}
         out = {names[id(p)]: self.grads[off:off + p.numel()].view(p.shape) for off, p in self._module_tensors()}
-        gv = self.pool.grad_views()
-        D = self.pool.D
-        out["aggregator.attention_V.0.weight"], out["aggregator.attention_U.0.weight"] = gv["Wcat"][:D], gv["Wcat"][D:]
-        out["aggregator.attention_V.0.bias"], out["aggregator.attention_U.0.bias"] = gv["bcat"][:D], gv["bcat"][D:]
-        out["aggregator.attention_weights.weight"] = gv["ww"].view(1, D)
-        out["aggregator.attention_weights.bias"] = gv["bw"]
+        for k, (a, b) in flat_layout(self.E, self.pool.D, self.C).items():
+            name = "fc.1." + k[len("head."):] if k.startswith("head.") else "aggregator." + k
+            out[name] = self.pool.grads[a:b].view(params[name].shape)
         return out
 
     def _refresh_compute_copy(self):
@@ -146,7 +143,7 @@ class FusionTrainer:
             segp = t._segments(segs)
             mk = lambda r, cc, dt=None: torch.empty((int(r), int(cc)), dtype=dt or self.dtype, device=dev)
             sdt = lambda s: torch.float32 if t.slot_f32[s] else self.dtype
-            B, Cn, T, E = n_bags, self.C, self.T, self.E
+            B, T, E = n_bags, self.T, self.E
             f32 = torch.float32
             b = dict(code=code,
                      arena=torch.empty(lib.milb200_tape_arena_bytes(c["ops"], c["n_ops"], slots_cap, c["n_slots"], code, segp),
@@ -155,8 +152,6 @@ class FusionTrainer:
                      # (the cached position tables are used in place: no staging buffer for them)
                      stage=[None if j in ((2,) if self.collapsed else (1, 3)) else mk(slots_cap[s].rows, slots_cap[s].cols, sdt(s))
                             for j, s in enumerate(t.inputs)],
-                     z=torch.empty((B, Cn), dtype=f32, device=dev), prob=torch.empty((B, Cn), dtype=f32, device=dev),
-                     dz=torch.empty((B, Cn), dtype=f32, device=dev), dM=torch.empty((B, E), dtype=f32, device=dev),
                      loss=torch.zeros(2, dtype=f32, device=dev),
                      cos_rows=torch.empty(max(B * T, 1), dtype=f32, device=dev),
                      da=mk(B * T, E), db=mk(B * T, E), offsets={})
@@ -221,8 +216,11 @@ class FusionTrainer:
         L.check(lib.milb200_tape_forward(c["ops"], c["n_ops"], slots, n_slots, c["params"], c["n_params"], ext, L.ptr(wcomp),
                                          L.ptr(self.params), L.ptr(b["arena"]), b["arena"].numel(), L.ptr(ws), ws.numel(),
                                          code, segp, L.stream_ptr()), "tape_forward")
-        self._set_targets(labels, B)
-        dbag = self._pool_head_losses(b, bag, B, offsets)
+        _, prob = self.pool.forward_backward_labels(bag, offsets, labels.reshape(B, Cn).to(torch.float32).contiguous(),
+                                                    loss=b["loss"][0:1])
+        # the program's backward replays as a CUDA graph keyed by its pointers: without the pool trainer's reference the
+        # next step's gradient of the packed bag reuses this block instead of alternating between two addresses
+        dbag, self.pool.last_dX = self.pool.last_dX, None
         dtok = b["dtok"]
         if not self.cosine_loss:
             dtok.zero_()                  # the backward accumulates into the seeded buffers in place
@@ -244,39 +242,7 @@ class FusionTrainer:
                                           L.ptr(wcomp), L.ptr(self.params), L.ptr(self.grads), L.ptr(b["arena"]),
                                           b["arena"].numel(), L.ptr(ws), ws.numel(), code, segp, L.stream_ptr()),
                 "tape_backward")
-        return b["loss"], b["prob"]
-
-    def _pool_head_losses(self, b, bag, B, offsets):
-        """Gated pool over the packed bag(s) (aggregator.py:199), head (:200) + BCE (train_ddp.py:99,319) and their
-        backward; returns the gradient of the packed bag."""
-        lib = L.lib()
-        E, Cn = self.E, self.C
-        M = self.pool.forward(bag, offsets)                                   # (B, E) fp32
-        Mh, seed_h = M, None
-        if self.head_p > 0.0:                                                 # aggregator.py:128-131 Dropout(0.25), train mode
-            seed_h = int(torch.randint(0, 2 ** 62, (1,), dtype=torch.int64).item())
-            Mh = F._dropout_raw(M, self.head_p, seed_h, 0)
-        hw = self.params[self.o_head_w:self.o_head_w + Cn * E]
-        hb = self.params[self.o_head_b:self.o_head_b + Cn]
-        lws = L.workspace(lib.milb200_linear_workspace_bytes(B, Cn, E, L.F32, 1), self.device)
-        L.check(lib.milb200_linear_fwd(L.ptr(Mh), None, L.ptr(hw), L.ptr(hb), L.ptr(b["z"]), B, Cn, E, L.ACT_NONE,
-                                       L.F32, L.ptr(lws), lws.numel(), L.stream_ptr()), "head linear_fwd")
-        L.check(lib.milb200_sigmoid_bce_fwd_bwd(L.ptr(b["z"]), L.ptr(self._targets), L.ptr(b["prob"]), L.ptr(b["loss"][0:1]),
-                                                L.ptr(b["dz"]), B * Cn, L.stream_ptr()), "sigmoid_bce")
-        gw = self.grads[self.o_head_w:self.o_head_w + Cn * E]
-        gb = self.grads[self.o_head_b:self.o_head_b + Cn]
-        L.check(lib.milb200_linear_bwd(L.ptr(Mh), None, L.ptr(hw), L.ptr(b["z"]), L.ptr(b["dz"]), L.ptr(b["dM"]), L.ptr(gw),
-                                       L.ptr(gb), B, Cn, E, L.ACT_NONE, L.F32, 0, L.ptr(lws), lws.numel(),
-                                       L.stream_ptr()), "head linear_bwd")
-        dM = b["dM"] if seed_h is None else F._dropout_raw(b["dM"], self.head_p, seed_h, 0)
-        return self.pool.backward(dM)                                         # (rows of the bag, E), compute dtype
-
-    @property
-    def _targets(self):
-        return self.__dict__["_tgt"]
-
-    def _set_targets(self, labels, B):
-        self.__dict__["_tgt"] = labels.reshape(B, self.C).to(torch.float32).contiguous()
+        return b["loss"], prob
 
     # ---- the projected-keys program of round 1 (T > 1, or MILB200_FUSION_COLLAPSED=0): one patient per step -------------
     def _forward_backward_projected(self, ct_tokens, x_path, x_text, label):
@@ -309,8 +275,9 @@ class FusionTrainer:
                                          L.ptr(self.params), L.ptr(b["arena"]), b["arena"].numel(), L.ptr(ws), ws.numel(),
                                          code, None, L.stream_ptr()), "tape_forward")
         bag = b["out"][0]                                                     # aggregator.py:173 row order
-        self._set_targets(label, 1)
-        dbag = self._pool_head_losses(b, bag, 1, offsets)
+        _, prob = self.pool.forward_backward_labels(bag, offsets, label.reshape(1, self.C).to(torch.float32).contiguous(),
+                                                    loss=b["loss"][0:1])
+        dbag, self.pool.last_dX = self.pool.last_dX, None                    # (see forward_backward_bags)
         if self.cosine_loss:
             a_rows, b_rows = bag[0:T], bag[T + Nc:2 * T + Nc]                 # x_CT2CI, x_Pth2CI (aggregator.py:160,168)
             L.check(lib.milb200_cosine_embedding_fwd_bwd(L.ptr(a_rows), L.ptr(b_rows), L.ptr(b["loss"][1:2]),
@@ -330,7 +297,7 @@ class FusionTrainer:
         L.check(lib.milb200_tape_backward(c["ops"], c["n_ops"], slots, n_slots, c["params"], c["n_params"], ext2, gext, seeds,
                                           L.ptr(wcomp), L.ptr(self.params), L.ptr(self.grads), L.ptr(b["arena"]),
                                           b["arena"].numel(), L.ptr(ws), ws.numel(), code, None, L.stream_ptr()), "tape_backward")
-        return b["loss"], b["prob"]
+        return b["loss"], prob
 
     # ---- exchange + optimiser -------------------------------------------------------------------------------------------
     def enable_symmetric_exchange(self):
@@ -358,8 +325,7 @@ class FusionTrainer:
             return False
         buf[:self.numel].copy_(self.grads)
         self.grads = buf[:self.numel]
-        sl = slice(self.o_pool, self.o_pool + self.n_pool)
-        self.pool.grads = self.grads[sl]                   # the embedded pool trainer writes into the same buffer
+        self.pool.grads = self.grads[self.o_pool:self.o_pool + self.pool.numel]    # the embedded pool trainer's view
         pads = torch.tensor([int(p) for p in hdl.signal_pad_ptrs], dtype=torch.int64, device=self.device)
         self._symm = dict(hdl=hdl, buf=buf, pads=pads, mc=mc, rank=int(hdl.rank))
         torch.cuda.synchronize()

@@ -522,8 +522,11 @@ def test_fusion_trainer_matches_module_autograd(T, dtype, tol):
         opt = torch.optim.Adam(m.parameters(), lr=1e-3, betas=(0.9, 0.999), weight_decay=1e-7)
         opt.step()                                         # m's parameters move in place; tr.params still holds the old ones
         tr.reduce_and_update()
+        from mil_b200.dp import flat_layout
+        lay = flat_layout(tr.E, tr.pool.D, tr.C)
+        head = [(tr.o_pool + lay["head.weight"][0], m.fc[1].weight), (tr.o_pool + lay["head.bias"][0], m.fc[1].bias)]
         compared = 0
-        for off, p in tr._module_tensors():
+        for off, p in tr._module_tensors() + head:
             g = p.grad
             if g is None:
                 continue

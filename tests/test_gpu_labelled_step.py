@@ -384,7 +384,7 @@ def test_flat_layout_with_head():
         lay = flat_layout(Lf, D, C)
         assert flat_layout(Lf, D, 0) == base and {k: lay[k] for k in base} == base
         h0, h1 = lay["head.weight"]
-        assert h0 % 4 == 0 and h0 >= base["attention_weights.bias"][1] and h1 - h0 == C * Lf
+        assert h0 % 8 == 0 and h0 >= base["attention_weights.bias"][1] and h1 - h0 == C * Lf
         assert lay["head.bias"] == (h1, h1 + C)
         tr = AbmilTrainer(Lf, D, torch.float32, device="cpu", head_classes=C)
         assert tr.numel == h1 + C and tr.n_pool == 2 * D * Lf + 3 * D + 1

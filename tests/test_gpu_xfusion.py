@@ -278,6 +278,52 @@ def test_fusion_trainer_train_mode_matches_module_train_mode_on_the_same_masks()
     m.eval()
 
 
+@pytest.mark.parametrize("T", [1, 10])
+def test_fusion_trainer_pool_head_bce_is_the_labelled_step(T):
+    """The pool, head and BCE of a FusionTrainer step (collapsed program with B = 3 patients, projected-keys program with
+    T = 10) are the pool trainer's labelled step: the head's row dots come from the pooling pass, so the backward makes no
+    pass over the packed bag; its loss and prob equal the two-pass route's (forward, head + BCE, backward(dM)) on the same
+    bag bit for bit, and the bag's gradient differs by reassociation only."""
+    import mil_b200
+    from mil_b200.dp import AbmilTrainer
+    from tests.test_gpu_labelled_step import _two_pass
+    m, _ = _model(seed=37)
+    tr = mil_b200.FusionTrainer(m, n_text_tokens=T, compute_dtype=torch.float32)
+    seen, names = {}, []
+    step = tr.pool.forward_backward_labels
+
+    def spy(X, offsets, labels, loss=None):
+        seen.update(X=X.clone(), offsets=offsets.clone(), labels=labels.clone())
+        out = step(X, offsets, labels, loss=loss)
+        seen["dX"] = tr.pool.last_dX.clone()          # the program's backward then adds the cosine loss's rows in place
+        return out
+
+    tr.pool.forward_backward_labels = spy
+    tr.pool.phase_hook = names.append
+    g = torch.Generator(device="cuda").manual_seed(14)
+    if T == 1:
+        lens, B = [900, 64, 3100], 3
+        ct = torch.randn(B, 160, 512, device="cuda", generator=g)
+        xp = torch.randn(sum(lens), 768, device="cuda", generator=g)
+        xt = torch.randn(B, 512, device="cuda", generator=g) * 0.05
+        labels = torch.tensor([[0.0, 1.0], [1.0, 0.0], [0.0, 1.0]], device="cuda")
+        loss, prob = tr.forward_backward_bags(ct, xp, lens, xt, labels)
+    else:
+        ct = torch.randn(160, 512, device="cuda", generator=g)
+        xp = torch.randn(1203, 768, device="cuda", generator=g)
+        xt = torch.randn(T, 512, device="cuda", generator=g) * 0.05
+        loss, prob = tr.forward_backward(ct, xp, xt, torch.tensor([1.0, 0.0], device="cuda"))
+    torch.cuda.synchronize()
+    assert "pool_bwd_headdot" in names and "segment_softmax_pool_bwd" not in names
+    assert tuple(loss.shape) == (2,) and float(loss[1]) > 0.0
+    ref = AbmilTrainer(512, tr.pool.D, torch.float32, device="cuda", need_input_grad=True, head_classes=2)
+    ref.params.copy_(tr.pool.params)
+    l2, p2, dX2 = _two_pass(ref, seen["X"], seen["offsets"], seen["labels"])
+    torch.cuda.synchronize()
+    assert torch.equal(loss[0:1], l2) and torch.equal(prob, p2)
+    assert _rel(seen["dX"], dX2) <= 1e-5
+
+
 @pytest.mark.parametrize("case", ["tiny_bags", "sixteen_segments", "one_huge_bag"])
 def test_collapsed_fusion_edge_shapes_vs_oracle(case):
     """Segment machinery at its edges: 2-row bags (fewer rows than warps), 8 patients = 16 segments with lengths that are
